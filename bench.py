@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native ReVolt dynamic-positioning hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--envs-per-gpu E]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--envs-per-gpu E] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -18,6 +18,9 @@ One JSON line on stdout (rank 0):
   roofline   HBM roofline of the env-step kernel: 177 algorithmic bytes per env-step (SURVEY.md 8d)
   cpu_baseline  the CPU oracle (vectorised NumPy port of the reference wrapper + float64 hull) on a bounded sample
   extra      secondary kernels of the path (QP allocations/s, pseudoinverse+PID/s, ...), each with its own roofline
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0) as DIR/<name>.npy, so that two builds
+run with the same arguments -- hence the same seeded inputs -- can be compared output for output.
 """
 import argparse
 import json
@@ -51,6 +54,7 @@ ROLLOUT_TRAIN_BYTES = 185  # state r/w 108 + trajectory record 77 (SURVEY.md 8d)
 GAE_BYTES = 17            # read r, V, flag byte; write A, R
 ACTION_POOL = 2           # flat U(-1,1) buffers; step i reads a [7, n] window at a new offset: fresh actions per (env, step)
 ACTION_SHIFT = 4 * 1031   # floats between consecutive windows (16-byte aligned, so the vectorised kernel path is kept)
+DUMP_ENVS = 1 << 19       # environments sampled by --dump-outputs: 11 float32 outputs + 1 float64 index each, 27 MB in all
 
 
 def load_tensor_peak():
@@ -306,24 +310,19 @@ def run_reference(args, rank, world):
     for _ in range(max(1, min(args.warmup, 2))):
         step_all(1)
     t0 = time.perf_counter()
-    done_steps = 0
-    budget_s = 120.0
     for _ in range(args.steps):
         step_all(inner)
-        done_steps += 1
-        if time.perf_counter() - t0 > budget_s:
-            break
     wall = time.perf_counter() - t0
     for a in pipes:
         a.send(0)
     for pr in procs:
         pr.join(timeout=5)
     n_total = per * cores
-    value = n_total * inner * done_steps / wall
-    sample = "%d envs x %d env-steps per bench step, %d bench steps, %d persistent processes" % (n_total, inner, done_steps, cores)
+    value = n_total * inner * args.steps / wall
+    sample = "%d envs x %d env-steps per bench step, %d bench steps, %d persistent processes" % (n_total, inner, args.steps, cores)
     line = {
         "impl": "reference", "metric": "env_steps_per_sec", "value": value, "unit": "env-steps/s",
-        "n_gpus": args.gpus, "steps": done_steps, "warmup": args.warmup, "ms_per_step": 1e3 * wall / done_steps,
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * wall / args.steps,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": workload_config(args, world),
         "cpu_baseline": {"value": value, "unit": "env-steps/s", "cores": cores, "kind": "port", "sample": sample},
@@ -381,24 +380,20 @@ def run_reference_code(args, world):
     for _ in range(max(1, min(args.warmup, 2))):
         step_all(2)
     t0 = time.perf_counter()
-    done_steps = 0
     for _ in range(args.steps):
         step_all(inner)
-        done_steps += 1
-        if time.perf_counter() - t0 > 120.0:
-            break
     wall = time.perf_counter() - t0
     for a in pipes:
         a.send(0)
     for pr in procs:
         pr.join(timeout=5)
-    value = per * cores * inner * done_steps / wall
+    value = per * cores * inner * args.steps / wall
     sample = ("%d reference RevoltFinal objects (%s) x %d env-steps per bench step, %d bench steps, %d persistent processes; "
-              "simulator = the float64 stand-in twin" % (per * cores, ref_loader.source(), inner, done_steps, cores))
+              "simulator = the float64 stand-in twin" % (per * cores, ref_loader.source(), inner, args.steps, cores))
     port_val, _, port_sample = cpu_env_steps_per_s(1 << 16, 8)
     emit({
         "impl": "reference", "metric": "env_steps_per_sec", "value": value, "unit": "env-steps/s",
-        "n_gpus": args.gpus, "steps": done_steps, "warmup": args.warmup, "ms_per_step": 1e3 * wall / done_steps,
+        "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * wall / args.steps,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": workload_config(args, world),
         "cpu_baseline": {"value": value, "unit": "env-steps/s", "cores": cores, "kind": "reference", "sample": sample,
@@ -417,6 +412,20 @@ def workload_config(args, world):
 
 
 # ---- GPU side ----------------------------------------------------------------------------------------------------
+def dump_outputs(path, obs, rew, done):
+    """obs [9, n], reward [n] and the done flag byte [n] of one env step, on a fixed seeded sample of DUMP_ENVS
+    environments (all of them when n is smaller), as float32; env_index.npy holds the sampled indices (float64)."""
+    import numpy as np
+    import torch
+    n = rew.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_ENVS), replace=False))
+    sel = torch.as_tensor(idx, device=obs.device)
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("obs", obs[:, sel]), ("reward", rew[sel]), ("done", done[sel])):
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+
+
 def bind_to_gpu_cpus(index):
     """Multi-rank runs: pin this process to the CPUs NVML reports as local to its GPU, BEFORE the pinned host buffers of the
     end-to-end leg are allocated (first touch puts them on that NUMA node).  The launcher does not bind ranks, and eight
@@ -500,6 +509,8 @@ def run_b200(args, rank, local_rank, world):
     sampler.mark("end")
     ms = ev0.elapsed_time(ev1)
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:        # before the sustained leg below overwrites `out`
+        dump_outputs(args.dump_outputs, *out)
     barrier()
     ms_all = max_over_ranks(ms)
     ms_per_step = ms_all / args.steps
@@ -842,7 +853,13 @@ def main():
     ap.add_argument("--envs-per-gpu", type=int, default=1 << 24)
     ap.add_argument("--skip-cpu", action="store_true", help="omit the CPU baseline leg (used for ncu captures)")
     ap.add_argument("--skip-extra", action="store_true", help="omit the secondary-kernel figures under 'extra'")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (obs, reward, done of a fixed env sample) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

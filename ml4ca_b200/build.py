@@ -54,6 +54,8 @@ def build(force=False, verbose=False, extra_flags=(), out=None):
         LIB = os.path.join(HERE, out)
         STAMP = LIB + ".stamp"
         force = True
+    if not force and _up_to_date(_digest()):
+        return LIB      # nothing to write: a read-only tree that was built beforehand loads as it is
     # one builder at a time: under torchrun every rank may get here at once and would write the same .o / .so / stamp files
     import fcntl
     with open(os.path.join(HERE, ".build.lock"), "w") as lock:
@@ -64,13 +66,18 @@ def build(force=False, verbose=False, extra_flags=(), out=None):
             fcntl.flock(lock, fcntl.LOCK_UN)
 
 
+def _up_to_date(digest):
+    if not (os.path.exists(LIB) and os.path.exists(STAMP)):
+        return False
+    with open(STAMP) as fh:
+        return fh.read().strip() == digest
+
+
 def _build_locked(force, verbose, extra_flags, out):
     global LIB, STAMP
     digest = _digest()
-    if not force and os.path.exists(LIB) and os.path.exists(STAMP):
-        with open(STAMP) as fh:
-            if fh.read().strip() == digest:
-                return LIB
+    if not force and _up_to_date(digest):
+        return LIB
     objs = []
     log = []
 
@@ -91,12 +98,18 @@ def _build_locked(force, verbose, extra_flags, out):
             sys.stderr.write("\n".join(log)[-6000:])
             raise RuntimeError("nvcc failed on %s" % src)
         objs.append(obj)
-    cmd = [_nvcc(), "-shared", "-o", LIB] + objs + ["-lcudart"]
+    # link under a temporary name and rename: a caller that found the stamp current without the lock (build() above) may be
+    # loading LIB while a forced rebuild runs, and must see the old or the new library, never a partly written one
+    tmp = "%s.tmp%d.so" % (os.path.splitext(LIB)[0], os.getpid())     # still matched by the *.so ignore rule
+    cmd = [_nvcc(), "-shared", "-o", tmp] + objs + ["-lcudart"]
     res = subprocess.run(cmd, capture_output=True, text=True)
     log.append("$ " + " ".join(cmd) + "\n" + res.stdout + res.stderr)
     if res.returncode != 0:
+        if os.path.exists(tmp):
+            os.remove(tmp)
         sys.stderr.write("\n".join(log)[-6000:])
         raise RuntimeError("link failed")
+    os.replace(tmp, LIB)
     with open(os.path.join(HERE, "build.log"), "w") as fh:
         fh.write("\n".join(log))
     with open(STAMP, "w") as fh:

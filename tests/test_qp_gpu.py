@@ -137,7 +137,7 @@ def test_single_env_reference_call_shape(cuda_device):
         ta.solve_QP(np.zeros((3, 1)), weight_matrix=Q)
 
 
-def test_both_kernel_mappings_agree(cuda_device):
+def test_both_kernel_mappings_agree(cuda_device, tmp_path):
     """One thread per demand (default) and one demand over 8 lanes (ML4CA_QP_MAPPING=group, csrc/qp_group.cuh) are the same
     solver: equal flags and iteration counts, end points equal to fp32 output resolution."""
     import subprocess
@@ -147,7 +147,7 @@ def test_both_kernel_mappings_agree(cuda_device):
             "np.savez(sys.argv[1], x=x.cpu().numpy(), st=ta.last_status.cpu().numpy())")
     outs = []
     for mapping in ("thread", "group"):
-        path = "/tmp/qp_mapping_%s.npz" % mapping
+        path = str(tmp_path / ("qp_mapping_%s.npz" % mapping))
         env = dict(os.environ, ML4CA_QP_MAPPING=mapping)
         subprocess.run([sys.executable, "-c", code % (ROOT, os.path.join(ROOT, "tests", "golden", "qp_config1.npz")), path],
                        check=True, env=env, cwd=ROOT)
