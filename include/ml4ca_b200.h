@@ -115,6 +115,32 @@ ML4CA_API int ml4ca_env_get_state(ml4ca_env* env, float* eta, float* nu, float* 
                         void* stream);
 ML4CA_API int64_t ml4ca_env_size(const ml4ca_env* env);
 
+/* Environmental disturbance (DECLARED model, DESIGN.md section 4; the reference's Cybersea simulator sets its environment
+ * through DigiTwin.val, digitwin.py:213-217).  Ocean current: constant in the NED frame over an episode,
+ * v_c = V [cos beta, sin beta] with V ~ U(current_speed_min, current_speed_max) and beta ~ U(current_dir_min,
+ * current_dir_max) drawn at every reset (explicit or in-kernel); beta is the direction the water flows towards (0 = north,
+ * pi/2 = east).  The hull equations act on the velocity relative to the water; the observed nu stays the velocity over
+ * ground.  Bias force: b = [X_N, Y_E, N_psi] in the NED frame, a first-order Gauss-Markov process
+ * b <- a b + bias_std sqrt(1 - a^2) w per env step, a = exp(-step_dt / bias_time_s), drawn as b = bias_std w0 at every reset;
+ * bias_time_s = 0 keeps b constant over the episode.  Holding station against a beam current of 0.3 m/s takes the full sway
+ * thrust of either hull model: 0 to 0.2 m/s is the useful range. */
+typedef struct ml4ca_disturbance_cfg {
+  float current_speed_min, current_speed_max; /* m/s, 0 <= min <= max */
+  float current_dir_min, current_dir_max;     /* rad, min <= max */
+  float bias_std[3];                          /* N, N, Nm, >= 0: stationary standard deviation of b */
+  float bias_time_s;                          /* >= 0: time constant of b; 0 = constant over the episode */
+} ml4ca_disturbance_cfg;
+
+/* Enable (cfg != NULL) or switch off (cfg = NULL) the disturbance.  Enabling draws the current and the bias of every env
+ * from the new ranges on `stream`; every later reset draws them again.  Launch parameter: CUDA graphs captured earlier
+ * keep the values they were captured with.  Bad ranges: ML4CA_ERR_INVALID. */
+ML4CA_API int ml4ca_env_set_disturbance(ml4ca_env* env, const ml4ca_disturbance_cfg* cfg, void* stream);
+/* Overwrite the disturbance state: current [2, n] (NED, m/s) and bias [3, n] (N, N, Nm), either nullable.  The values hold
+ * until that env's next reset.  Needs an enabled disturbance. */
+ML4CA_API int ml4ca_env_set_disturbance_state(ml4ca_env* env, const float* current, const float* bias, void* stream);
+/* Copies of the disturbance state: current [2, n], bias [3, n], either nullable.  Needs an enabled disturbance. */
+ML4CA_API int ml4ca_env_get_disturbance(ml4ca_env* env, float* current, float* bias, void* stream);
+
 /* Stateless pieces of the wrapper, exposed for callers that own their own state (and for parity tests):
  * ErrorFrame.transform (errorFrame.py:25-32): eta, ref [3, n] -> err [3, n] body-frame error. */
 ML4CA_API int ml4ca_error_frame(int64_t n, const float* eta, const float* ref, float* err, void* stream);

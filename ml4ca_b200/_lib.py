@@ -27,6 +27,15 @@ class EnvCfg(ctypes.Structure):
     ]
 
 
+class DisturbanceCfg(ctypes.Structure):
+    """struct ml4ca_disturbance_cfg"""
+    _fields_ = [
+        ("current_speed_min", ctypes.c_float), ("current_speed_max", ctypes.c_float),
+        ("current_dir_min", ctypes.c_float), ("current_dir_max", ctypes.c_float),
+        ("bias_std", ctypes.c_float * 3), ("bias_time_s", ctypes.c_float),
+    ]
+
+
 class PolicyCfg(ctypes.Structure):
     """struct ml4ca_policy_cfg"""
     _fields_ = [("obs_dim", ctypes.c_int32), ("act_dim", ctypes.c_int32), ("hidden", ctypes.c_int32),
@@ -59,6 +68,9 @@ _SIGNATURES = {
     "ml4ca_env_step_host": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_u8p, c_stream]),
     "ml4ca_env_get_state": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_f32p, c_i32p, c_stream]),
     "ml4ca_env_size": (ctypes.c_int64, [ctypes.c_void_p]),
+    "ml4ca_env_set_disturbance": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(DisturbanceCfg), c_stream]),
+    "ml4ca_env_set_disturbance_state": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_stream]),
+    "ml4ca_env_get_disturbance": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_stream]),
     "ml4ca_error_frame": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_stream]),
     "ml4ca_scale_and_clip": (ctypes.c_int, [ctypes.POINTER(EnvCfg), ctypes.c_int64, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),
     "ml4ca_pinv_pid": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_stream]),

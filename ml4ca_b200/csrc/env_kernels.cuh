@@ -29,6 +29,10 @@
                                  // 0.514 ms against 0.504 ms per 16 Mi envs over 200 steps)
 #endif
 
+#ifndef ML4CA_ENV_MIN_BLOCKS_DIST
+#define ML4CA_ENV_MIN_BLOCKS_DIST 4  // disturbed step: 64 registers; 40 would spill around the Philox / Box-Muller draws
+#endif
+
 namespace ml4ca {
 
 struct EnvParams {
@@ -57,6 +61,15 @@ struct EnvParams {
   int64_t count, io_stride;
 };
 
+// Environmental disturbance (ml4ca_env_set_disturbance).  Passed as the LAST argument of the step kernel rather than
+// inside EnvParams: the arguments of the kernels without disturbance then keep their parameter-bank offsets, and
+// their code stays what it was.  Both pointers are NULL while no disturbance is enabled.
+struct DistParams {
+  float* current;      // [2, n] NED current (m/s) of the episode
+  float* bias;         // [3, n] NED bias force (N, N, Nm)
+  DistConsts k;
+};
+
 }  // namespace ml4ca
 
 namespace ml4ca {
@@ -79,8 +92,10 @@ struct ml4ca_env {
   int32_t device;
   void* slab;
   ml4ca::HostPipe* pipe = nullptr;
+  void* dist_slab = nullptr;  // current [2, n] + bias [3, n] rows, allocated when a disturbance is first enabled
   bool tail_valid;     // obs_tail rows describe the last returned observation (true after a reset, false after a step)
   ml4ca::EnvParams p;
+  ml4ca::DistParams dist = {};
 };
 
 namespace ml4ca {
@@ -155,12 +170,17 @@ __device__ __forceinline__ void st_flags(uint8_t* __restrict__ row, int64_t i, c
 
 // ---- K3 ------------------------------------------------------------------------------------------------------------
 // LAG = true (one env per thread only): the wrench lag of cfg.actuator_lag_s, three more state rows in and out.
-template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false>
-__global__ void __launch_bounds__(256, VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1)) env_step_kernel(const EnvParams p, const float* __restrict__ action,
+// DIST = true (one env per thread only): the ocean current and the bias force of ml4ca_env_set_disturbance.  The hull
+// recurrence runs unchanged on the velocity relative to the water, nu_r = nu - R(psi0)^T v_c, with the bias added to
+// the wrench as R(psi0)^T b (after the lag); the pose then drifts by n_sub h v_c and nu = nu_r + R(psi1)^T v_c is the
+// velocity over ground again.  20 B more read (current, bias) and 12 B more written (bias) per env-step: 209 B.
+template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false>
+__global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
                                                        float* __restrict__ obs, float* __restrict__ rew,
-                                                       uint8_t* __restrict__ done) {
+                                                       uint8_t* __restrict__ done, const DistParams d) {
   using T = EnvTraits<KIND, CONT>;
   static_assert(!LAG || VEC == 1, "the lagged integrator is scalar");
+  static_assert(!DIST || VEC == 1, "the disturbed step is scalar");
   const int64_t n = p.n, ios = p.io_stride;
   const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
   if (i0 >= p.count) return;
@@ -193,6 +213,13 @@ __global__ void __launch_bounds__(256, VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC ==
   if constexpr (LAG) {
 #pragma unroll
     for (int c = 0; c < 3; ++c) ld_row<VEC>(p.tau_act + (int64_t)c * n, i0, tact[c]);
+  }
+  float cur[2][VEC], bia[3][VEC];
+  if constexpr (DIST) {
+#pragma unroll
+    for (int c = 0; c < 2; ++c) ld_row<VEC>(d.current + (int64_t)c * n, i0, cur[c]);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) ld_row<VEC>(d.bias + (int64_t)c * n, i0, bia[c]);
   }
 
   float o[9][VEC], rw[VEC];
@@ -235,7 +262,28 @@ __global__ void __launch_bounds__(256, VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC ==
   }
   // ---- phase B: dTwin.step(n_steps), :124 ---------------------------------------------------------------------------
   if (p.n_sub > 0) {
-    if constexpr (LAG) {
+    if constexpr (DIST) {                                              // VEC == 1
+      const float cN = cur[0][0], cE = cur[1][0];
+      float s0, c0;
+      sincos_heading(eta[2][0], s0, c0);
+      nu[0][0] -= fmaf(c0, cN, s0 * cE);                               // nu_r = nu - R(psi0)^T v_c
+      nu[1][0] -= fmaf(c0, cE, -s0 * cN);
+      const float fx = fmaf(c0, bia[0][0], s0 * bia[1][0]);            // R(psi0)^T b, held over the sub-steps
+      const float fy = fmaf(c0, bia[1][0], -s0 * bia[0][0]);
+      if constexpr (LAG) {
+        integrate_hull_lag<true>(eta[0][0], eta[1][0], eta[2][0], nu[0][0], nu[1][0], nu[2][0], wx[0], wy[0], wn[0],
+                                 tact[0][0], tact[1][0], tact[2][0], p.n_sub, p.hull, fx, fy, bia[2][0]);
+      } else {
+        integrate_hull(eta[0][0], eta[1][0], eta[2][0], nu[0][0], nu[1][0], nu[2][0], wx[0] + fx, wy[0] + fy,
+                       wn[0] + bia[2][0], p.n_sub, p.hull);
+      }
+      eta[0][0] = fmaf(d.k.t_step, cN, eta[0][0]);                  // + n_sub h v_c
+      eta[1][0] = fmaf(d.k.t_step, cE, eta[1][0]);
+      float s1, c1;
+      sincos_heading(eta[2][0], s1, c1);
+      nu[0][0] += fmaf(c1, cN, s1 * cE);                               // back to the velocity over ground
+      nu[1][0] += fmaf(c1, cE, -s1 * cN);
+    } else if constexpr (LAG) {
       integrate_hull_lag(eta[0][0], eta[1][0], eta[2][0], nu[0][0], nu[1][0], nu[2][0], wx[0], wy[0], wn[0], tact[0][0],
                          tact[1][0], tact[2][0], p.n_sub, p.hull);
     } else if constexpr (VEC == 2) {                                   // two envs per thread: packed FP32 pipe
@@ -279,6 +327,9 @@ __global__ void __launch_bounds__(256, VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC ==
     for (int c = 0; c < 3; ++c) pth[c][j] = thrust[c];
     any_reset |= (flags[j] != 0u);
   }
+  if constexpr (DIST) {                                                // the step applied b's value at its start
+    if (d.k.gm) advance_bias(p.seed, p.env_off + i0, ep[0], d.k, bia[0][0], bia[1][0], bia[2][0]);
+  }
 
   if (p.auto_reset && any_reset) {  // rare (1 / episode length): keeps the RNG off the common path
 #pragma unroll
@@ -292,6 +343,12 @@ __global__ void __launch_bounds__(256, VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC ==
                    nu[1][j], nu[2][j]);
       ang[0][j] = T::DEF_BOW, ang[1][j] = T::DEF_PORT, ang[2][j] = T::DEF_STAR;
       if constexpr (LAG) tact[0][j] = tact[1][j] = tact[2][j] = 0.f;
+      if constexpr (DIST) {                                            // a new current and bias (old episode word)
+        float cj[2], bj[3];
+        sample_disturbance(p.seed, p.env_off + i0 + j, ep[j], d.k, cj, bj);
+        d.current[i0 + j] = cj[0], d.current[n + i0 + j] = cj[1];
+        bia[0][j] = bj[0], bia[1][j] = bj[1], bia[2][j] = bj[2];
+      }
       float t0[3] = {0.f, 0.f, 0.f};                                   // customEnv.py:190
       if (p.reset_acts) sample_reset_thrust(p.seed, p.env_off + i0 + j, ep[j], t0);   // :179-188 (old episode word)
       ep[j] = next_episode_word(ep[j]);
@@ -316,6 +373,10 @@ __global__ void __launch_bounds__(256, VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC ==
 #pragma unroll
     for (int c = 0; c < 3; ++c) st_row<VEC>(p.tau_act + (int64_t)c * n, i0, tact[c]);
   }
+  if constexpr (DIST) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) st_row<VEC>(d.bias + (int64_t)c * n, i0, bia[c]);
+  }
 #pragma unroll
   for (int c = 0; c < (EXT ? 9 : 6); ++c) st_row<VEC>(obs + (int64_t)c * ios, i0, o[c]);
   st_row<VEC>(rew, i0, rw);
@@ -328,7 +389,7 @@ template <int KIND, bool CONT, bool EXT>
 __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const uint8_t* __restrict__ mask,
                                                         const float* __restrict__ eta_in,
                                                         const float* __restrict__ nu_in,
-                                                        float* __restrict__ obs) {
+                                                        float* __restrict__ obs, const DistParams d) {
   using T = EnvTraits<KIND, CONT>;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= p.n) return;
@@ -350,6 +411,12 @@ __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const
   p.angles[i] = T::DEF_BOW, p.angles[n + i] = T::DEF_PORT, p.angles[2 * n + i] = T::DEF_STAR;  // :173-177,192
   p.tau_act[i] = 0.f, p.tau_act[n + i] = 0.f, p.tau_act[2 * n + i] = 0.f;
   p.obs_tail[i] = div100(t0[0]), p.obs_tail[n + i] = div100(t0[1]), p.obs_tail[2 * n + i] = div100(t0[2]);
+  if (d.current != nullptr) {                                                          // disturbance enabled
+    float cur[2], b[3];
+    sample_disturbance(p.seed, p.env_off + i, epi, d.k, cur, b);
+    d.current[i] = cur[0], d.current[n + i] = cur[1];
+    d.bias[i] = b[0], d.bias[n + i] = b[1], d.bias[2 * n + i] = b[2];
+  }
   p.ep_len[i] = next_episode_word(epi);
   if (obs != nullptr) {
     float xb, yb, pb;

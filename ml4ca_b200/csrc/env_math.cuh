@@ -299,9 +299,12 @@ __device__ __forceinline__ void integrate_hull(float& N, float& E, float& psi, f
 // integrate_hull with a first-order lag of the thruster wrench (ml4ca_env_cfg.actuator_lag_s > 0; oracle/vessel.py):
 // tau_act is a state of the env; every sub-step first moves it towards the command by lag_k, then advances the hull with it.
 // Nine more FP32 instructions per sub-step than integrate_hull.
+// FORCE: (fx, fy, fn) is a body-frame force added to the lagged wrench (the environmental bias, which is not lagged).
+template <bool FORCE = false>
 __device__ __forceinline__ void integrate_hull_lag(float& N, float& E, float& psi, float& u, float& v, float& r,
                                                    float tx, float ty, float tn, float& ta_x, float& ta_y, float& ta_n,
-                                                   int n_sub, const HullConsts& k) {
+                                                   int n_sub, const HullConsts& k, float fx = 0.f, float fy = 0.f,
+                                                   float fn = 0.f) {
   float s, c;
   sincos_heading(psi, s, c);
   float sN = 0.f, sE = 0.f, sr = 0.f;
@@ -311,9 +314,10 @@ __device__ __forceinline__ void integrate_hull_lag(float& N, float& E, float& ps
     ta_y = fmaf(k.lag_k, ty - ta_y, ta_y);
     ta_n = fmaf(k.lag_k, tn - ta_n, ta_n);
     const float vr = v * r, ur = u * r, uv = u * v;
-    const float un = fmaf(fmaf(-k.xuu, fabsf(u), k.one_xu), u, fmaf(k.k_vr, vr, k.hm1 * ta_x));
-    const float vn = fmaf(fmaf(-k.yvv, fabsf(v), k.one_yv), v, fmaf(-k.k_ur, ur, k.hm2 * ta_y));
-    const float rn = fmaf(fmaf(-k.nrr, fabsf(r), k.one_nr), r, fmaf(-k.k_uv, uv, k.hm3 * ta_n));
+    const float fx_ = FORCE ? ta_x + fx : ta_x, fy_ = FORCE ? ta_y + fy : ta_y, fn_ = FORCE ? ta_n + fn : ta_n;
+    const float un = fmaf(fmaf(-k.xuu, fabsf(u), k.one_xu), u, fmaf(k.k_vr, vr, k.hm1 * fx_));
+    const float vn = fmaf(fmaf(-k.yvv, fabsf(v), k.one_yv), v, fmaf(-k.k_ur, ur, k.hm2 * fy_));
+    const float rn = fmaf(fmaf(-k.nrr, fabsf(r), k.one_nr), r, fmaf(-k.k_uv, uv, k.hm3 * fn_));
     u = un;
     v = vn;
     r = rn;
@@ -444,7 +448,7 @@ __device__ __forceinline__ void sample_reset(uint64_t seed, int64_t env_id, int3
   const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ 0x5EED5EEDu;
   const uint32_t lo = (uint32_t)((uint64_t)env_id), hi = (uint32_t)((uint64_t)env_id >> 32);
   // one Philox block = 128 bits = six 21-bit uniforms (resolution 2^-20 of each interval)
-  const Philox4 q = philox4x32_10(lo, hi, (uint32_t)episode, 0u, k0, k1);
+  const Philox4 q = philox4x32_10(lo, hi, (uint32_t)episode, kTagResetPose, k0, k1);
   N = __fmul_rn(scale[0], symmetric_unit21(q.x));
   E = __fmul_rn(scale[1], symmetric_unit21(q.y));
   psi = __fmul_rn(scale[2], symmetric_unit21(q.z));
@@ -453,22 +457,85 @@ __device__ __forceinline__ void sample_reset(uint64_t seed, int64_t env_id, int3
   r = __fmul_rn(scale[5], symmetric_unit21(((q.z >> 21) | (q.w >> 21 << 11)) & 0x1FFFFFu));
 }
 
+// Three standard normals from one Philox block of (env, episode word, tag): Box-Muller on (x, y) -> r0 cos, r0 sin and
+// on (z, w) -> r1 cos, with r = sqrt(-2 ln unit_open(.)), angle = 2 pi (. >> 8) 2^-24 (tests/disturbance_oracle.py::normals3).
+__device__ __forceinline__ void philox_normals3(uint64_t seed, int64_t env_id, int32_t episode, uint32_t tag,
+                                                float (&z)[3]) {
+  const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ 0x5EED5EEDu;
+  const uint32_t lo = (uint32_t)((uint64_t)env_id), hi = (uint32_t)((uint64_t)env_id >> 32);
+  const Philox4 q = philox4x32_10(lo, hi, (uint32_t)episode, tag, k0, k1);
+  const float r0 = sqrtf(-2.0f * logf(unit_open(q.x))), r1 = sqrtf(-2.0f * logf(unit_open(q.z)));
+  float s0, c0, s1, c1;
+  sincospif((float)(q.y >> 8) * 1.1920928955078125e-07f, &s0, &c0);   // angle = 2 pi * (y >> 8) * 2^-24
+  sincospif((float)(q.w >> 8) * 1.1920928955078125e-07f, &s1, &c1);
+  z[0] = r0 * c0, z[1] = r0 * s0, z[2] = r1 * c1;
+}
+
 // customEnv.py:179-188 (reset_acts=True): prev_thrust <- scale_and_clip([N(0, 0.1)]^3) = clip(100 * (0.1 z), +-100);
 // the thrust commands themselves only reach the simulator after the settle steps and are overwritten by the next
 // step's action, so the previous-thrust state (observation tail + first derivative penalty) is the whole effect.
 // Second Philox block of the restart (counter word 3 = 1), Box-Muller on (x, y) and (z, w).  Rare path: kept out
 // of line so that logf / sincospif do not enter the step kernel's register budget.
 static __device__ __noinline__ void sample_reset_thrust(uint64_t seed, int64_t env_id, int32_t episode, float* __restrict__ t) {
-  const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ 0x5EED5EEDu;
-  const uint32_t lo = (uint32_t)((uint64_t)env_id), hi = (uint32_t)((uint64_t)env_id >> 32);
-  const Philox4 q = philox4x32_10(lo, hi, (uint32_t)episode, 1u, k0, k1);
-  const float r0 = sqrtf(-2.0f * logf(unit_open(q.x))), r1 = sqrtf(-2.0f * logf(unit_open(q.z)));
-  float s0, c0, s1, c1;
-  sincospif((float)(q.y >> 8) * 1.1920928955078125e-07f, &s0, &c0);   // angle = 2 pi * (y >> 8) * 2^-24
-  sincospif((float)(q.w >> 8) * 1.1920928955078125e-07f, &s1, &c1);
-  const float z[3] = {r0 * c0, r0 * s0, r1 * c1};
+  float z[3];
+  philox_normals3(seed, env_id, episode, kTagResetThrust, z);
 #pragma unroll
   for (int c = 0; c < 3; ++c) t[c] = fminf(fmaxf(__fmul_rn(__fmul_rn(0.1f, z[c]), 100.0f), -100.0f), 100.0f);
+}
+
+// ---- environmental disturbance (DECLARED model, DESIGN.md section 4; tests/disturbance_oracle.py) ------------------------------
+// Ocean current v_c = V [cos beta, sin beta] (NED, constant over an episode) and a NED bias force b = [X_N, Y_E, N_psi]
+// following the first-order Gauss-Markov process b <- a b + sigma sqrt(1 - a^2) w per env step, a = exp(-step_dt / T_b)
+// (T_b = 0: a = 1, constant over the episode).  Per-launch constants, folded on the host (ml4ca_env_set_disturbance).
+struct DistConsts {
+  float speed_lo, speed_span;   // V ~ U(speed_lo, speed_lo + speed_span), m/s
+  float dir_lo, dir_span;       // beta ~ U(dir_lo, dir_lo + dir_span), rad: the direction the water flows towards
+  float bias_std[3];            // sigma: stationary std of b (N, N, Nm); a reset draws b = sigma w0
+  float gm_a;                   // a
+  float gm_gain[3];             // sigma sqrt(1 - a^2)
+  float t_step;                 // n_sub * h: time one env step integrates (drift of the pose with the current)
+  int32_t gm;                   // 1: b is updated every env step (T_b > 0)
+  int32_t noise;                // 1: ... with a random term (some sigma > 0); 0: b <- a b only
+};
+
+// Uniform in [0, 1) from the top 24 bits: (x >> 8) * 2^-24, exact in fp32.
+__device__ __forceinline__ float unit01(uint32_t x) { return (float)(x >> 8) * 5.9604644775390625e-08f; }
+
+// Current of a new episode: third Philox block of the restart (counter word 3 = kTagCurrent); speed from x, direction
+// from y.  `episode` is the episode word at the moment of the reset, as for sample_reset.
+__device__ __forceinline__ void sample_current(uint64_t seed, int64_t env_id, int32_t episode, const DistConsts& d,
+                                               float& cN, float& cE) {
+  const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ 0x5EED5EEDu;
+  const uint32_t lo = (uint32_t)((uint64_t)env_id), hi = (uint32_t)((uint64_t)env_id >> 32);
+  const Philox4 q = philox4x32_10(lo, hi, (uint32_t)episode, kTagCurrent, k0, k1);
+  const float V = fmaf(d.speed_span, unit01(q.x), d.speed_lo);
+  const float beta = fmaf(d.dir_span, unit01(q.y), d.dir_lo);
+  float s, c;
+  sincosf(beta, &s, &c);
+  cN = V * c;
+  cE = V * s;
+}
+
+// The disturbance state of a new episode: the current and b = sigma w0 (stationary draw, counter word 3 = kTagBias0).
+// Rare path (resets only), kept out of line like sample_reset_thrust.
+static __device__ __noinline__ void sample_disturbance(uint64_t seed, int64_t env_id, int32_t episode, const DistConsts& d,
+                                                       float* __restrict__ cur, float* __restrict__ b) {
+  sample_current(seed, env_id, episode, d, cur[0], cur[1]);
+  float z[3];
+  philox_normals3(seed, env_id, episode, kTagBias0, z);
+#pragma unroll
+  for (int c = 0; c < 3; ++c) b[c] = d.bias_std[c] * z[c];
+}
+
+// One env step of the Gauss-Markov bias.  `word` is the episode word AFTER the step's increment (counter word 3 =
+// kTagBiasStep): every step of every episode has its own block, so a replayed CUDA graph draws fresh noise.
+__device__ __forceinline__ void advance_bias(uint64_t seed, int64_t env_id, int32_t word, const DistConsts& d,
+                                             float& bN, float& bE, float& bP) {
+  float z[3] = {0.f, 0.f, 0.f};
+  if (d.noise) philox_normals3(seed, env_id, word, kTagBiasStep, z);
+  bN = fmaf(d.gm_gain[0], z[0], d.gm_a * bN);
+  bE = fmaf(d.gm_gain[1], z[1], d.gm_a * bE);
+  bP = fmaf(d.gm_gain[2], z[2], d.gm_a * bP);
 }
 
 }  // namespace ml4ca

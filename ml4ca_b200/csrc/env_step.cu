@@ -2,6 +2,7 @@
 // Kernels: env_kernels.cuh; per-class instantiations: env_step_inst.cu.
 #include <stdlib.h>
 
+#include <cmath>
 #include <new>
 
 #include "env_kernels.cuh"
@@ -67,6 +68,50 @@ static int validate_cfg(const ml4ca_env_cfg* c) {
   return ML4CA_OK;
 }
 
+static int validate_disturbance(const ml4ca_disturbance_cfg* d) {
+  ML4CA_REQUIRE(std::isfinite(d->current_speed_min) && std::isfinite(d->current_speed_max) &&
+                    std::isfinite(d->current_dir_min) && std::isfinite(d->current_dir_max) &&
+                    std::isfinite(d->bias_time_s) && std::isfinite(d->bias_std[0]) && std::isfinite(d->bias_std[1]) &&
+                    std::isfinite(d->bias_std[2]),
+                "disturbance: every field must be finite");
+  ML4CA_REQUIRE(d->current_speed_min >= 0.f && d->current_speed_min <= d->current_speed_max,
+                "disturbance: current speed range needs 0 <= current_speed_min <= current_speed_max");
+  ML4CA_REQUIRE(d->current_dir_min <= d->current_dir_max, "disturbance: current direction range needs current_dir_min <= current_dir_max");
+  ML4CA_REQUIRE(d->bias_std[0] >= 0.f && d->bias_std[1] >= 0.f && d->bias_std[2] >= 0.f,
+                "disturbance: bias_std must be non-negative");
+  ML4CA_REQUIRE(d->bias_time_s >= 0.f, "disturbance: bias_time_s must be non-negative (0 = constant over the episode)");
+  return ML4CA_OK;
+}
+
+// Per-launch constants of the disturbance (env_math.cuh: DistConsts).
+static DistConsts dist_consts(const ml4ca_env_cfg& c, const ml4ca_disturbance_cfg& d) {
+  DistConsts k;
+  k.speed_lo = d.current_speed_min;
+  k.speed_span = d.current_speed_max - d.current_speed_min;
+  k.dir_lo = d.current_dir_min;
+  k.dir_span = d.current_dir_max - d.current_dir_min;
+  const double a = d.bias_time_s > 0.f ? std::exp(-(double)c.step_dt / (double)d.bias_time_s) : 1.0;
+  k.gm_a = (float)a;
+  for (int i = 0; i < 3; ++i) {
+    k.bias_std[i] = d.bias_std[i];
+    k.gm_gain[i] = (float)((double)d.bias_std[i] * std::sqrt(1.0 - a * a));
+  }
+  k.t_step = (float)((double)c.n_substeps * (double)c.sim_dt);
+  k.gm = d.bias_time_s > 0.f ? 1 : 0;
+  k.noise = (k.gm && (d.bias_std[0] > 0.f || d.bias_std[1] > 0.f || d.bias_std[2] > 0.f)) ? 1 : 0;
+  return k;
+}
+
+// The disturbance state of every env, drawn as a reset would draw it (episode word of the moment).
+__global__ void __launch_bounds__(256) draw_disturbance_kernel(const EnvParams p, const DistParams d) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
+  if (i >= n) return;
+  float cur[2], b[3];
+  sample_disturbance(p.seed, p.env_off + i, p.ep_len[i], d.k, cur, b);
+  d.current[i] = cur[0], d.current[n + i] = cur[1];
+  d.bias[i] = b[0], d.bias[n + i] = b[1], d.bias[2 * n + i] = b[2];
+}
+
 static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&scale)[6]) {
   // fp32, one rounding per product, same order as oracle/env_oracle.py::sample_reset
   const float vfr = (float)ML4CA_VEL_FRACTION * fraction;
@@ -75,7 +120,8 @@ static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&sca
 }
 
 #define ML4CA_DECL_UNIT(name)                                                                                   \
-  int launch_step_##name(const ml4ca_env*, const EnvParams&, const float*, float*, float*, uint8_t*, cudaStream_t); \
+  int launch_step_##name(const ml4ca_env*, const EnvParams&, const DistParams&, const float*, float*, float*, uint8_t*, \
+                         cudaStream_t);                                                                            \
   int launch_reset_##name(const ml4ca_env*, const EnvParams&, const uint8_t*, const float*, const float*, float*, \
                           cudaStream_t);
 ML4CA_DECL_UNIT(full)
@@ -93,16 +139,18 @@ static int launch_step(const ml4ca_env* e, int64_t first, int64_t count, int64_t
   p.tau_act += first;
   p.ep_len += first;
   if (p.cut_obs != nullptr) p.cut_obs += first;
+  DistParams d = e->dist;
+  if (d.current != nullptr) d.current += first, d.bias += first;
   p.env_off += first;
   p.count = count;
   p.io_stride = io_stride;
   switch (e->cfg.kind) {
-    case ML4CA_ENV_FULL: return launch_step_full(e, p, action, obs, rew, done, st);
-    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, action, obs, rew, done, st);
-    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, action, obs, rew, done, st);
+    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, action, obs, rew, done, st);
+    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, action, obs, rew, done, st);
+    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, action, obs, rew, done, st);
     default:
-      return e->cfg.cont_ang ? launch_step_final_cont(e, p, action, obs, rew, done, st)
-                             : launch_step_final_wrap(e, p, action, obs, rew, done, st);
+      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, action, obs, rew, done, st)
+                             : launch_step_final_wrap(e, p, d, action, obs, rew, done, st);
   }
 }
 
@@ -244,6 +292,7 @@ int ml4ca_env_destroy(ml4ca_env* env) {
     cudaFree(hp->slab);
     delete hp;
   }
+  cudaFree(env->dist_slab);
   cudaFree(env->slab);
   delete env;
   return ML4CA_OK;
@@ -280,6 +329,47 @@ int ml4ca_env_set_reset_fraction(ml4ca_env* env, float fraction) {
   ML4CA_REQUIRE(fraction >= 0.f, "fraction must be non-negative");
   env->cfg.reset_fraction = fraction;
   make_reset_scale(env->cfg, fraction, env->p.reset_scale);
+  return ML4CA_OK;
+}
+
+int ml4ca_env_set_disturbance(ml4ca_env* env, const ml4ca_disturbance_cfg* cfg, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  if (cfg == nullptr) {
+    env->dist.current = env->dist.bias = nullptr;     // the rows stay allocated for a later enable
+    return ML4CA_OK;
+  }
+  int stv = validate_disturbance(cfg);
+  if (stv != ML4CA_OK) return stv;
+  DeviceGuard guard(env->device);
+  const int64_t n = env->n;
+  if (env->dist_slab == nullptr) ML4CA_CUDA(cudaMalloc(&env->dist_slab, 5 * (size_t)n * sizeof(float) + 256));
+  float* f = static_cast<float*>(env->dist_slab);
+  env->dist.current = f;
+  env->dist.bias = f + 2 * n;
+  env->dist.k = dist_consts(env->cfg, *cfg);
+  draw_disturbance_kernel<<<(unsigned)((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(env->p, env->dist);
+  return check_launch("draw_disturbance_kernel");
+}
+
+int ml4ca_env_set_disturbance_state(ml4ca_env* env, const float* current, const float* bias, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  ML4CA_REQUIRE(env->dist.current != nullptr, "no disturbance is enabled (ml4ca_env_set_disturbance)");
+  DeviceGuard guard(env->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t row = (size_t)env->n * sizeof(float);
+  if (current) ML4CA_CUDA(cudaMemcpyAsync(env->dist.current, current, 2 * row, cudaMemcpyDeviceToDevice, st));
+  if (bias) ML4CA_CUDA(cudaMemcpyAsync(env->dist.bias, bias, 3 * row, cudaMemcpyDeviceToDevice, st));
+  return ML4CA_OK;
+}
+
+int ml4ca_env_get_disturbance(ml4ca_env* env, float* current, float* bias, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  ML4CA_REQUIRE(env->dist.current != nullptr, "no disturbance is enabled (ml4ca_env_set_disturbance)");
+  DeviceGuard guard(env->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t row = (size_t)env->n * sizeof(float);
+  if (current) ML4CA_CUDA(cudaMemcpyAsync(current, env->dist.current, 2 * row, cudaMemcpyDeviceToDevice, st));
+  if (bias) ML4CA_CUDA(cudaMemcpyAsync(bias, env->dist.bias, 3 * row, cudaMemcpyDeviceToDevice, st));
   return ML4CA_OK;
 }
 

@@ -8,6 +8,14 @@
 
 namespace ml4ca {
 
+// Counter = (env id lo, env id hi, episode word, tag): the tag (counter word 3) keeps the streams of one env and episode
+// word apart.  Every new stream takes a tag no other stream uses.
+constexpr uint32_t kTagResetPose = 0u;     // sample_reset: pose and velocity of a new episode
+constexpr uint32_t kTagResetThrust = 1u;   // sample_reset_thrust: previous thrust of a new episode (reset_acts)
+constexpr uint32_t kTagCurrent = 2u;       // sample_current: ocean current of a new episode (speed, direction)
+constexpr uint32_t kTagBias0 = 3u;         // sample_disturbance: bias force of a new episode (stationary draw)
+constexpr uint32_t kTagBiasStep = 4u;      // advance_bias: Gauss-Markov noise of one env step (word after the step)
+
 struct Philox4 {
   uint32_t x, y, z, w;
 };

@@ -201,6 +201,7 @@ class Revolt(object):
         self._rew = torch.empty(n, dtype=torch.float32, device=self.device)
         self._done = torch.empty(n, dtype=torch.uint8, device=self.device)
         self._has_reset = False          # self._obs holds nothing until the first reset()
+        self._disturbance = None         # the arguments of the last set_disturbance(), None = calm water
         self.EF = _EnvErrorFrame(self)
 
     # -- per-class tables (customEnv.py:58-65); subclasses override --------------------------------
@@ -345,6 +346,41 @@ class Revolt(object):
         self._cfg.reset_fraction = float(fraction)
         _lib.check(_lib.lib().ml4ca_env_set_reset_fraction(self._handle, float(fraction)), "ml4ca_env_set_reset_fraction")
 
+    def set_disturbance(self, current_speed=(0.0, 0.0), current_direction=(0.0, 2 * np.pi), bias_std=(0.0, 0.0, 0.0),
+                        bias_time_s=0.0):
+        """Environmental loads (the declared model of DESIGN.md section 4); ``set_disturbance(None)`` is calm water again.
+
+        Every reset (explicit or in-kernel) draws an ocean current, constant in the NED frame over the episode, with speed
+        ~ U(current_speed) m/s and direction ~ U(current_direction) rad (the direction the water flows towards: 0 = north,
+        pi/2 = east), and a NED bias force b = [X_N, Y_E, N_psi] (N, N, Nm) with standard deviation ``bias_std``.  b follows
+        a first-order Gauss-Markov process with time constant ``bias_time_s`` (0 = constant over the episode).  Enabling
+        draws the state of every env at once.  0 to 0.2 m/s is the useful current range: a 0.3 m/s beam current takes all
+        of the sway thrust.  Like the restart fraction, the setting is a launch parameter: CUDA graphs captured earlier
+        keep theirs."""
+        with torch.cuda.device(self.device):
+            if current_speed is None:
+                _lib.check(_lib.lib().ml4ca_env_set_disturbance(self._handle, None, self._stream()), "ml4ca_env_set_disturbance")
+                self._disturbance = None
+                return
+            c = _lib.DisturbanceCfg()
+            c.current_speed_min, c.current_speed_max = (float(x) for x in current_speed)
+            c.current_dir_min, c.current_dir_max = (float(x) for x in current_direction)
+            for i, x in enumerate(bias_std):
+                c.bias_std[i] = float(x)
+            c.bias_time_s = float(bias_time_s)
+            _lib.check(_lib.lib().ml4ca_env_set_disturbance(self._handle, ctypes.byref(c), self._stream()),
+                       "ml4ca_env_set_disturbance")
+        self._disturbance = (tuple(current_speed), tuple(current_direction), tuple(bias_std), float(bias_time_s))
+
+    def set_disturbance_state(self, current=None, bias=None):
+        """Overwrite the disturbance state: ``current`` [2, num_envs] (NED, m/s), ``bias`` [3, num_envs] (N, N, Nm); either
+        may be None.  The values hold until that env's next reset."""
+        cur = None if current is None else self._to_device(current, 2)[0]
+        b = None if bias is None else self._to_device(bias, 3)[0]
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().ml4ca_env_set_disturbance_state(self._handle, _lib.ptr(cur), _lib.ptr(b), self._stream()),
+                       "ml4ca_env_set_disturbance_state")
+
     def observe(self):
         """state() / state_extended() (customEnv.py:196-205) of the current device-side state."""
         obs = torch.empty_like(self._obs)
@@ -361,6 +397,10 @@ class Revolt(object):
             _lib.check(_lib.lib().ml4ca_env_get_state(self._handle, _lib.ptr(st["eta"]), _lib.ptr(st["nu"]),
                                                       _lib.ptr(st["prev_thrust"]), _lib.ptr(st["angles"]),
                                                       _lib.ptr(st["ep_len"]), self._stream()))
+            if self._disturbance is not None:   # current [2, n] (NED, m/s) and bias [3, n] (N, N, Nm) of the episode
+                st["current"], st["bias"] = f(2), f(3)
+                _lib.check(_lib.lib().ml4ca_env_get_disturbance(self._handle, _lib.ptr(st["current"]), _lib.ptr(st["bias"]),
+                                                                self._stream()), "ml4ca_env_get_disturbance")
         return st
 
     @property

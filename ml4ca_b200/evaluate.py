@@ -22,11 +22,16 @@ def fixed_test_poses(n):
     return np.stack([5 * np.sin(ang), 5 * np.cos(ang), np.deg2rad(np.asarray(FIXED_ANGLES_DEG)[k])])
 
 
-def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None):
+def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False):
     """test_policy.py:97-186 for every env of ``env`` at once (one episode each, no early stop: finished runs keep
     being recorded, ``done_at`` tells where the reference loop would have cut).  Returns a dict of device tensors:
     obs [T+1, obs, n], rew [T, n], eta [T+1, 3, n], thrust [T+1, 3, n], angles [T+1, 2, n], done_at [n], ep_ret [n],
-    metrics [3, n] = IAE, W*, IADC."""
+    metrics [3, n] = IAE, W*, IADC.
+
+    integrator=True: the thesis' ``RLintegral`` configuration.  The policy's three error rows come from the deployment
+    node's state assembly with its body-frame integrator (ml4ca_ros_state, rl_allocator.py:252-273, one env step = h):
+    the error plus an integral that starts 5 s after the vessel entered the 5 m / 140 deg zone.  ``obs`` keeps the env's
+    own observation; the final integrator state is returned as ``integrator`` [3, n]."""
     n, dev = env.num_envs, env.device
     T = int(max_ep_len if max_ep_len is not None else env.max_ep_len)
     eta0 = fixed_test_poses(n)
@@ -41,8 +46,22 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None):
     st = env.get_state()
     rec["obs"][0], rec["eta"][0], rec["angles"][0] = o, st["eta"], st["angles"][1:3]
     ref = env._ref.clone()
+    if integrator:
+        integ, t_inside = torch.zeros(3, n, **f), torch.zeros(n, **f)
+        prev_u, ros = torch.zeros(6, n, **f), torch.empty(9, n, **f)       # ROS-order previous thrust: rows 6-8 unused here
+
+    def policy_input(o, st):
+        if not integrator:
+            return o
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().ml4ca_ros_state(n, _lib.ptr(st["eta"]), _lib.ptr(st["nu"]), _lib.ptr(ref), _lib.ptr(prev_u),
+                                                  _lib.ptr(integ), _lib.ptr(t_inside), float(env.dt), _lib.ptr(ros),
+                                                  _lib.current_stream()), "ml4ca_ros_state")
+        x = o.clone()
+        x[0:3] = ros[0:3]
+        return x
     for t in range(T):
-        a = ac.get_action(o)                                                 # deterministic action = mu (:90-93)
+        a = ac.get_action(policy_input(o, st))                               # deterministic action = mu (:90-93)
         if ref_change_at is not None and t == ref_change_at and new_ref is not None:
             o, r, d, _ = env.step(torch.zeros_like(a), new_ref=new_ref)      # :141-146
         else:
@@ -56,6 +75,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None):
     steps = torch.arange(T, device=dev)[:, None]
     rec["ep_ret"] = (rec["rew"] * (steps < done_at[None, :])).sum(dim=0)
     rec["metrics"] = metrics(rec["eta"], ref, rec["thrust"], rec["angles"], env.dt)
+    if integrator:
+        rec["integrator"] = integ
     return rec
 
 
