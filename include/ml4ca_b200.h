@@ -279,9 +279,9 @@ ML4CA_API int ml4ca_alloc_to_action(int64_t n, int32_t cont_ang, float ang_bound
  * caller all-reduces them over ranks and divides by the global sample count -- Allreduce(SUM) / num_procs of
  * mpi_tf.py:59-62 with equal shards.  stats (8 doubles, device): [0] sum min(ratio adv, min_adv) (= -N pi_loss),
  * [1] sum (ret - v)^2, [2] sum 0.5 (logp_old - logp)^2 (approx_kl), [3] sum -logp (approx_ent), [4] clipped count,
- * [5] sample count.  Networks: hidden 64 x 64 (the BASELINE training config: tcgen05 kernel, or the register-tiled fp32 one) and
- * any width <= 96 with 1..3 hidden layers -- the reference's own 80 x 80 x 80 (train.py:30-32) and 64 x 64 x 64 -- on the
- * generic fp32 kernel (csrc/ppo_update_generic.cu). */
+ * [5] sample count.  Networks: every one ml4ca_policy_create accepts -- hidden 64 x 64 (the BASELINE training config) and the
+ * reference's own 80 x 80 x 80 (train.py:30-32) and 64 x 64 x 64 -- on the tcgen05 kernel, or with ml4ca_ppo_use_fp32(1) on
+ * the register-tiled fp32 one (64 x 64, obs_dim <= 12) or the generic fp32 kernel (csrc/ppo_update_generic.cu: the others). */
 ML4CA_API int ml4ca_ppo_grad(ml4ca_policy* p, int32_t net, int64_t n, int32_t T, const float* obs, const float* act,
                              const float* adv, const float* ret, const float* logp_old, float clip_ratio, float* grad,
                              double* stats, void* stream);

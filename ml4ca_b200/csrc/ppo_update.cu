@@ -21,13 +21,16 @@
 // Bound: FP32 FMA pipe (~15.6 k FMA per sample and network against 77 B of HBM traffic).  This is the CUDA-core
 // version; moving the three big GEMMs per layer onto tcgen05 (MN-major views of the same smem operands) is
 // round-2 work (DESIGN.md section 3).
+//
+// Host side: every gradient entry point (PPO, TRPO KL, TRPO forward-only) fills one GradArgs (ppo_grad.h) and goes through
+// grad_pass, which picks this kernel, the tcgen05 one (ppo_update_tc.cu) or the generic fp32 one (ppo_update_generic.cu) for
+// the networks ml4ca_policy_create accepts: 64 x 64, 64^3 and 80^3.
 #include <new>
 
 #include <stdlib.h>
 
 #include "common.h"
-#include "ppo_generic.h"
-#include "ppo_tc.h"
+#include "ppo_grad.h"
 
 namespace ml4ca {
 namespace ppo {
@@ -37,31 +40,6 @@ constexpr int RS = 132;   // smem row stride in floats
 constexpr int H = 64;     // hidden width (BASELINE config 64 x 64)
 constexpr int OP = 8;     // padded output width (act_dim <= 7, value head 1)
 constexpr int XR = 12;    // padded input rows (obs_dim <= 12)
-
-struct Args {
-  const float* params;     // flat fp32 master parameters
-  int obs, act, nout;      // nout = act (pi) or 1 (v)
-  int off_w1, off_b1, off_w2, off_b2, off_wo, off_bo, off_ls;   // offsets of this net's variables in params / grad
-  int64_t n;               // envs (row length)
-  int T;
-  const float* obs_buf;    // [T, obs, n]
-  const float* act_buf;    // [T, act, n]    (pi)
-  const float* adv;        // [T, n]         (pi)
-  const float* logp_old;   // [T, n]         (pi)
-  const float* ret;        // [T, n]         (v)
-  float clip;
-  // TRPO (spinup/algos/tf1/trpo): loss_mode 1 = d_kl = mean KL(pi_theta || pi_old) (trpo/core.py:52-60,98) in place of the PPO
-  // surrogate: act_buf then carries mu_old [T, act, n] and kl_ls_old the old log_std [act]; adv / logp_old unused.
-  // mu_out [T, act, n] (nullable): forward only, the means of every sample are stored and no gradient is computed.
-  int loss_mode;
-  const float* kl_ls_old;
-  float* mu_out;
-  float* grad;             // flat, same layout as params; this net's block is accumulated into (caller zeroes)
-  double* stats;           // [8]: 0 sum pi objective, 1 sum (ret - v)^2, 2 sum 0.5 (logp_old - logp)^2, 3 sum -logp,
-                           //      4 clipped count, 5 sample count
-  const int32_t* ctl;      // ml4ca_ppo_ctl (device) or NULL: skip the pass when ctl[0] != 0 && ctl[1] < iter
-  int iter;
-};
 
 // the device-side early stop of the policy loop (include/ml4ca_b200.h: ml4ca_ppo_ctl)
 __device__ __forceinline__ bool pass_skipped(const int32_t* ctl, int iter) {
@@ -118,7 +96,7 @@ __device__ __forceinline__ void gemm_tile(float (&acc)[8][4], const float (*in)[
 }
 
 template <int ACTIVATION, int NET>
-__global__ void __launch_bounds__(256, 1) ppo_grad_kernel(const Args A) {
+__global__ void __launch_bounds__(256, 1) ppo_grad_kernel(const GradArgs A) {
   if (pass_skipped(A.ctl, A.iter)) return;
   extern __shared__ __align__(16) uint8_t smem_raw[];
   Smem& S = *reinterpret_cast<Smem*>(smem_raw);
@@ -128,24 +106,24 @@ __global__ void __launch_bounds__(256, 1) ppo_grad_kernel(const Args A) {
   // ---- weights -> smem (column-permuted copies, see header) -----------------------------------------------------------
   for (int e = tid; e < XR * H; e += 256) {
     const int k = e / H, c = e % H, f = (c >> 2) + 16 * (c & 3);
-    S.w1p[k][c] = k < obs ? A.params[A.off_w1 + k * H + f] : 0.f;
+    S.w1p[k][c] = k < obs ? A.params[A.off_w[0] + k * H + f] : 0.f;
   }
   for (int e = tid; e < H * H; e += 256) {
     const int r = e / H, c = e % H, f = (c >> 2) + 16 * (c & 3);
-    S.w2p[r][c] = A.params[A.off_w2 + r * H + f];      // W2[k = r][j = f]
-    S.w2tp[r][c] = A.params[A.off_w2 + f * H + r];     // W2[k = f][j = r]
+    S.w2p[r][c] = A.params[A.off_w[1] + r * H + f];      // W2[k = r][j = f]
+    S.w2tp[r][c] = A.params[A.off_w[1] + f * H + r];     // W2[k = f][j = r]
   }
   for (int e = tid; e < H * OP; e += 256) {
     const int k = e / OP, o = e % OP;
-    S.wo[k][o] = o < nout ? A.params[A.off_wo + k * nout + o] : 0.f;
+    S.wo[k][o] = o < nout ? A.params[A.off_w[2] + k * nout + o] : 0.f;
   }
   for (int e = tid; e < OP * H; e += 256) {
     const int o = e / H, c = e % H, f = (c >> 2) + 16 * (c & 3);
-    S.wotp[o][c] = o < nout ? A.params[A.off_wo + f * nout + o] : 0.f;
+    S.wotp[o][c] = o < nout ? A.params[A.off_w[2] + f * nout + o] : 0.f;
   }
-  if (tid < H) S.b1[tid] = A.params[A.off_b1 + tid], S.b2[tid] = A.params[A.off_b2 + tid];
+  if (tid < H) S.b1[tid] = A.params[A.off_b[0] + tid], S.b2[tid] = A.params[A.off_b[1] + tid];
   if (tid < OP) {
-    S.bo[tid] = tid < nout ? A.params[A.off_bo + tid] : 0.f;
+    S.bo[tid] = tid < nout ? A.params[A.off_b[2] + tid] : 0.f;
     const float ls = (NET == 0 && tid < nout) ? A.params[A.off_ls + tid] : 0.f;
     const float sd = expf(ls);
     S.ls[tid] = ls, S.sd[tid] = sd, S.inv[tid] = 1.0f / (sd + 1e-8f);
@@ -449,21 +427,21 @@ __global__ void __launch_bounds__(256, 1) ppo_grad_kernel(const Args A) {
 #pragma unroll
   for (int a = 0; a < 4; ++a)
 #pragma unroll
-    for (int b = 0; b < 4; ++b) atomicAdd(g + A.off_w2 + (4 * ty + a) * H + (tx + 16 * b), dW2[a][b]);
+    for (int b = 0; b < 4; ++b) atomicAdd(g + A.off_w[1] + (4 * ty + a) * H + (tx + 16 * b), dW2[a][b]);
   {
     const int k = tid >> 2, o = 2 * (tid & 3);
-    if (o < nout) atomicAdd(g + A.off_wo + k * nout + o, dWo[0]);
-    if (o + 1 < nout) atomicAdd(g + A.off_wo + k * nout + o + 1, dWo[1]);
+    if (o < nout) atomicAdd(g + A.off_w[2] + k * nout + o, dWo[0]);
+    if (o + 1 < nout) atomicAdd(g + A.off_w[2] + k * nout + o + 1, dWo[1]);
     const int j = tid & 63, kq = tid >> 6;
-    if (kq < obs) atomicAdd(g + A.off_w1 + kq * H + j, dW1[0]);
-    if (kq + 4 < obs) atomicAdd(g + A.off_w1 + (kq + 4) * H + j, dW1[1]);
-    if (kq + 8 < obs) atomicAdd(g + A.off_w1 + (kq + 8) * H + j, dW1[2]);
+    if (kq < obs) atomicAdd(g + A.off_w[0] + kq * H + j, dW1[0]);
+    if (kq + 4 < obs) atomicAdd(g + A.off_w[0] + (kq + 4) * H + j, dW1[1]);
+    if (kq + 8 < obs) atomicAdd(g + A.off_w[0] + (kq + 8) * H + j, dW1[2]);
     if ((tid & 3) == 0) {
-      atomicAdd(g + A.off_b1 + (tid >> 2), db1);
-      atomicAdd(g + A.off_b2 + (tid >> 2), db2);
+      atomicAdd(g + A.off_b[0] + (tid >> 2), db1);
+      atomicAdd(g + A.off_b[1] + (tid >> 2), db2);
     }
     const int w = tid >> 5;
-    if ((tid & 31) == 0 && w < nout) atomicAdd(g + A.off_bo + w, dbo);
+    if ((tid & 31) == 0 && w < nout) atomicAdd(g + A.off_b[2] + w, dbo);
   }
   // log_std gradient and statistics: reduce over the 128 sample threads (warps 0-3)
   if (tid < TS) {
@@ -573,101 +551,29 @@ extern "C" int ml4ca_trpo_use_tensor_cores(int enable) {
 static int tc_blob(int32_t device, __half** out) {
   static __half* blob[64] = {};
   ML4CA_REQUIRE(device >= 0 && device < 64, "device index out of range");
-  if (blob[device] == nullptr) ML4CA_CUDA(cudaMalloc(&blob[device], sizeof(__half) * ppotc::kBlobHalves));
+  if (blob[device] == nullptr) ML4CA_CUDA(cudaMalloc(&blob[device], sizeof(__half) * kTcBlobHalves));
   *out = blob[device];
   return ML4CA_OK;
-}
-
-static ppotc::Args tc_args(const ppo::Args& a) {
-  ppotc::Args t = {};
-  t.params = a.params, t.obs = a.obs, t.act = a.act, t.nout = a.nout;
-  t.hidden = 64, t.n_hidden = 2;
-  t.off_w[0] = a.off_w1, t.off_b[0] = a.off_b1, t.off_w[1] = a.off_w2, t.off_b[1] = a.off_b2, t.off_w[2] = a.off_wo;
-  t.off_b[2] = a.off_bo, t.off_ls = a.off_ls;
-  t.n = a.n, t.T = a.T;
-  t.obs_buf = a.obs_buf, t.act_buf = a.act_buf, t.adv = a.adv, t.logp_old = a.logp_old, t.ret = a.ret;
-  t.clip = a.clip, t.loss_mode = a.loss_mode, t.kl_ls_old = a.kl_ls_old, t.mu_out = a.mu_out;
-  t.grad = a.grad, t.stats = a.stats;
-  t.ctl = a.ctl, t.iter = a.iter;
-  return t;
 }
 
 // policy.cu
 extern "C" int ml4ca_policy_describe(const ml4ca_policy* p, ml4ca_policy_cfg* cfg, int32_t* device);
 
-extern "C" {
-
-// Offsets of one network's variables in the flat parameter vector + the checks shared by every pass of this file.
-static int ppo_args(ml4ca_policy* p, int32_t net, int64_t n, int32_t T, const char* who, ppo::Args* out, ml4ca_policy_cfg* cfg_out,
-                    int32_t* device_out) {
-  ML4CA_REQUIRE(p != nullptr, "policy is NULL");
-  ML4CA_REQUIRE(n >= 0 && T >= 0, "bad sizes");
-  ml4ca_policy_cfg cfg;
-  int32_t device = 0;
-  int rc = ml4ca_policy_describe(p, &cfg, &device);
-  if (rc != ML4CA_OK) return rc;
-  *cfg_out = cfg, *device_out = device;
-  if (!(cfg.hidden == 64 && cfg.n_hidden == 2 && cfg.obs_dim <= ppo::XR)) {
-    // not the 64 x 64 config ppo::Args describes: the caller takes the tensor-core kernel of that shape (ppo_update_tc.cu:
-    // the reference's 80^3 and 64^3 networks) or the generic fp32 kernel (ppo_update_generic.cu: any width <= 96, 1..3 hidden
-    // layers; fp32 mode and every other shape)
-    if (cfg.hidden > 96 || cfg.n_hidden < 1 || cfg.n_hidden > 3 || cfg.obs_dim > 15) {
-      set_error("%s: training kernels exist for hidden widths <= 96 and 1..3 hidden layers", who);
-      return ML4CA_ERR_UNSUPPORTED;
-    }
-    out->params = nullptr;     // marks "generic"
-    return ML4CA_OK;
-  }
-  const int H = ppo::H, O = cfg.obs_dim, Ad = cfg.act_dim;
-  const int pi_size = O * H + H + H * H + H + H * Ad + Ad;
-  ppo::Args a = {};
-  a.params = ml4ca_policy_params(p);
-  a.obs = O, a.act = Ad, a.nout = net == 0 ? Ad : 1;
-  const int base = net == 0 ? 0 : pi_size + Ad;     // v block follows pi block and log_std
-  a.off_w1 = base, a.off_b1 = base + O * H, a.off_w2 = a.off_b1 + H, a.off_b2 = a.off_w2 + H * H, a.off_wo = a.off_b2 + H;
-  a.off_bo = a.off_wo + H * a.nout;
-  a.off_ls = pi_size;
-  a.n = n, a.T = T;
-  *out = a, *cfg_out = cfg, *device_out = device;
-  return ML4CA_OK;
-}
-
-// Argument block of the generic kernel for one net of policy p.
-static ppogen::Args generic_args(ml4ca_policy* p, const ml4ca_policy_cfg& cfg, int32_t net, int64_t n, int32_t T) {
+// Shape and flat offsets of net 0 (pi, then log_std) or net 1 (v) of a policy with configuration cfg.  A net's block is W1 [obs, H],
+// b1, then W [H, H], b per further hidden layer, then Wo [H, nout], bo; the v block follows the pi block and log_std.
+static void net_layout(const ml4ca_policy_cfg& cfg, int32_t net, GradArgs* a) {
   const int H = cfg.hidden, O = cfg.obs_dim, Ad = cfg.act_dim, NL = cfg.n_hidden;
-  auto net_size = [&](int outw) { return O * H + H + (NL - 1) * (H * H + H) + H * outw + outw; };
-  ppogen::Args g = {};
-  g.params = ml4ca_policy_params(p);
-  g.obs = O, g.act = Ad, g.nout = net == 0 ? Ad : 1;
-  g.hidden = H, g.n_hidden = NL;
-  g.net_off = net == 0 ? 0 : net_size(Ad) + Ad;
-  g.net_params = net_size(g.nout);
-  g.off_ls = net_size(Ad);
-  g.n = n, g.T = T;
-  return g;
+  const int pi_size = O * H + H + (NL - 1) * (H * H + H) + H * Ad + Ad;
+  a->obs = O, a->act = Ad, a->nout = net == 0 ? Ad : 1;
+  a->hidden = H, a->n_hidden = NL;
+  a->off_w[0] = net == 0 ? 0 : pi_size + Ad, a->off_b[0] = a->off_w[0] + O * H;
+  for (int l = 1; l < NL; ++l) a->off_w[l] = a->off_b[l - 1] + H, a->off_b[l] = a->off_w[l] + H * H;
+  a->off_w[NL] = a->off_b[NL - 1] + H, a->off_b[NL] = a->off_w[NL] + H * a->nout;
+  a->off_ls = pi_size;
 }
 
-// Argument block of the tensor-core kernel for one net of a policy whose shape is not the 64 x 64 of ppo::Args
-// (80^3, 64^3, 80 x 80: ml4ca_ppo_tc_supports).
-static ppotc::Args tc_deep_args(ml4ca_policy* p, const ml4ca_policy_cfg& cfg, int32_t net, int64_t n, int32_t T) {
-  const int H = cfg.hidden, O = cfg.obs_dim, Ad = cfg.act_dim, NL = cfg.n_hidden;
-  auto net_size = [&](int outw) { return O * H + H + (NL - 1) * (H * H + H) + H * outw + outw; };
-  ppotc::Args t = {};
-  t.params = ml4ca_policy_params(p);
-  t.obs = O, t.act = Ad, t.nout = net == 0 ? Ad : 1;
-  t.hidden = H, t.n_hidden = NL;
-  const int base = net == 0 ? 0 : net_size(Ad) + Ad;
-  t.off_w[0] = base, t.off_b[0] = base + O * H;
-  for (int l = 1; l < NL; ++l) t.off_w[l] = t.off_b[l - 1] + H, t.off_b[l] = t.off_w[l] + H * H;
-  t.off_w[NL] = t.off_b[NL - 1] + H, t.off_b[NL] = t.off_w[NL] + H * t.nout;
-  t.off_ls = net_size(Ad);
-  t.n = n, t.T = T;
-  return t;
-}
-
-static int ppo_launch_fp32(const ppo::Args& a, int activation, int net, cudaStream_t st) {
+static int ppo_launch_fp32(const GradArgs& a, int activation, int net, cudaStream_t st) {
   const int64_t tiles = (a.n * (int64_t)a.T + ppo::TS - 1) / ppo::TS;
-  if (tiles == 0) return ML4CA_OK;
   const int grid = (int)(tiles < kNumSMs ? tiles : kNumSMs);
   const size_t smem = sizeof(ppo::Smem);
 #define ML4CA_PPO_LAUNCH(ACTV, NETV)                                                                             \
@@ -684,6 +590,36 @@ static int ppo_launch_fp32(const ppo::Args& a, int activation, int net, cudaStre
 #undef ML4CA_PPO_LAUNCH
   return check_launch("ppo_grad_kernel");
 }
+
+// The pass behind ml4ca_ppo_grad_ex, ml4ca_trpo_policy_mu and ml4ca_trpo_kl_grad.  `a` arrives with the buffers, the loss mode and
+// ctl / iter; tensor_cores is the process-wide switch that applies to the pass.  A gradient pass (grad != NULL) zeroes grad and
+// stats, also when the batch is empty.  The tcgen05 kernel (fp16 operands, fp32 TMEM accumulation) runs when the switch is on;
+// otherwise the fp32 CUDA-core kernels: ppo_grad_kernel for the 64 x 64 config, the generic one for the other shapes.
+static int grad_pass(ml4ca_policy* p, int32_t net, int64_t n, int32_t T, GradArgs a, bool tensor_cores, cudaStream_t st) {
+  ML4CA_REQUIRE(p != nullptr, "policy is NULL");
+  ML4CA_REQUIRE(n >= 0 && T >= 0, "bad sizes");
+  ml4ca_policy_cfg cfg;
+  int32_t device = 0;
+  int rc = ml4ca_policy_describe(p, &cfg, &device);
+  if (rc != ML4CA_OK) return rc;
+  if (a.grad != nullptr) {
+    ML4CA_CUDA(cudaMemsetAsync(a.grad, 0, sizeof(float) * (size_t)ml4ca_policy_num_params(&cfg), st));
+    ML4CA_CUDA(cudaMemsetAsync(a.stats, 0, sizeof(double) * 8, st));
+  }
+  if (n * (int64_t)T == 0) return ML4CA_OK;
+  net_layout(cfg, net, &a);
+  a.params = ml4ca_policy_params(p), a.n = n, a.T = T;
+  if (tensor_cores && ml4ca_ppo_tc_supports(cfg.hidden, cfg.n_hidden, cfg.obs_dim, cfg.act_dim)) {
+    __half* blob = nullptr;
+    rc = tc_blob(device, &blob);
+    if (rc != ML4CA_OK) return rc;
+    return ml4ca_ppo_grad_tc_launch(a, cfg.activation, net, blob, st);
+  }
+  if (cfg.hidden == ppo::H && cfg.n_hidden == 2 && cfg.obs_dim <= ppo::XR) return ppo_launch_fp32(a, cfg.activation, net, st);
+  return ml4ca_ppo_grad_generic_launch(a, cfg.activation, net, st);
+}
+
+extern "C" {
 
 int ml4ca_ppo_grad(ml4ca_policy* p, int32_t net, int64_t n, int32_t T, const float* obs, const float* act, const float* adv,
                    const float* ret, const float* logp_old, float clip_ratio, float* grad, double* stats, void* stream) {
@@ -720,115 +656,28 @@ int ml4ca_ppo_grad_ex(ml4ca_policy* p, int32_t net, int64_t n, int32_t T, const 
   ML4CA_REQUIRE(net == 0 || net == 1, "net: 0 = pi, 1 = v");
   if (net == 0) ML4CA_REQUIRE(act && adv && logp_old, "pi pass needs act, adv and logp_old");
   else ML4CA_REQUIRE(ret != nullptr, "v pass needs ret");
-  ppo::Args a;
-  ml4ca_policy_cfg cfg;
-  int32_t device = 0;
-  int rc = ppo_args(p, net, n, T, "ml4ca_ppo_grad", &a, &cfg, &device);
-  if (rc != ML4CA_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  ML4CA_CUDA(cudaMemsetAsync(grad, 0, sizeof(float) * (size_t)ml4ca_policy_num_params(&cfg), st));
-  ML4CA_CUDA(cudaMemsetAsync(stats, 0, sizeof(double) * 8, st));
-  if (a.params == nullptr && !g_use_fp32 && ml4ca_ppo_tc_supports(cfg.hidden, cfg.n_hidden, cfg.obs_dim, cfg.act_dim)) {
-    // the reference's own shapes (80^3, 64^3) on the tensor cores, like the 64 x 64 config
-    ppotc::Args t = tc_deep_args(p, cfg, net, n, T);
-    t.obs_buf = obs, t.act_buf = act, t.adv = adv, t.logp_old = logp_old, t.ret = ret;
-    t.clip = clip_ratio, t.grad = grad, t.stats = stats;
-    t.ctl = reinterpret_cast<const int32_t*>(ctl), t.iter = iter;
-    if (n * (int64_t)T == 0) return ML4CA_OK;
-    __half* blob = nullptr;
-    rc = tc_blob(device, &blob);
-    if (rc != ML4CA_OK) return rc;
-    return ml4ca_ppo_grad_tc_launch(t, cfg.activation, net, blob, st);
-  }
-  if (a.params == nullptr) {     // fp32 mode or another shape: generic fp32 kernel
-    ppogen::Args g = generic_args(p, cfg, net, n, T);
-    g.obs_buf = obs, g.act_buf = act, g.adv = adv, g.logp_old = logp_old, g.ret = ret;
-    g.clip = clip_ratio, g.grad = grad, g.stats = stats;
-    g.ctl = reinterpret_cast<const int32_t*>(ctl), g.iter = iter;
-    return ml4ca_ppo_grad_generic_launch(g, cfg.activation, net, st);
-  }
+  GradArgs a = {};
   a.obs_buf = obs, a.act_buf = act, a.adv = adv, a.logp_old = logp_old, a.ret = ret;
   a.clip = clip_ratio;
   a.grad = grad, a.stats = stats;
   a.ctl = reinterpret_cast<const int32_t*>(ctl), a.iter = iter;
-  const int64_t tiles = (n * (int64_t)T + ppo::TS - 1) / ppo::TS;
-  if (tiles == 0) return ML4CA_OK;
-  // Default: the tcgen05 kernel (fp16 operands, fp32 TMEM accumulation).  ML4CA_PPO_FP32=1 selects the fp32
-  // CUDA-core kernel (gradients to 1e-5 instead of 1e-3).
-  if (!g_use_fp32) {
-    __half* blob = nullptr;
-    rc = tc_blob(device, &blob);
-    if (rc != ML4CA_OK) return rc;
-    return ml4ca_ppo_grad_tc_launch(tc_args(a), cfg.activation, net, blob, st);
-  }
-  return ppo_launch_fp32(a, cfg.activation, net, st);
+  return grad_pass(p, net, n, T, a, !g_use_fp32, static_cast<cudaStream_t>(stream));
 }
 
 int ml4ca_trpo_policy_mu(ml4ca_policy* p, int64_t n, int32_t T, const float* obs, float* mu, void* stream) {
   ML4CA_REQUIRE(obs != nullptr && mu != nullptr, "obs and mu are required");
-  ppo::Args a;
-  ml4ca_policy_cfg cfg;
-  int32_t device = 0;
-  int rc = ppo_args(p, 0, n, T, "ml4ca_trpo_policy_mu", &a, &cfg, &device);
-  if (rc != ML4CA_OK) return rc;
-  if (a.params == nullptr && g_trpo_tc && n * (int64_t)T > 0 && ml4ca_ppo_tc_supports(cfg.hidden, cfg.n_hidden, cfg.obs_dim, cfg.act_dim)) {
-    ppotc::Args t = tc_deep_args(p, cfg, 0, n, T);
-    t.obs_buf = obs, t.mu_out = mu;
-    __half* blob = nullptr;
-    rc = tc_blob(device, &blob);
-    if (rc != ML4CA_OK) return rc;
-    return ml4ca_ppo_grad_tc_launch(t, cfg.activation, 0, blob, static_cast<cudaStream_t>(stream));
-  }
-  if (a.params == nullptr) {
-    ppogen::Args g = generic_args(p, cfg, 0, n, T);
-    g.obs_buf = obs, g.mu_out = mu;
-    return ml4ca_ppo_grad_generic_launch(g, cfg.activation, 0, static_cast<cudaStream_t>(stream));
-  }
+  GradArgs a = {};
   a.obs_buf = obs, a.mu_out = mu;
-  if (g_trpo_tc && ((n + ppo::TS - 1) / ppo::TS) * T > 0) {
-    __half* blob = nullptr;
-    rc = tc_blob(device, &blob);
-    if (rc != ML4CA_OK) return rc;
-    return ml4ca_ppo_grad_tc_launch(tc_args(a), cfg.activation, 0, blob, static_cast<cudaStream_t>(stream));
-  }
-  return ppo_launch_fp32(a, cfg.activation, 0, static_cast<cudaStream_t>(stream));
+  return grad_pass(p, 0, n, T, a, g_trpo_tc, static_cast<cudaStream_t>(stream));
 }
 
 int ml4ca_trpo_kl_grad(ml4ca_policy* p, int64_t n, int32_t T, const float* obs, const float* mu_old, const float* log_std_old,
                        float* grad, double* stats, void* stream) {
   ML4CA_REQUIRE(obs && mu_old && log_std_old && grad && stats, "obs, mu_old, log_std_old, grad and stats are required");
-  ppo::Args a;
-  ml4ca_policy_cfg cfg;
-  int32_t device = 0;
-  int rc = ppo_args(p, 0, n, T, "ml4ca_trpo_kl_grad", &a, &cfg, &device);
-  if (rc != ML4CA_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  ML4CA_CUDA(cudaMemsetAsync(grad, 0, sizeof(float) * (size_t)ml4ca_policy_num_params(&cfg), st));
-  ML4CA_CUDA(cudaMemsetAsync(stats, 0, sizeof(double) * 8, st));
-  if (a.params == nullptr && g_trpo_tc && n * (int64_t)T > 0 && ml4ca_ppo_tc_supports(cfg.hidden, cfg.n_hidden, cfg.obs_dim, cfg.act_dim)) {
-    ppotc::Args t = tc_deep_args(p, cfg, 0, n, T);
-    t.obs_buf = obs, t.act_buf = mu_old, t.kl_ls_old = log_std_old, t.loss_mode = 1;
-    t.grad = grad, t.stats = stats;
-    __half* blob = nullptr;
-    rc = tc_blob(device, &blob);
-    if (rc != ML4CA_OK) return rc;
-    return ml4ca_ppo_grad_tc_launch(t, cfg.activation, 0, blob, st);
-  }
-  if (a.params == nullptr) {
-    ppogen::Args g = generic_args(p, cfg, 0, n, T);
-    g.obs_buf = obs, g.act_buf = mu_old, g.kl_ls_old = log_std_old, g.loss_mode = 1;
-    g.grad = grad, g.stats = stats;
-    return ml4ca_ppo_grad_generic_launch(g, cfg.activation, 0, st);
-  }
+  GradArgs a = {};
   a.obs_buf = obs, a.act_buf = mu_old, a.kl_ls_old = log_std_old, a.loss_mode = 1;
   a.grad = grad, a.stats = stats;
-  if (g_trpo_tc && ((n + ppo::TS - 1) / ppo::TS) * T > 0) {
-    __half* blob = nullptr;
-    rc = tc_blob(device, &blob);
-    if (rc != ML4CA_OK) return rc;
-    return ml4ca_ppo_grad_tc_launch(tc_args(a), cfg.activation, 0, blob, st);
-  }
-  return ppo_launch_fp32(a, cfg.activation, 0, st);
+  return grad_pass(p, 0, n, T, a, g_trpo_tc, static_cast<cudaStream_t>(stream));
 }
 
 int ml4ca_adam_step(int64_t m, float* params, const float* grad, float* m1, float* m2, float lr, float beta1, float beta2,

@@ -5,9 +5,10 @@
 // Same contract as ppo_grad_kernel (ppo_update.cu; reference ppo.py:234-250, core.py:29-46): forward, loss and backward
 // of ONE network (NET 0 = pi incl. log_std, 1 = v) over every sample of a [T, ., n] buffer in fp32, gradient SUMS into the
 // flat vector, loss statistics in double; also the TRPO passes (loss_mode 1 = d_kl, mu_out = forward only).
-// Any width H <= 96 and 1..3 hidden layers, obs <= 16.  A persistent CTA (8 warps) works on tiles of 64 samples; the three
-// GEMM shapes of a layer are register-tiled so that a fused multiply-add costs 0.2 .. 0.4 shared-memory loads (the first
-// version of this kernel had no register tiling, 2 loads per FMA, and ran at the shared-memory bandwidth: 83 M sample-passes/s):
+// Hidden 64 x 64, 64^3 and 80^3 (the networks ml4ca_policy_create accepts), obs <= 16.  A persistent CTA (8 warps) works on
+// tiles of 64 samples; the three GEMM shapes of a layer are register-tiled so that a fused multiply-add costs 0.2 .. 0.4
+// shared-memory loads (the first version of this kernel had no register tiling, 2 loads per FMA, and ran at the shared-memory
+// bandwidth: 83 M sample-passes/s):
 //   forward        h_l[j][s] = f(b_l[j] + sum_k h_{l-1}[k][s] W_l[k][j])     warp w owns HP/8 features, a lane two samples:
 //                                                                            per k two activation loads + HP/16 64-bit weight loads
 //   weight grad.   dW_l[k][j] += sum_s h_{l-1}[k][s] g_l[j][s]               thread (k-block, j-block) owns a (HP/16)^2 tile of
@@ -15,7 +16,7 @@
 //                                                                            = 256 threads); bias gradients ride on the first k-block
 //   backward data  g_{l-1}[k][s] = f'(h_{l-1}[k][s]) sum_j W_l[k][j] g_l[j][s]   warp w owns HP/8 rows k, a lane two samples:
 //                                                                            per 4 j: 8 signal loads + HP/8 128-bit weight loads
-// HP = the width rounded up to 64 / 80 / 96 (template parameter: the register tiles need compile-time shapes).  The weights are
+// HP = the width rounded up to 64 / 80 (template parameter: the register tiles need compile-time shapes).  The weights are
 // copied to shared memory ZERO-PADDED to HP, so every row / column offset is an immediate and nothing on the path is masked.
 // Weights, activations and back-propagated signals live in shared memory (80^3: 173 KB); activation rows have stride 66: a
 // lane's two samples are one 64-bit access, conflict-free both for lane = sample reads and for the strided tiles of the
@@ -28,10 +29,10 @@
 #include <stdlib.h>
 
 #include "common.h"
-#include "ppo_generic.h"
+#include "ppo_grad.h"
 
 namespace ml4ca {
-namespace ppogen {
+namespace generic {
 
 constexpr int TS = 64;     // samples per tile: lane s owns samples 2 s and 2 s + 1 (one 64-bit access)
 constexpr int RS = 66;     // activation row stride (floats): even, so sample pairs are 8-byte aligned in every row
@@ -50,7 +51,7 @@ __device__ __forceinline__ float act_grad(float h) {          // derivative expr
   return 1.0f - h * h;
 }
 
-__host__ __device__ inline int padded_width(int H) { return H <= 64 ? 64 : (H <= 80 ? 80 : 96); }
+__host__ __device__ inline int padded_width(int H) { return H <= 64 ? 64 : 80; }
 
 // The net's parameters in shared memory, ZERO-PADDED to the compile-time width HP: W1 [obs][HP], b1 [HP], then per further hidden
 // layer W_l [HP][HP], b_l [HP], then Wo [HP][OP], bo [OP].  Every row / column offset is a compile-time constant (immediate
@@ -68,7 +69,7 @@ __host__ __device__ inline size_t smem_floats(int obs, int H, int NL) {
 }
 
 // Feature (forward) / row (backward data) jj of warp w: eight consecutive ones from the first 64, the rest from the tail, so
-// that a warp's slice of a weight row is two 128-bit words plus one 64- (HP = 80) or 128-bit (HP = 96) word.
+// that a warp's slice of a weight row is two 128-bit words plus one 64-bit word (HP = 80).
 template <int JT>
 __device__ __forceinline__ int warp_feature(int w, int jj) { return jj < 8 ? w * 8 + jj : 64 + (JT - 8) * w + (jj - 8); }
 template <int JT>
@@ -78,14 +79,11 @@ __device__ __forceinline__ void load_slice(const float* __restrict__ row, int w,
   if constexpr (JT == 10) {
     const float2 c = *reinterpret_cast<const float2*>(row + 64 + 2 * w);
     v[8] = c.x, v[9] = c.y;
-  } else if constexpr (JT == 12) {
-    const float4 c = *reinterpret_cast<const float4*>(row + 64 + 4 * w);
-    v[8] = c.x, v[9] = c.y, v[10] = c.z, v[11] = c.w;
   }
 }
 
 template <int ACTIVATION, int NET, int HP>
-__global__ void __launch_bounds__(NT, 1) ppo_grad_generic_kernel(const Args A) {
+__global__ void __launch_bounds__(NT, 1) ppo_grad_generic_kernel(const GradArgs A) {
   if (A.ctl != nullptr && A.ctl[0] != 0 && A.ctl[1] < A.iter) return;   // the policy loop has stopped (ml4ca_ppo_ctl)
   constexpr int JT = HP / 8;     // features (forward) / rows (backward data) per warp
   constexpr int BT = HP / 16;    // edge of a thread's weight-gradient tile
@@ -114,7 +112,7 @@ __global__ void __launch_bounds__(NT, 1) ppo_grad_generic_kernel(const Args A) {
   __syncthreads();
   for (int l = 0; l <= NL; ++l) {          // flat order W1 [obs,H], b1, W2 [H,H], b2, ..., Wo [H,nout], bo -> padded rows
     const int K = layer_in(l), N = (l == NL) ? nout : H, NP = (l == NL) ? OP : HP;
-    const float* src = A.params + A.net_off + w_off(l);
+    const float* src = A.params + A.off_w[0] + w_off(l);
     float* dst = W + wp_off(l);
     for (int e = tid; e < (K + 1) * N; e += NT) {
       const int k = e / N, j = e - k * N;
@@ -450,7 +448,7 @@ __global__ void __launch_bounds__(NT, 1) ppo_grad_generic_kernel(const Args A) {
 
   if (A.mu_out != nullptr) return;       // forward-only pass (uniform)
   // ---- flush ---------------------------------------------------------------------------------------------------------------------
-  float* grad = A.grad + A.net_off;
+  float* grad = A.grad + A.off_w[0];
   {
     // layer 0: row kb of dW1, bias b1
 #pragma unroll
@@ -510,18 +508,18 @@ __global__ void __launch_bounds__(NT, 1) ppo_grad_generic_kernel(const Args A) {
   }
 }
 
-}  // namespace ppogen
+}  // namespace generic
 }  // namespace ml4ca
 
 using namespace ml4ca;
 
 template <int HP>
-static int launch_generic(const ppogen::Args& a, int activation, int net, int grid, size_t smem, cudaStream_t st) {
+static int launch_generic(const GradArgs& a, int activation, int net, int grid, size_t smem, cudaStream_t st) {
 #define ML4CA_PPOGEN_LAUNCH(ACTV, NETV)                                                                          \
   do {                                                                                                           \
-    auto k = ppogen::ppo_grad_generic_kernel<ACTV, NETV, HP>;                                                    \
+    auto k = generic::ppo_grad_generic_kernel<ACTV, NETV, HP>;                                                   \
     ML4CA_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-    k<<<grid, ppogen::NT, smem, st>>>(a);                                                                        \
+    k<<<grid, generic::NT, smem, st>>>(a);                                                                       \
   } while (0)
   if (activation == 1) {
     if (net == 0) ML4CA_PPOGEN_LAUNCH(1, 0); else ML4CA_PPOGEN_LAUNCH(1, 1);
@@ -532,16 +530,14 @@ static int launch_generic(const ppogen::Args& a, int activation, int net, int gr
   return check_launch("ppo_grad_generic_kernel");
 }
 
-int ml4ca_ppo_grad_generic_launch(const ppogen::Args& a, int activation, int net, cudaStream_t st) {
-  const int64_t tiles = (a.n * (int64_t)a.T + ppogen::TS - 1) / ppogen::TS;
-  if (tiles == 0) return ML4CA_OK;
-  ML4CA_REQUIRE(a.hidden >= 1 && a.hidden <= 96 && a.n_hidden >= 1 && a.n_hidden <= 3 && a.obs >= 1 && a.obs <= 16 && a.nout <= ppogen::OP,
-                "generic gradient kernel: hidden width 1..96, 1..3 hidden layers, obs_dim <= 16, outputs <= 8");
+int ml4ca_ppo_grad_generic_launch(const GradArgs& a, int activation, int net, cudaStream_t st) {
+  const bool shape = (a.hidden == 64 && (a.n_hidden == 2 || a.n_hidden == 3)) || (a.hidden == 80 && a.n_hidden == 3);
+  ML4CA_REQUIRE(shape && a.obs >= 1 && a.obs <= 16 && a.nout <= generic::OP,
+                "generic gradient kernel: hidden 64 x 64, 64^3 or 80^3, obs_dim <= 16, outputs <= 8");
+  const int64_t tiles = (a.n * (int64_t)a.T + generic::TS - 1) / generic::TS;
   const int grid = (int)(tiles < kNumSMs ? tiles : kNumSMs);
-  const size_t smem = sizeof(float) * ppogen::smem_floats(a.obs, a.hidden, a.n_hidden);
+  const size_t smem = sizeof(float) * generic::smem_floats(a.obs, a.hidden, a.n_hidden);
   ML4CA_REQUIRE(smem <= 227 * 1024, "network too large for the shared-memory plan of the generic gradient kernel");
-  const int HP = ppogen::padded_width(a.hidden);
-  if (HP == 64) return launch_generic<64>(a, activation, net, grid, smem, st);
-  if (HP == 80) return launch_generic<80>(a, activation, net, grid, smem, st);
-  return launch_generic<96>(a, activation, net, grid, smem, st);
+  if (a.hidden == 64) return launch_generic<64>(a, activation, net, grid, smem, st);
+  return launch_generic<80>(a, activation, net, grid, smem, st);
 }

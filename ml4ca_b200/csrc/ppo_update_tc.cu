@@ -35,14 +35,14 @@
 //
 // Numerics: fp16 operands (activations, weights, back-propagated signals x 64), fp32 accumulation: gradients agree
 // with the float64 oracle to ~1e-3 of the largest component for two hidden layers, 4.5e-3 stated for three (the rounding
-// enters once per layer; tests/test_ppo_update_gpu.py); the fp32 CUDA-core kernels (ppo_update.cu for 64 x 64,
-// ppo_update_generic.cu for every other shape) remain available (ML4CA_PPO_FP32=1) where 1e-4 .. 1e-5 is wanted.
+// enters once per layer; tests/test_ppo_update_gpu.py); the fp32 CUDA-core kernels (ppo_update.cu for 64 x 64 with obs_dim
+// <= 12, ppo_update_generic.cu for the other networks) remain available (ML4CA_PPO_FP32=1) where 1e-4 .. 1e-5 is wanted.
 #include <stdlib.h>
 
 #include <cuda_fp16.h>
 
 #include "common.h"
-#include "ppo_tc.h"
+#include "ppo_grad.h"
 #include "tc05.cuh"
 
 namespace ml4ca {
@@ -54,8 +54,8 @@ constexpr int TS = 128, OP = 16;
 constexpr float kScale = 64.0f;            // loss scaling of the back-propagated signals (fp16 range)
 
 // Sizes, shared-memory plan and tensor-memory plan of one network shape (H hidden units, NL hidden layers).
-// SH: the variant with tile groups on SHARED weight-gradient accumulators (80^3, large batches; also built for 64 x 64 as a
-// measured-and-rejected experiment); false: every group owns its accumulators
+// SH: the variant with tile groups on SHARED weight-gradient accumulators (80^3, large batches); false: every group owns its
+// accumulators
 template <int H_, int NL_, bool SH_ = false>
 struct Shape {
   static constexpr int H = H_, NL = NL_, KP = H_ + 16;
@@ -75,11 +75,8 @@ struct Shape {
   //  * both groups accumulate into ONE set of weight-gradient accumulators (TMEM: 2 x 80 + 192 columns).  MMAs into the same
   //    accumulator must not be in flight from two issuing threads at once: a weight-gradient chain is issued under a CTA-wide
   //    lock (shared-memory word) that its group releases when the chain has completed (the wait every stage ends with).
-  static constexpr bool SHARED = SH_ && ((H_ == 80 && NL_ == 3) || (H_ == 64 && NL_ == 2));
-#ifndef ML4CA_TC_G64X2_SHARED
-#define ML4CA_TC_G64X2_SHARED 4
-#endif
-  static constexpr int G = (H_ == 64 && NL_ == 2) ? (SHARED ? ML4CA_TC_G64X2_SHARED : ML4CA_TC_G64X2) : ((H_ == 80 && NL_ == 3) ? (SHARED ? 2 : 1) : 2);
+  static constexpr bool SHARED = SH_ && H_ == 80 && NL_ == 3;
+  static constexpr int G = (H_ == 64 && NL_ == 2) ? ML4CA_TC_G64X2 : ((H_ == 80 && NL_ == 3) ? (SHARED ? 2 : 1) : 2);
   // threads per sample row: with a single group nothing overlaps its epilogues, so two threads share a row (two warps may read
   // the same TMEM lane quadrant: warp w reaches lanes 32 (w % 4) ..) and each converts half of the accumulator columns
   static constexpr int SPLIT = (G == 1) ? 2 : ((H_ == 64 && NL_ == 2) ? ML4CA_TC_SPLIT64X2 : ML4CA_TC_SPLIT64X3);
@@ -106,7 +103,7 @@ struct Shape {
   static constexpr int TMEM_G = H + TMEM_ACC;
   static_assert((SHARED ? G * H + TMEM_ACC : G * TMEM_G) <= 512, "tensor memory");
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory");
-  static_assert(BLOB_E <= kBlobHalves, "operand blob scratch");
+  static_assert(BLOB_E <= kTcBlobHalves, "operand blob scratch");
 };
 
 __host__ __device__ __forceinline__ int canon(int row, int k, int K_total) {
@@ -122,7 +119,7 @@ __host__ __device__ constexpr uint32_t idesc(int M, int N, int a_mn, int b_mn) {
 // fp32 master parameters of one net -> its fp16 operand images (canonical K-major).  off_w / off_b: [0] layer 1 (obs -> H),
 // [l - 1] hidden layer l, [NL] output layer.
 template <int H, int NL>
-__global__ void pack_kernel(Args A, __half* __restrict__ blob) {
+__global__ void pack_kernel(GradArgs A, __half* __restrict__ blob) {
   using S = Shape<H, NL>;     // (the operand images do not depend on the group arrangement)
   constexpr int KP = S::KP;
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -183,7 +180,7 @@ __device__ __forceinline__ float2 act_grad2(uint32_t h2) {
 
 // S97: the 9 -> 7 (pi) / 9 -> 1 (v) networks of RevoltFinal(extended_state, cont_ang) with the dims known at compile time.
 template <int ACTIVATION, int NET, bool S97, int H, int NL, bool SH>
-__global__ void __launch_bounds__((Shape<H, NL, SH>::THREADS), 1) ppo_grad_tc_kernel(const Args A) {
+__global__ void __launch_bounds__((Shape<H, NL, SH>::THREADS), 1) ppo_grad_tc_kernel(const GradArgs A) {
   if (A.ctl != nullptr && A.ctl[0] != 0 && A.ctl[1] < A.iter) return;   // uniform: before any barrier / TMEM allocation
   using S = Shape<H, NL, SH>;
   constexpr int KP = S::KP, G = S::G, THREADS = S::THREADS, GROUP_B = S::GROUP_B, A0_B = S::A0_B, AH_B = S::AH_B, GO_B = S::GO_B;
@@ -615,12 +612,12 @@ __global__ void __launch_bounds__((Shape<H, NL, SH>::THREADS), 1) ppo_grad_tc_ke
 
 using namespace ml4ca;
 
-// Host side: called by ml4ca_ppo_grad (ppo_update.cu) unless ML4CA_PPO_FP32 is set.  `blob` is scratch for the packed
-// fp16 operands (>= ppotc::kBlobHalves halves), owned by the caller.
+// Host side: called by grad_pass (ppo_update.cu) when the tensor-core switch of the pass is on.  `blob` is scratch for the
+// packed fp16 operands (>= kTcBlobHalves halves), owned by the caller.
 template <int H, int NL, bool SH = false>
-static int launch_shape(const ppotc::Args& args, int activation, int net, void* blob, cudaStream_t st) {
+static int launch_shape(const GradArgs& args, int activation, int net, void* blob, cudaStream_t st) {
   using S = ppotc::Shape<H, NL, SH>;
-  ppotc::Args a = args;
+  GradArgs a = args;
   __half* b = static_cast<__half*>(blob);
   ppotc::pack_kernel<H, NL><<<(S::BLOB_E + 255) / 256, 256, 0, st>>>(a, b);
   int rc = check_launch("ppo pack_kernel");
@@ -652,15 +649,10 @@ bool ml4ca_ppo_tc_supports(int hidden, int n_hidden, int obs, int act) {
   return shape && obs >= 1 && obs <= 15 && act >= 1 && act <= 8;
 }
 
-int ml4ca_ppo_grad_tc_launch(const ppotc::Args& args, int activation, int net, void* blob, cudaStream_t st) {
+int ml4ca_ppo_grad_tc_launch(const GradArgs& args, int activation, int net, void* blob, cudaStream_t st) {
   ML4CA_REQUIRE(ml4ca_ppo_tc_supports(args.hidden, args.n_hidden, args.obs, args.act), "shape not built for the tensor-core gradient kernel");
-#ifndef ML4CA_TC_SHARED64X2
-#define ML4CA_TC_SHARED64X2 0
-#endif
-  const int64_t tiles64 = (args.n * (int64_t)args.T + ppotc::TS - 1) / ppotc::TS;
   if (args.hidden == 64) {
     if (args.n_hidden == 3) return launch_shape<64, 3>(args, activation, net, blob, st);
-    if (ML4CA_TC_SHARED64X2 && tiles64 > 2 * kNumSMs) return launch_shape<64, 2, true>(args, activation, net, blob, st);
     return launch_shape<64, 2>(args, activation, net, blob, st);
   }
   // 80^3: the two-group kernel on shared accumulators streams large batches 1.4 x faster (5.1 against 3.65 G sample-passes/s), the
