@@ -141,6 +141,30 @@ ML4CA_API int ml4ca_env_set_disturbance_state(ml4ca_env* env, const float* curre
 /* Copies of the disturbance state: current [2, n], bias [3, n], either nullable.  Needs an enabled disturbance. */
 ML4CA_API int ml4ca_env_get_disturbance(ml4ca_env* env, float* current, float* bias, void* stream);
 
+/* First-order wave-frequency motion (DECLARED model, DESIGN.md section 4; set at the same DigiTwin.val seam).  Per env
+ * and DOF d (surge, sway, yaw; body frame) a linear oscillator driven by white noise,
+ * x'' + 2 lambda w0 x' + w0^2 x = sigma_d sqrt(4 lambda w0^3) w(t), with stationary std sigma_d of x and w0 sigma_d of x'.
+ * w0 ~ U(omega_min, omega_max) is drawn at every reset (explicit or in-kernel) together with a stationary state; the state
+ * then takes one exact step per env step (also with n_substeps = 0).  The motion never moves the hull: eta and nu stay
+ * the low-frequency state.  The observation, the reward and the termination of every step and reset, cut_obs and
+ * ml4ca_env_observe see the measured values N + cos(psi) x_s - sin(psi) x_w, E + sin(psi) x_s + cos(psi) x_w,
+ * psi + x_psi and nu + x'. */
+typedef struct ml4ca_wave_cfg {
+  float sigma[3];             /* m, m, rad, >= 0: stationary std of the WF motion in surge, sway, yaw (body frame) */
+  float omega_min, omega_max; /* rad/s, 0 < min <= max, max * step_dt < pi: peak frequency, drawn per episode */
+  float damping;              /* 0 < lambda < 1 */
+} ml4ca_wave_cfg;
+/* cfg = NULL switches waves off (rows stay allocated).  Enabling draws every env's state on `stream`.  Launch
+ * parameter, like the restart fraction and the disturbance: CUDA graphs captured earlier keep theirs.  Bad values:
+ * ML4CA_ERR_INVALID. */
+ML4CA_API int ml4ca_env_set_waves(ml4ca_env* env, const ml4ca_wave_cfg* cfg, void* stream);
+/* motion [3, n], rate [3, n] (body frame), omega [n]; any may be NULL; needs enabled waves.  Set values hold until that
+ * env's next reset. */
+ML4CA_API int ml4ca_env_set_wave_state(ml4ca_env* env, const float* motion, const float* rate, const float* omega,
+                                       void* stream);
+/* Copies of the wave state: motion [3, n], rate [3, n], omega [n]; any may be NULL; needs enabled waves. */
+ML4CA_API int ml4ca_env_get_waves(ml4ca_env* env, float* motion, float* rate, float* omega, void* stream);
+
 /* Stateless pieces of the wrapper, exposed for callers that own their own state (and for parity tests):
  * ErrorFrame.transform (errorFrame.py:25-32): eta, ref [3, n] -> err [3, n] body-frame error. */
 ML4CA_API int ml4ca_error_frame(int64_t n, const float* eta, const float* ref, float* err, void* stream);

@@ -36,6 +36,12 @@ class DisturbanceCfg(ctypes.Structure):
     ]
 
 
+class WaveCfg(ctypes.Structure):
+    """struct ml4ca_wave_cfg"""
+    _fields_ = [("sigma", ctypes.c_float * 3), ("omega_min", ctypes.c_float), ("omega_max", ctypes.c_float),
+                ("damping", ctypes.c_float)]
+
+
 class PolicyCfg(ctypes.Structure):
     """struct ml4ca_policy_cfg"""
     _fields_ = [("obs_dim", ctypes.c_int32), ("act_dim", ctypes.c_int32), ("hidden", ctypes.c_int32),
@@ -71,6 +77,9 @@ _SIGNATURES = {
     "ml4ca_env_set_disturbance": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(DisturbanceCfg), c_stream]),
     "ml4ca_env_set_disturbance_state": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_stream]),
     "ml4ca_env_get_disturbance": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_stream]),
+    "ml4ca_env_set_waves": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(WaveCfg), c_stream]),
+    "ml4ca_env_set_wave_state": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_stream]),
+    "ml4ca_env_get_waves": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_stream]),
     "ml4ca_error_frame": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_stream]),
     "ml4ca_scale_and_clip": (ctypes.c_int, [ctypes.POINTER(EnvCfg), ctypes.c_int64, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),
     "ml4ca_pinv_pid": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_stream]),

@@ -33,6 +33,14 @@
 #define ML4CA_ENV_MIN_BLOCKS_DIST 4  // disturbed step: 64 registers; 40 would spill around the Philox / Box-Muller draws
 #endif
 
+#ifndef ML4CA_ENV_MIN_BLOCKS_WAVE
+#define ML4CA_ENV_MIN_BLOCKS_WAVE 4  // step with wave motion: 64 registers, no spills
+#endif
+
+#ifndef ML4CA_ENV_MIN_BLOCKS_WAVE_DIST
+#define ML4CA_ENV_MIN_BLOCKS_WAVE_DIST 3  // wave motion and disturbance together: 4 CTAs (64 registers) would spill 12-16 B
+#endif
+
 namespace ml4ca {
 
 struct EnvParams {
@@ -59,6 +67,16 @@ struct EnvParams {
   // pointers above are then advanced by `first` (row stride stays n) and the caller's action / obs rows have
   // their own stride io_stride.  Whole-batch launches: count = io_stride = n.
   int64_t count, io_stride;
+};
+
+// Wave-frequency motion (ml4ca_env_set_waves): the step kernel's last argument, after DistParams, for the reason given
+// there (and appended to DistParams it would grow the stack copy the DIST kernels make of it).  The three pointers are
+// NULL while waves are off.
+struct WaveParams {
+  float* motion;       // [3, n] x: surge (m), sway (m), yaw (rad), body frame
+  float* rate;         // [3, n] x' (m/s, m/s, rad/s)
+  float* omega;        // [n] peak frequency w0 of the episode (rad/s)
+  WaveConsts k;
 };
 
 // Environmental disturbance (ml4ca_env_set_disturbance).  Passed as the LAST argument of the step kernel rather than
@@ -93,9 +111,11 @@ struct ml4ca_env {
   void* slab;
   ml4ca::HostPipe* pipe = nullptr;
   void* dist_slab = nullptr;  // current [2, n] + bias [3, n] rows, allocated when a disturbance is first enabled
+  void* wave_slab = nullptr;  // motion [3, n] + rate [3, n] + omega [n] rows, allocated when waves are first enabled
   bool tail_valid;     // obs_tail rows describe the last returned observation (true after a reset, false after a step)
   ml4ca::EnvParams p;
   ml4ca::DistParams dist = {};
+  ml4ca::WaveParams wave = {};
 };
 
 namespace ml4ca {
@@ -174,13 +194,19 @@ __device__ __forceinline__ void st_flags(uint8_t* __restrict__ row, int64_t i, c
 // recurrence runs unchanged on the velocity relative to the water, nu_r = nu - R(psi0)^T v_c, with the bias added to
 // the wrench as R(psi0)^T b (after the lag); the pose then drifts by n_sub h v_c and nu = nu_r + R(psi1)^T v_c is the
 // velocity over ground again.  20 B more read (current, bias) and 12 B more written (bias) per env-step: 209 B.
-template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false>
-__global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
+// WAVE = true (one env per thread only): the wave-frequency motion of ml4ca_env_set_waves.  After the hull step the wave
+// state takes one exact step (advance_waves), and the observation, reward and termination are computed from the measured
+// pose and velocity (add_wave_motion) instead of the LF state, which is stored unchanged.  28 B more read (x, x', w0)
+// and 24 B more written (x, x') per env-step: 229 B, 261 B together with the disturbance.
+template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false, bool WAVE = false>
+__global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_DIST : ML4CA_ENV_MIN_BLOCKS_WAVE) : (DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1)))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
                                                        float* __restrict__ obs, float* __restrict__ rew,
-                                                       uint8_t* __restrict__ done, const DistParams d) {
+                                                       uint8_t* __restrict__ done, const DistParams d,
+                                                       const WaveParams wv) {
   using T = EnvTraits<KIND, CONT>;
   static_assert(!LAG || VEC == 1, "the lagged integrator is scalar");
   static_assert(!DIST || VEC == 1, "the disturbed step is scalar");
+  static_assert(!WAVE || VEC == 1, "the step with wave motion is scalar");
   const int64_t n = p.n, ios = p.io_stride;
   const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
   if (i0 >= p.count) return;
@@ -220,6 +246,12 @@ __global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC =
     for (int c = 0; c < 2; ++c) ld_row<VEC>(d.current + (int64_t)c * n, i0, cur[c]);
 #pragma unroll
     for (int c = 0; c < 3; ++c) ld_row<VEC>(d.bias + (int64_t)c * n, i0, bia[c]);
+  }
+  float wm[3], wr[3], w0 = 0.f;                                        // VEC == 1 when WAVE
+  if constexpr (WAVE) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) wm[c] = wv.motion[(int64_t)c * n + i0], wr[c] = wv.rate[(int64_t)c * n + i0];
+    w0 = wv.omega[i0];
   }
 
   float o[9][VEC], rw[VEC];
@@ -302,12 +334,15 @@ __global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC =
     }
   }
   // ---- phase C: observation, reward, termination --------------------------------------------------------------------
+  if constexpr (WAVE) advance_waves(p.seed, p.env_off + i0, ep[0] + 1, wv.k, w0, wm, wr);   // word after this step
 #pragma unroll
   for (int j = 0; j < VEC; ++j) {
+    float mN = eta[0][j], mE = eta[1][j], mP = eta[2][j], mu = nu[0][j], mv = nu[1][j], mr = nu[2][j];
+    if constexpr (WAVE) add_wave_motion(mN, mE, mP, mu, mv, mr, wm, wr);       // the measured pose and velocity
     float xb, yb, pb;                                                  // state_extended(), :125
-    error_frame(eta[0][j], eta[1][j], eta[2][j], ref[0][j], ref[1][j], ref[2][j], xb, yb, pb);
+    error_frame(mN, mE, mP, ref[0][j], ref[1][j], ref[2][j], xb, yb, pb);
     o[0][j] = xb, o[1][j] = yb, o[2][j] = pb;
-    o[3][j] = nu[0][j], o[4][j] = nu[1][j], o[5][j] = nu[2][j];
+    o[3][j] = mu, o[4][j] = mv, o[5][j] = mr;
     float old_thrust[3] = {0.f, 0.f, 0.f};
     if constexpr (EXT) {
 #pragma unroll
@@ -317,9 +352,9 @@ __global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC =
       }
     }
     const float thrust[3] = {thr[0][j], thr[1][j], thr[2][j]};
-    rw[j] = reward_fn<EXT>(xb, yb, pb, nu[0][j], nu[1][j], nu[2][j], thrust, old_thrust, dang[0][j], dang[1][j],
-                           dang[2][j], p.inv_step_dt, 1.0f / T::ANG_BOUND);                        // :128
-    const bool term = is_terminal(xb, yb, pb, nu[0][j], nu[1][j], nu[2][j], p.bounds);           // :129
+    rw[j] = reward_fn<EXT>(xb, yb, pb, mu, mv, mr, thrust, old_thrust, dang[0][j], dang[1][j], dang[2][j], p.inv_step_dt,
+                           1.0f / T::ANG_BOUND);                                                   // :128
+    const bool term = is_terminal(xb, yb, pb, mu, mv, mr, p.bounds);                             // :129
     ep[j] += 1;                                                        // low half: steps in this episode
     const bool trunc = (int32_t)((uint32_t)ep[j] & kEpLenMask) >= p.max_ep_len;   // ppo.py:304
     flags[j] = (term ? ML4CA_DONE_TERMINAL : 0u) | (trunc ? ML4CA_DONE_TRUNCATED : 0u);
@@ -349,12 +384,22 @@ __global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC =
         d.current[i0 + j] = cj[0], d.current[n + i0 + j] = cj[1];
         bia[0][j] = bj[0], bia[1][j] = bj[1], bia[2][j] = bj[2];
       }
+      float mN = eta[0][j], mE = eta[1][j], mP = eta[2][j], mu = nu[0][j], mv = nu[1][j], mr = nu[2][j];
+      if constexpr (WAVE) {                                            // a new w0 and a stationary draw (old episode word)
+        float xj[3], xdj[3], wj;
+        sample_waves(p.seed, p.env_off + i0 + j, ep[j], wv.k.sigma[0], wv.k.sigma[1], wv.k.sigma[2], wv.k.omega_lo,
+                     wv.k.omega_span, xj, xdj, &wj);
+        wv.omega[i0 + j] = wj;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) wm[c] = xj[c], wr[c] = xdj[c];
+        add_wave_motion(mN, mE, mP, mu, mv, mr, wm, wr);
+      }
       float t0[3] = {0.f, 0.f, 0.f};                                   // customEnv.py:190
       if (p.reset_acts) sample_reset_thrust(p.seed, p.env_off + i0 + j, ep[j], t0);   // :179-188 (old episode word)
       ep[j] = next_episode_word(ep[j]);
       pth[0][j] = t0[0], pth[1][j] = t0[1], pth[2][j] = t0[2];
-      error_frame(eta[0][j], eta[1][j], eta[2][j], ref[0][j], ref[1][j], ref[2][j], o[0][j], o[1][j], o[2][j]);
-      o[3][j] = nu[0][j], o[4][j] = nu[1][j], o[5][j] = nu[2][j];
+      error_frame(mN, mE, mP, ref[0][j], ref[1][j], ref[2][j], o[0][j], o[1][j], o[2][j]);
+      o[3][j] = mu, o[4][j] = mv, o[5][j] = mr;
       if constexpr (EXT) o[6][j] = div100(t0[0]), o[7][j] = div100(t0[1]), o[8][j] = div100(t0[2]);
     }
   }
@@ -377,6 +422,10 @@ __global__ void __launch_bounds__(256, DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC =
 #pragma unroll
     for (int c = 0; c < 3; ++c) st_row<VEC>(d.bias + (int64_t)c * n, i0, bia[c]);
   }
+  if constexpr (WAVE) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) wv.motion[(int64_t)c * n + i0] = wm[c], wv.rate[(int64_t)c * n + i0] = wr[c];
+  }
 #pragma unroll
   for (int c = 0; c < (EXT ? 9 : 6); ++c) st_row<VEC>(obs + (int64_t)c * ios, i0, o[c]);
   st_row<VEC>(rew, i0, rw);
@@ -389,7 +438,8 @@ template <int KIND, bool CONT, bool EXT>
 __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const uint8_t* __restrict__ mask,
                                                         const float* __restrict__ eta_in,
                                                         const float* __restrict__ nu_in,
-                                                        float* __restrict__ obs, const DistParams d) {
+                                                        float* __restrict__ obs, const DistParams d,
+                                                        const WaveParams wv) {
   using T = EnvTraits<KIND, CONT>;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= p.n) return;
@@ -416,6 +466,15 @@ __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const
     sample_disturbance(p.seed, p.env_off + i, epi, d.k, cur, b);
     d.current[i] = cur[0], d.current[n + i] = cur[1];
     d.bias[i] = b[0], d.bias[n + i] = b[1], d.bias[2 * n + i] = b[2];
+  }
+  if (wv.motion != nullptr) {                                                        // waves enabled
+    float x[3], xd[3], w0;
+    sample_waves(p.seed, p.env_off + i, epi, wv.k.sigma[0], wv.k.sigma[1], wv.k.sigma[2], wv.k.omega_lo, wv.k.omega_span,
+                 x, xd, &w0);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) wv.motion[c * n + i] = x[c], wv.rate[c * n + i] = xd[c];
+    wv.omega[i] = w0;
+    add_wave_motion(N, E, psi, u, v, r, x, xd);                                        // the observation is measured
   }
   p.ep_len[i] = next_episode_word(epi);
   if (obs != nullptr) {

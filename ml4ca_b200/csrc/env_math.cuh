@@ -538,4 +538,90 @@ __device__ __forceinline__ void advance_bias(uint64_t seed, int64_t env_id, int3
   bP = fmaf(d.gm_gain[2], z[2], d.gm_a * bP);
 }
 
+// ---- first-order wave-frequency motion (DECLARED model, DESIGN.md section 4; tests/wave_oracle.py) ----------------------
+// Per env and DOF d (surge, sway, yaw; body frame) the linear oscillator x'' + 2 lambda w0 x' + w0^2 x = sigma_d
+// sqrt(4 lambda w0^3) w(t), stationary law P = diag(sigma^2, w0^2 sigma^2).  w0 ~ U(omega range) per episode, shared by
+// the three DOFs.  It never feeds back into the hull: it is added to the measured pose and velocity only.
+// Per-launch constants, folded on the host (ml4ca_env_set_waves).
+struct WaveConsts {
+  float sigma[3];               // stationary std of x: m, m, rad
+  float omega_lo, omega_span;   // w0 ~ U(omega_lo, omega_lo + omega_span), rad/s
+  float lam_dt;                 // lambda * step_dt
+  float wd_dt;                  // sqrt(1 - lambda^2) * step_dt: the damped frequency per unit w0, times the step
+  float lam_ratio;              // lambda / sqrt(1 - lambda^2)
+  float inv_sq;                 // 1 / sqrt(1 - lambda^2)
+  int32_t noise;                // 1: some sigma > 0 (the per-step draws run); 0: they are skipped
+};
+
+// The wave state of a new episode: w0 from out0 of the kTagWaveOmega block, then the stationary draw x = sigma z1
+// (kTagWaveMotion0), x' = w0 sigma z2 (kTagWaveRate0).  `episode` is the episode word at the moment of the reset.  Rare
+// path (resets only), kept out of line like sample_disturbance.  The constants come as scalars: a reference into the
+// kernel's parameters would make every thread copy them to local memory on entry.
+static __device__ __noinline__ void sample_waves(uint64_t seed, int64_t env_id, int32_t episode, float sigma0, float sigma1,
+                                                 float sigma2, float omega_lo, float omega_span, float* __restrict__ x,
+                                                 float* __restrict__ xd, float* __restrict__ w0) {
+  const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ 0x5EED5EEDu;
+  const uint32_t lo = (uint32_t)((uint64_t)env_id), hi = (uint32_t)((uint64_t)env_id >> 32);
+  const Philox4 q = philox4x32_10(lo, hi, (uint32_t)episode, kTagWaveOmega, k0, k1);
+  const float w = fmaf(omega_span, unit01(q.x), omega_lo);
+  const float sigma[3] = {sigma0, sigma1, sigma2};
+  float z1[3], z2[3];
+  philox_normals3(seed, env_id, episode, kTagWaveMotion0, z1);
+  philox_normals3(seed, env_id, episode, kTagWaveRate0, z2);
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    x[c] = sigma[c] * z1[c];
+    xd[c] = w * (sigma[c] * z2[c]);
+  }
+  *w0 = w;
+}
+
+// One env step of the wave motion, the exact discretisation s <- Phi s + sigma L z of s = [x, x'] over step_dt.  In the
+// scaled state y = x' / w0 the stationary covariance is the identity, so Phi' = D^-1 Phi D (D = diag(1, w0)) with
+//   e = exp(-lambda w0 dt), (sn, cs) = (sin, cos)(w0 sqrt(1 - lambda^2) dt), g = e sn / sqrt(1 - lambda^2):
+//   Phi' = [[e (cs + lambda' sn), g], [-g, e (cs - lambda' sn)]],  lambda' = lambda / sqrt(1 - lambda^2),
+// Q' = I - Phi' Phi'^T and L' its Cholesky factor (L = D L').  The diagonal of Q' is O((w0 dt)^3) small; written as
+// Q'11 = (1 - e^2) - 2 lambda' sn e Phi'11 and Q'22 = (1 - e^2) + 2 lambda' sn e Phi'22 (with 1 - e^2 from expm1f) it does
+// not cancel against 1 in fp32.  `word` is the episode word AFTER the step's increment: the two normals of each DOF come
+// from the kTagWaveStep1 / kTagWaveStep2 blocks of it.
+__device__ __forceinline__ void advance_waves(uint64_t seed, int64_t env_id, int32_t word, const WaveConsts& k, float w0,
+                                              float (&x)[3], float (&xd)[3]) {
+  const float e = expf(-k.lam_dt * w0);
+  float sn, cs;
+  sincosf(k.wd_dt * w0, &sn, &cs);
+  const float g = e * sn * k.inv_sq;
+  const float f11 = e * fmaf(k.lam_ratio, sn, cs), f22 = e * fmaf(-k.lam_ratio, sn, cs);
+  const float one_m_e2 = -expm1f(-2.0f * k.lam_dt * w0), h = 2.0f * k.lam_ratio * sn * e;
+  const float q11 = fmaf(-h, f11, one_m_e2), q22 = fmaf(h, f22, one_m_e2), q12 = g * (f11 - f22);
+  const float l11 = sqrtf(fmaxf(q11, 0.f));
+  const float l21 = l11 > 0.f ? q12 / l11 : 0.f;
+  const float l22 = sqrtf(fmaxf(fmaf(-l21, l21, q22), 0.f));
+  float z1[3] = {0.f, 0.f, 0.f}, z2[3] = {0.f, 0.f, 0.f};
+  if (k.noise) {
+    philox_normals3(seed, env_id, word, kTagWaveStep1, z1);
+    philox_normals3(seed, env_id, word, kTagWaveStep2, z2);
+  }
+  const float iw = 1.0f / w0;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const float y = xd[c] * iw;
+    const float xn = fmaf(f11, x[c], fmaf(g, y, k.sigma[c] * (l11 * z1[c])));
+    const float yn = fmaf(-g, x[c], fmaf(f22, y, k.sigma[c] * fmaf(l21, z1[c], l22 * z2[c])));
+    x[c] = xn;
+    xd[c] = w0 * yn;
+  }
+}
+
+// The measured pose and velocity: the LF pose plus the wave motion rotated by the LF heading psi (x_s surge, x_w sway),
+// psi + x_psi, and nu + x' (body frame).  In place.
+__device__ __forceinline__ void add_wave_motion(float& N, float& E, float& psi, float& u, float& v, float& r,
+                                                const float (&x)[3], const float (&xd)[3]) {
+  float s, c;
+  sincos_heading(psi, s, c);
+  N = fmaf(c, x[0], fmaf(-s, x[1], N));
+  E = fmaf(s, x[0], fmaf(c, x[1], E));
+  psi += x[2];
+  u += xd[0], v += xd[1], r += xd[2];
+}
+
 }  // namespace ml4ca

@@ -18,14 +18,22 @@ __global__ void __launch_bounds__(256) error_frame_kernel(int64_t n, const float
   err[i] = xb, err[n + i] = yb, err[2 * n + i] = pb;
 }
 
-// Revolt.state() / state_extended() (customEnv.py:196-205) from the state in HBM.
-__global__ void __launch_bounds__(256) observe_kernel(const EnvParams p, int ext, float* __restrict__ obs) {
+// Revolt.state() / state_extended() (customEnv.py:196-205) from the state in HBM; with waves enabled, of the measured
+// pose and velocity.
+__global__ void __launch_bounds__(256) observe_kernel(const EnvParams p, int ext, float* __restrict__ obs,
+                                                      const WaveParams w) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
   if (i >= n) return;
+  float N = p.eta[i], E = p.eta[n + i], psi = p.eta[2 * n + i], u = p.nu[i], v = p.nu[n + i], r = p.nu[2 * n + i];
+  if (w.motion != nullptr) {
+    const float x[3] = {w.motion[i], w.motion[n + i], w.motion[2 * n + i]};
+    const float xd[3] = {w.rate[i], w.rate[n + i], w.rate[2 * n + i]};
+    add_wave_motion(N, E, psi, u, v, r, x, xd);
+  }
   float xb, yb, pb;
-  error_frame(p.eta[i], p.eta[n + i], p.eta[2 * n + i], p.ref[i], p.ref[n + i], p.ref[2 * n + i], xb, yb, pb);
+  error_frame(N, E, psi, p.ref[i], p.ref[n + i], p.ref[2 * n + i], xb, yb, pb);
   obs[i] = xb, obs[n + i] = yb, obs[2 * n + i] = pb;
-  obs[3 * n + i] = p.nu[i], obs[4 * n + i] = p.nu[n + i], obs[5 * n + i] = p.nu[2 * n + i];
+  obs[3 * n + i] = u, obs[4 * n + i] = v, obs[5 * n + i] = r;
   if (ext) obs[6 * n + i] = p.obs_tail[i], obs[7 * n + i] = p.obs_tail[n + i], obs[8 * n + i] = p.obs_tail[2 * n + i];
 }
 
@@ -112,6 +120,46 @@ __global__ void __launch_bounds__(256) draw_disturbance_kernel(const EnvParams p
   d.bias[i] = b[0], d.bias[n + i] = b[1], d.bias[2 * n + i] = b[2];
 }
 
+static int validate_waves(const ml4ca_env_cfg& c, const ml4ca_wave_cfg* w) {
+  ML4CA_REQUIRE(std::isfinite(w->sigma[0]) && std::isfinite(w->sigma[1]) && std::isfinite(w->sigma[2]) &&
+                    std::isfinite(w->omega_min) && std::isfinite(w->omega_max) && std::isfinite(w->damping),
+                "waves: every field must be finite");
+  ML4CA_REQUIRE(w->sigma[0] >= 0.f && w->sigma[1] >= 0.f && w->sigma[2] >= 0.f, "waves: sigma must be non-negative");
+  ML4CA_REQUIRE(w->omega_min > 0.f && w->omega_min <= w->omega_max,
+                "waves: peak frequency range needs 0 < omega_min <= omega_max");
+  ML4CA_REQUIRE((double)w->omega_max * (double)c.step_dt < ML4CA_PI,
+                "waves: omega_max * step_dt must stay below pi (the observation would alias the motion)");
+  ML4CA_REQUIRE(w->damping > 0.f && w->damping < 1.f, "waves: damping must lie in (0, 1)");
+  return ML4CA_OK;
+}
+
+// Per-launch constants of the wave motion (env_math.cuh: WaveConsts).
+static WaveConsts wave_consts(const ml4ca_env_cfg& c, const ml4ca_wave_cfg& w) {
+  WaveConsts k;
+  const double lam = w.damping, sq = std::sqrt(1.0 - lam * lam), dt = c.step_dt;
+  for (int i = 0; i < 3; ++i) k.sigma[i] = w.sigma[i];
+  k.omega_lo = w.omega_min;
+  k.omega_span = w.omega_max - w.omega_min;
+  k.lam_dt = (float)(lam * dt);
+  k.wd_dt = (float)(sq * dt);
+  k.lam_ratio = (float)(lam / sq);
+  k.inv_sq = (float)(1.0 / sq);
+  k.noise = (w.sigma[0] > 0.f || w.sigma[1] > 0.f || w.sigma[2] > 0.f) ? 1 : 0;
+  return k;
+}
+
+// The wave state of every env, drawn as a reset would draw it (episode word of the moment).
+__global__ void __launch_bounds__(256) draw_waves_kernel(const EnvParams p, const WaveParams w) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
+  if (i >= n) return;
+  float x[3], xd[3], w0;
+  sample_waves(p.seed, p.env_off + i, p.ep_len[i], w.k.sigma[0], w.k.sigma[1], w.k.sigma[2], w.k.omega_lo, w.k.omega_span, x,
+               xd, &w0);
+#pragma unroll
+  for (int c = 0; c < 3; ++c) w.motion[c * n + i] = x[c], w.rate[c * n + i] = xd[c];
+  w.omega[i] = w0;
+}
+
 static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&scale)[6]) {
   // fp32, one rounding per product, same order as oracle/env_oracle.py::sample_reset
   const float vfr = (float)ML4CA_VEL_FRACTION * fraction;
@@ -120,8 +168,8 @@ static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&sca
 }
 
 #define ML4CA_DECL_UNIT(name)                                                                                   \
-  int launch_step_##name(const ml4ca_env*, const EnvParams&, const DistParams&, const float*, float*, float*, uint8_t*, \
-                         cudaStream_t);                                                                            \
+  int launch_step_##name(const ml4ca_env*, const EnvParams&, const DistParams&, const WaveParams&, const float*, float*, \
+                         float*, uint8_t*, cudaStream_t);                                                          \
   int launch_reset_##name(const ml4ca_env*, const EnvParams&, const uint8_t*, const float*, const float*, float*, \
                           cudaStream_t);
 ML4CA_DECL_UNIT(full)
@@ -141,16 +189,18 @@ static int launch_step(const ml4ca_env* e, int64_t first, int64_t count, int64_t
   if (p.cut_obs != nullptr) p.cut_obs += first;
   DistParams d = e->dist;
   if (d.current != nullptr) d.current += first, d.bias += first;
+  WaveParams w = e->wave;
+  if (w.motion != nullptr) w.motion += first, w.rate += first, w.omega += first;
   p.env_off += first;
   p.count = count;
   p.io_stride = io_stride;
   switch (e->cfg.kind) {
-    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, action, obs, rew, done, st);
-    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, action, obs, rew, done, st);
-    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, action, obs, rew, done, st);
+    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, w, action, obs, rew, done, st);
+    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, w, action, obs, rew, done, st);
+    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, w, action, obs, rew, done, st);
     default:
-      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, action, obs, rew, done, st)
-                             : launch_step_final_wrap(e, p, d, action, obs, rew, done, st);
+      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, w, action, obs, rew, done, st)
+                             : launch_step_final_wrap(e, p, d, w, action, obs, rew, done, st);
   }
 }
 
@@ -293,6 +343,7 @@ int ml4ca_env_destroy(ml4ca_env* env) {
     delete hp;
   }
   cudaFree(env->dist_slab);
+  cudaFree(env->wave_slab);
   cudaFree(env->slab);
   delete env;
   return ML4CA_OK;
@@ -370,6 +421,53 @@ int ml4ca_env_get_disturbance(ml4ca_env* env, float* current, float* bias, void*
   const size_t row = (size_t)env->n * sizeof(float);
   if (current) ML4CA_CUDA(cudaMemcpyAsync(current, env->dist.current, 2 * row, cudaMemcpyDeviceToDevice, st));
   if (bias) ML4CA_CUDA(cudaMemcpyAsync(bias, env->dist.bias, 3 * row, cudaMemcpyDeviceToDevice, st));
+  return ML4CA_OK;
+}
+
+int ml4ca_env_set_waves(ml4ca_env* env, const ml4ca_wave_cfg* cfg, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  WaveParams& w = env->wave;
+  if (cfg == nullptr) {
+    w.motion = w.rate = w.omega = nullptr;            // the rows stay allocated for a later enable
+    return ML4CA_OK;
+  }
+  int stv = validate_waves(env->cfg, cfg);
+  if (stv != ML4CA_OK) return stv;
+  DeviceGuard guard(env->device);
+  const int64_t n = env->n;
+  if (env->wave_slab == nullptr) ML4CA_CUDA(cudaMalloc(&env->wave_slab, 7 * (size_t)n * sizeof(float) + 256));
+  float* f = static_cast<float*>(env->wave_slab);
+  w.motion = f;
+  w.rate = f + 3 * n;
+  w.omega = f + 6 * n;
+  w.k = wave_consts(env->cfg, *cfg);
+  draw_waves_kernel<<<(unsigned)((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(env->p, w);
+  return check_launch("draw_waves_kernel");
+}
+
+int ml4ca_env_set_wave_state(ml4ca_env* env, const float* motion, const float* rate, const float* omega, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  const WaveParams& w = env->wave;
+  ML4CA_REQUIRE(w.motion != nullptr, "waves are not enabled (ml4ca_env_set_waves)");
+  DeviceGuard guard(env->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t row = (size_t)env->n * sizeof(float);
+  if (motion) ML4CA_CUDA(cudaMemcpyAsync(w.motion, motion, 3 * row, cudaMemcpyDeviceToDevice, st));
+  if (rate) ML4CA_CUDA(cudaMemcpyAsync(w.rate, rate, 3 * row, cudaMemcpyDeviceToDevice, st));
+  if (omega) ML4CA_CUDA(cudaMemcpyAsync(w.omega, omega, row, cudaMemcpyDeviceToDevice, st));
+  return ML4CA_OK;
+}
+
+int ml4ca_env_get_waves(ml4ca_env* env, float* motion, float* rate, float* omega, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  const WaveParams& w = env->wave;
+  ML4CA_REQUIRE(w.motion != nullptr, "waves are not enabled (ml4ca_env_set_waves)");
+  DeviceGuard guard(env->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const size_t row = (size_t)env->n * sizeof(float);
+  if (motion) ML4CA_CUDA(cudaMemcpyAsync(motion, w.motion, 3 * row, cudaMemcpyDeviceToDevice, st));
+  if (rate) ML4CA_CUDA(cudaMemcpyAsync(rate, w.rate, 3 * row, cudaMemcpyDeviceToDevice, st));
+  if (omega) ML4CA_CUDA(cudaMemcpyAsync(omega, w.omega, row, cudaMemcpyDeviceToDevice, st));
   return ML4CA_OK;
 }
 
@@ -468,7 +566,7 @@ int ml4ca_env_observe(ml4ca_env* env, float* obs, void* stream) {
                 "ml4ca_env_step the observation lives in the caller's obs buffer");
   DeviceGuard guard(env->device);
   observe_kernel<<<(unsigned)((env->n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      env->p, env->cfg.extended_state, obs);
+      env->p, env->cfg.extended_state, obs, env->wave);
   return check_launch("observe_kernel");
 }
 

@@ -15,6 +15,11 @@ constexpr uint32_t kTagResetThrust = 1u;   // sample_reset_thrust: previous thru
 constexpr uint32_t kTagCurrent = 2u;       // sample_current: ocean current of a new episode (speed, direction)
 constexpr uint32_t kTagBias0 = 3u;         // sample_disturbance: bias force of a new episode (stationary draw)
 constexpr uint32_t kTagBiasStep = 4u;      // advance_bias: Gauss-Markov noise of one env step (word after the step)
+constexpr uint32_t kTagWaveOmega = 5u;     // sample_waves: peak frequency of a new episode's wave motion (uniform, out0)
+constexpr uint32_t kTagWaveMotion0 = 6u;   // sample_waves: stationary wave motion x of a new episode
+constexpr uint32_t kTagWaveRate0 = 7u;     // sample_waves: stationary wave rate x' of a new episode
+constexpr uint32_t kTagWaveStep1 = 8u;     // advance_waves: first normal of each DOF for one env step (word after the step)
+constexpr uint32_t kTagWaveStep2 = 9u;     // advance_waves: second normal of each DOF for one env step
 
 struct Philox4 {
   uint32_t x, y, z, w;

@@ -106,6 +106,15 @@ class ErrorFrame(object):
         return self._ref
 
 
+def measured_pose(eta, nu, wave, wave_rate):
+    """The measured pose and velocity a vessel's sensors report in waves (DESIGN.md section 4): the LF pose ``eta`` [3, n]
+    plus the body-frame wave motion ``wave`` [3, n] rotated by the LF heading, and ``nu`` [3, n] plus ``wave_rate``.
+    Host glue in torch; the env kernels compute the same sum for the observation."""
+    c, s = torch.cos(eta[2]), torch.sin(eta[2])
+    eta_m = torch.stack([eta[0] + c * wave[0] - s * wave[1], eta[1] + s * wave[0] + c * wave[1], eta[2] + wave[2]])
+    return eta_m, nu + wave_rate
+
+
 class _EnvErrorFrame(object):
     """``env.EF`` view (customEnv.py:66): reads the pose / reference held in the device-side state."""
 
@@ -202,6 +211,7 @@ class Revolt(object):
         self._done = torch.empty(n, dtype=torch.uint8, device=self.device)
         self._has_reset = False          # self._obs holds nothing until the first reset()
         self._disturbance = None         # the arguments of the last set_disturbance(), None = calm water
+        self._waves = None               # the arguments of the last set_waves(), None = no wave motion
         self.EF = _EnvErrorFrame(self)
 
     # -- per-class tables (customEnv.py:58-65); subclasses override --------------------------------
@@ -381,8 +391,40 @@ class Revolt(object):
             _lib.check(_lib.lib().ml4ca_env_set_disturbance_state(self._handle, _lib.ptr(cur), _lib.ptr(b), self._stream()),
                        "ml4ca_env_set_disturbance_state")
 
+    def set_waves(self, sigma=(0.0, 0.0, 0.0), peak_frequency=(1.0, 2.0), damping=0.1):
+        """First-order wave-frequency motion (the declared model of DESIGN.md section 4); ``set_waves(None)`` switches it off.
+
+        Per env and DOF (surge, sway, yaw; body frame) a second-order oscillator driven by white noise with stationary
+        std ``sigma`` (m, m, rad), damping ratio ``damping`` and peak frequency w0 ~ U(peak_frequency) rad/s, drawn at every
+        reset (explicit or in-kernel) together with a stationary state.  The motion never moves the hull: ``get_state()``'s
+        "eta" and "nu" stay the low-frequency state, while the observation, reward and termination of every step and reset
+        (and ``observe()``) see the measured pose and velocity, LF plus wave motion.  Enabling draws the state of every env
+        at once.  Like the disturbance, the setting is a launch parameter: CUDA graphs captured earlier keep theirs."""
+        with torch.cuda.device(self.device):
+            if sigma is None:
+                _lib.check(_lib.lib().ml4ca_env_set_waves(self._handle, None, self._stream()), "ml4ca_env_set_waves")
+                self._waves = None
+                return
+            c = _lib.WaveCfg()
+            for i, x in enumerate(sigma):
+                c.sigma[i] = float(x)
+            c.omega_min, c.omega_max = (float(x) for x in peak_frequency)
+            c.damping = float(damping)
+            _lib.check(_lib.lib().ml4ca_env_set_waves(self._handle, ctypes.byref(c), self._stream()), "ml4ca_env_set_waves")
+        self._waves = (tuple(float(x) for x in sigma), tuple(float(x) for x in peak_frequency), float(damping))
+
+    def set_wave_state(self, motion=None, rate=None, omega=None):
+        """Overwrite the wave state: ``motion`` [3, num_envs] (m, m, rad), ``rate`` [3, num_envs] (m/s, m/s, rad/s), both in
+        the body frame, and ``omega`` [num_envs] (rad/s); any may be None.  The values hold until that env's next reset."""
+        x = None if motion is None else self._to_device(motion, 3)[0]
+        xd = None if rate is None else self._to_device(rate, 3)[0]
+        w = None if omega is None else self._to_device(omega, 1)[0]
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().ml4ca_env_set_wave_state(self._handle, _lib.ptr(x), _lib.ptr(xd), _lib.ptr(w), self._stream()),
+                       "ml4ca_env_set_wave_state")
+
     def observe(self):
-        """state() / state_extended() (customEnv.py:196-205) of the current device-side state."""
+        """state() / state_extended() (customEnv.py:196-205) of the current device-side state (measured, with waves on)."""
         obs = torch.empty_like(self._obs)
         with torch.cuda.device(self.device):
             _lib.check(_lib.lib().ml4ca_env_observe(self._handle, _lib.ptr(obs), self._stream()), "ml4ca_env_observe")
@@ -401,6 +443,12 @@ class Revolt(object):
                 st["current"], st["bias"] = f(2), f(3)
                 _lib.check(_lib.lib().ml4ca_env_get_disturbance(self._handle, _lib.ptr(st["current"]), _lib.ptr(st["bias"]),
                                                                 self._stream()), "ml4ca_env_get_disturbance")
+            if self._waves is not None:         # wave motion [3, n], rate [3, n] (body frame), peak frequency [n]
+                st["wave"], st["wave_rate"] = f(3), f(3)
+                st["wave_omega"] = torch.empty(n, dtype=torch.float32, device=self.device)
+                _lib.check(_lib.lib().ml4ca_env_get_waves(self._handle, _lib.ptr(st["wave"]), _lib.ptr(st["wave_rate"]),
+                                                          _lib.ptr(st["wave_omega"]), self._stream()), "ml4ca_env_get_waves")
+                st["eta_measured"], st["nu_measured"] = measured_pose(st["eta"], st["nu"], st["wave"], st["wave_rate"])
         return st
 
     @property

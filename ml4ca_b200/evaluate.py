@@ -22,6 +22,14 @@ def fixed_test_poses(n):
     return np.stack([5 * np.sin(ang), 5 * np.cos(ang), np.deg2rad(np.asarray(FIXED_ANGLES_DEG)[k])])
 
 
+def sensed(st):
+    """The pose and velocity a controller receives from ``env.get_state()``: the measured values while the env has wave
+    motion on (LF state plus waves, what a vessel's sensors report), else the state itself."""
+    if "eta_measured" in st:
+        return st["eta_measured"], st["nu_measured"]
+    return st["eta"], st["nu"]
+
+
 def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False):
     """test_policy.py:97-186 for every env of ``env`` at once (one episode each, no early stop: finished runs keep
     being recorded, ``done_at`` tells where the reference loop would have cut).  Returns a dict of device tensors:
@@ -31,7 +39,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     integrator=True: the thesis' ``RLintegral`` configuration.  The policy's three error rows come from the deployment
     node's state assembly with its body-frame integrator (ml4ca_ros_state, rl_allocator.py:252-273, one env step = h):
     the error plus an integral that starts 5 s after the vessel entered the 5 m / 140 deg zone.  ``obs`` keeps the env's
-    own observation; the final integrator state is returned as ``integrator`` [3, n]."""
+    own observation; the final integrator state is returned as ``integrator`` [3, n].  With wave motion on, the state
+    assembly reads the measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose."""
     n, dev = env.num_envs, env.device
     T = int(max_ep_len if max_ep_len is not None else env.max_ep_len)
     eta0 = fixed_test_poses(n)
@@ -53,8 +62,9 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     def policy_input(o, st):
         if not integrator:
             return o
+        eta_s, nu_s = sensed(st)
         with torch.cuda.device(dev):
-            _lib.check(_lib.lib().ml4ca_ros_state(n, _lib.ptr(st["eta"]), _lib.ptr(st["nu"]), _lib.ptr(ref), _lib.ptr(prev_u),
+            _lib.check(_lib.lib().ml4ca_ros_state(n, _lib.ptr(eta_s), _lib.ptr(nu_s), _lib.ptr(ref), _lib.ptr(prev_u),
                                                   _lib.ptr(integ), _lib.ptr(t_inside), float(env.dt), _lib.ptr(ros),
                                                   _lib.current_stream()), "ml4ca_ros_state")
         x = o.clone()
@@ -84,7 +94,8 @@ def run_allocator(env, method="qp", max_ep_len=None):
     """The classical DP pipeline in the same batched env: PID on the body-frame error (ml4ca_pinv_pid) -> thrust
     allocation by the SLSQP-equivalent kernel (``method='qp'``, QPTA.tau_controller_callback_func) or the fixed-matrix
     pseudoinverse (``'pinv'``) -> env step.  Same records and metrics as run_RL_policy: with it, the thesis' comparison
-    RL vs QP vs IPI (results/all_plots) runs for thousands of poses at once."""
+    RL vs QP vs IPI (results/all_plots) runs for thousands of poses at once.  With wave motion on, the PID acts on the
+    measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose."""
     from .pinv import pinv_pid
     from .qp_allocator import QPTA
     n, dev = env.num_envs, env.device
@@ -116,7 +127,8 @@ def run_allocator(env, method="qp", max_ep_len=None):
                             f0 * (lx[0] * s0 - ly[0] * c0) + f1 * (lx[1] * s1 - ly[1] * c1) + f2 * lx[2]])
     trust = torch.ones(n, **f)     # per-run scale of the clip: halved when the programme is infeasible (the allocator then
     for t in range(T):             # holds its state, qp_allocator.py:267-269), restored step by step when it succeeds
-        n_pct, alpha, tau = pinv_pid(st["eta"], st["nu"], ref, integ, return_tau=True)
+        eta_s, nu_s = sensed(st)
+        n_pct, alpha, tau = pinv_pid(eta_s, nu_s, ref, integ, return_tau=True)
         if qp is not None:
             now = delivered(qp._prev)
             lim = slew * trust[None, :]
