@@ -183,6 +183,36 @@ ML4CA_API int ml4ca_pinv_pid(int64_t n, const float* eta, const float* nu, const
 /* Allocation only: tau [3, n] -> n_pct [3, n], alpha [2, n]. */
 ML4CA_API int ml4ca_pinv_allocate(int64_t n, const float* tau, float* n_pct, float* alpha, void* stream);
 
+/* Passive nonlinear DP observer (Fossen & Strand 1999; Fossen 2011 section 11.4.1), the state estimator between the sensors
+ * and the controller of a DP stack.  ABSENT from the reference like the PID (dp_controller); declared model, DESIGN.md
+ * section 4.  Per env it removes the wave-frequency part of the measured pose y [3, n] (N, E, psi), and estimates the
+ * low-frequency pose, the low-frequency body velocity and the slowly varying environmental force (NED, N, N, Nm: the frame
+ * and units of the env's bias).  Inputs of a step: y after the env step, and the thrust [3, n] (%) and azimuths
+ * angles [3, n] (rad) that step applied, env order bow, port, star (ml4ca_env_get_state's prev_thrust and angles).
+ * state [15, n] (caller-owned) rows: xi1^[3], xi2^[3] (wave states; xi2^ is the WF pose estimate), eta^[3], nu^[3], b^[3].
+ * omega_o [n]: the observer's wave peak frequency per env (a fixed tuning or the env's wave_omega); values outside
+ * [0.1, 10] rad/s, NaN included, are clamped into it (NaN -> 0.1).  The kinetic model is the declared hull hull_model
+ * without actuator lag; the rotation uses the measured heading, held over the step. */
+typedef struct ml4ca_observer_cfg {
+  int32_t hull_model;  /* 0 / 1: the declared hull of the kinetic model */
+  float step_dt;       /* s, > 0: n_sub = max(1, round(step_dt / 0.01)) sub-steps of step_dt / n_sub */
+  float notch_damping; /* zeta_n > wave_damping */
+  float wave_damping;  /* lambda, 0 < lambda < 1 */
+  float cutoff_ratio;  /* omega_c / omega_o > 1 */
+  float bias_time_s;   /* >= 0, 0 = infinity */
+  float k3[3], k4[3];  /* >= 0: bias and velocity injection gains per DOF */
+} ml4ca_observer_cfg;
+/* The declared defaults (ml4ca_constants.h ML4CA_OBS_*) for hull_model 0 or 1.  Host-only. */
+ML4CA_API int ml4ca_observer_cfg_default(int32_t hull_model, ml4ca_observer_cfg* cfg);
+/* eta^ = y, xi^ = nu^ = b^ = 0 for every env whose mask byte is non-zero (mask = NULL: all). */
+ML4CA_API int ml4ca_observer_reset(int64_t n, const float* y, const uint8_t* mask, float* state, void* stream);
+/* One env step.  restart [n] (nullable): an env whose byte is non-zero is re-initialised from this y (as by
+ * ml4ca_observer_reset) instead of stepped: pass the done-flag byte of an auto_reset env.  Bad configurations or
+ * arguments: ML4CA_ERR_INVALID.  n = 0: no launch. */
+ML4CA_API int ml4ca_observer_step(const ml4ca_observer_cfg* cfg, int64_t n, const float* y, const float* thrust,
+                                  const float* angles, const float* omega_o, const uint8_t* restart, float* state,
+                                  void* stream);
+
 /* QPTA.solve_QP (src/qp/ROS/qp_allocator/src/qp_allocator.py:108-234): tau [3, n] desired wrench, prev [5, n]
  * previous thruster state [f_port, f_star, f_bow, a_port, a_star] -> x [8, n] = [f(3), a(2), s(3)] after the
  * |x| < 0.01 clean-up (:232), status [n]: bit 0 = success (the reference's second return value; on failure the

@@ -42,6 +42,13 @@ class WaveCfg(ctypes.Structure):
                 ("damping", ctypes.c_float)]
 
 
+class ObserverCfg(ctypes.Structure):
+    """struct ml4ca_observer_cfg"""
+    _fields_ = [("hull_model", ctypes.c_int32), ("step_dt", ctypes.c_float), ("notch_damping", ctypes.c_float),
+                ("wave_damping", ctypes.c_float), ("cutoff_ratio", ctypes.c_float), ("bias_time_s", ctypes.c_float),
+                ("k3", ctypes.c_float * 3), ("k4", ctypes.c_float * 3)]
+
+
 class PolicyCfg(ctypes.Structure):
     """struct ml4ca_policy_cfg"""
     _fields_ = [("obs_dim", ctypes.c_int32), ("act_dim", ctypes.c_int32), ("hidden", ctypes.c_int32),
@@ -84,6 +91,10 @@ _SIGNATURES = {
     "ml4ca_scale_and_clip": (ctypes.c_int, [ctypes.POINTER(EnvCfg), ctypes.c_int64, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),
     "ml4ca_pinv_pid": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_stream]),
     "ml4ca_pinv_allocate": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_stream]),
+    "ml4ca_observer_cfg_default": (ctypes.c_int, [ctypes.c_int32, ctypes.POINTER(ObserverCfg)]),
+    "ml4ca_observer_reset": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_u8p, c_f32p, c_stream]),
+    "ml4ca_observer_step": (ctypes.c_int, [ctypes.POINTER(ObserverCfg), ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_u8p,
+                                           c_f32p, c_stream]),
     "ml4ca_qp_solve": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),
     "ml4ca_qp_options_default": (ctypes.c_int, [ctypes.POINTER(QpOptions)]),
     "ml4ca_qp_solve_ex": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, ctypes.POINTER(QpOptions), c_f32p, ctypes.c_void_p, c_stream]),

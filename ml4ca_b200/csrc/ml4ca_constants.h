@@ -103,4 +103,19 @@
 #define ML4CA_PID_SAT_N (80.0)
 #define ML4CA_PID_DT (0.2)
 
+// ---- passive nonlinear DP observer (Fossen & Strand 1999; DECLARED defaults of ml4ca_observer_cfg_default) -----
+// Per DOF: K11 = -2 (zeta_n - lambda) w_c / w_o, K12 = 2 w_o (zeta_n - lambda), K2 = w_c = CUTOFF_RATIO w_o,
+// K4 = K4_PER_MASS diag(m11, m22, m33) of the selected hull, K3 = K3_PER_K4 K4; 1/T_b <= K3/K4 < w_o < w_c.
+// Mirrored in tests/observer_oracle.py and checked there by tests/test_observer_cpu.py.
+#define ML4CA_OBS_NOTCH_DAMPING (1.0)   // zeta_n
+#define ML4CA_OBS_WAVE_DAMPING (0.1)    // lambda
+#define ML4CA_OBS_CUTOFF_RATIO (1.2)    // w_c / w_o
+#define ML4CA_OBS_BIAS_TIME_S (0.0)     // T_b, 0 = infinity
+#define ML4CA_OBS_K4_PER_MASS (0.2)     // 1/s^2
+#define ML4CA_OBS_K3_PER_K4 (0.2)       // 1/s
+#define ML4CA_OBS_PEAK_FREQUENCY (1.5)  // rad/s: the fixed w_o a DPObserver starts with
+#define ML4CA_OBS_OMEGA_MIN (0.1)       // rad/s: the kernel clamps every w_o (NaN included) into [MIN, MAX]
+#define ML4CA_OBS_OMEGA_MAX (10.0)
+#define ML4CA_OBS_STATE_ROWS 15         // xi1[3], xi2[3], eta[3], nu[3], b[3]
+
 #endif  // ML4CA_CONSTANTS_H_

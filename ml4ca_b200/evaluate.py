@@ -30,7 +30,7 @@ def sensed(st):
     return st["eta"], st["nu"]
 
 
-def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False):
+def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False, observer=None):
     """test_policy.py:97-186 for every env of ``env`` at once (one episode each, no early stop: finished runs keep
     being recorded, ``done_at`` tells where the reference loop would have cut).  Returns a dict of device tensors:
     obs [T+1, obs, n], rew [T, n], eta [T+1, 3, n], thrust [T+1, 3, n], angles [T+1, 2, n], done_at [n], ep_ret [n],
@@ -40,7 +40,13 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     node's state assembly with its body-frame integrator (ml4ca_ros_state, rl_allocator.py:252-273, one env step = h):
     the error plus an integral that starts 5 s after the vessel entered the 5 m / 140 deg zone.  ``obs`` keeps the env's
     own observation; the final integrator state is returned as ``integrator`` [3, n].  With wave motion on, the state
-    assembly reads the measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose."""
+    assembly reads the measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose.
+
+    observer: a ``DPObserver`` between the sensors and the policy.  It is reset on the measured pose after the env reset
+    and stepped after every env step with the measured pose and the thrust and azimuths the step applied; the policy's
+    rows 0-2 are then the deployment node's state assembly (ml4ca_ros_state, with or without the integrator) on the
+    estimated pose eta^, rows 3-5 the estimated velocity nu^, rows 6-8 stay the env's.  ``eta_hat`` and ``bias_hat``
+    [T+1, 3, n] are recorded; ``eta`` and the metrics keep the LF pose and the applied thrust."""
     n, dev = env.num_envs, env.device
     T = int(max_ep_len if max_ep_len is not None else env.max_ep_len)
     eta0 = fixed_test_poses(n)
@@ -55,20 +61,28 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     st = env.get_state()
     rec["obs"][0], rec["eta"][0], rec["angles"][0] = o, st["eta"], st["angles"][1:3]
     ref = env._ref.clone()
+    integ = t_inside = None
     if integrator:
         integ, t_inside = torch.zeros(3, n, **f), torch.zeros(n, **f)
+    if integrator or observer is not None:
         prev_u, ros = torch.zeros(6, n, **f), torch.empty(9, n, **f)       # ROS-order previous thrust: rows 6-8 unused here
+    if observer is not None:
+        rec["eta_hat"], rec["bias_hat"] = torch.empty(T + 1, 3, n, **f), torch.empty(T + 1, 3, n, **f)
+        observer.reset(sensed(st)[0])
+        rec["eta_hat"][0], rec["bias_hat"][0] = observer.eta_hat, observer.bias_hat
 
     def policy_input(o, st):
-        if not integrator:
+        if not integrator and observer is None:
             return o
-        eta_s, nu_s = sensed(st)
+        eta_s, nu_s = sensed(st) if observer is None else (observer.eta_hat.contiguous(), observer.nu_hat.contiguous())
         with torch.cuda.device(dev):
             _lib.check(_lib.lib().ml4ca_ros_state(n, _lib.ptr(eta_s), _lib.ptr(nu_s), _lib.ptr(ref), _lib.ptr(prev_u),
                                                   _lib.ptr(integ), _lib.ptr(t_inside), float(env.dt), _lib.ptr(ros),
                                                   _lib.current_stream()), "ml4ca_ros_state")
         x = o.clone()
         x[0:3] = ros[0:3]
+        if observer is not None:
+            x[3:6] = nu_s
         return x
     for t in range(T):
         a = ac.get_action(policy_input(o, st))                               # deterministic action = mu (:90-93)
@@ -79,6 +93,9 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
         st = env.get_state()
         rec["obs"][t + 1], rec["rew"][t], rec["eta"][t + 1] = o, r, st["eta"]
         rec["thrust"][t + 1], rec["angles"][t + 1] = st["prev_thrust"], st["angles"][1:3]
+        if observer is not None:
+            observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
+            rec["eta_hat"][t + 1], rec["bias_hat"][t + 1] = observer.eta_hat, observer.bias_hat
         first = d & (done_at == T)
         done_at = torch.where(first, torch.full_like(done_at, t + 1), done_at)
     rec["done_at"] = done_at
@@ -90,12 +107,15 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     return rec
 
 
-def run_allocator(env, method="qp", max_ep_len=None):
+def run_allocator(env, method="qp", max_ep_len=None, observer=None):
     """The classical DP pipeline in the same batched env: PID on the body-frame error (ml4ca_pinv_pid) -> thrust
     allocation by the SLSQP-equivalent kernel (``method='qp'``, QPTA.tau_controller_callback_func) or the fixed-matrix
     pseudoinverse (``'pinv'``) -> env step.  Same records and metrics as run_RL_policy: with it, the thesis' comparison
     RL vs QP vs IPI (results/all_plots) runs for thousands of poses at once.  With wave motion on, the PID acts on the
-    measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose."""
+    measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose.
+
+    observer: a ``DPObserver`` between the sensors and the PID, as in run_RL_policy: the PID acts on (eta^, nu^); the
+    records gain ``eta_hat`` and ``bias_hat`` [T+1, 3, n]."""
     from .pinv import pinv_pid
     from .qp_allocator import QPTA
     n, dev = env.num_envs, env.device
@@ -109,6 +129,10 @@ def run_allocator(env, method="qp", max_ep_len=None):
            "angles": torch.zeros(T + 1, 2, n, **f)}
     st = env.get_state()
     rec["eta"][0], rec["angles"][0] = st["eta"], st["angles"][1:3]
+    if observer is not None:
+        rec["eta_hat"], rec["bias_hat"] = torch.empty(T + 1, 3, n, **f), torch.empty(T + 1, 3, n, **f)
+        observer.reset(sensed(st)[0])
+        rec["eta_hat"][0], rec["bias_hat"][0] = observer.eta_hat, observer.bias_hat
     integ = torch.zeros(3, n, **f)
     qp = QPTA(num_envs=n, device=dev) if method == "qp" else None
     action = torch.empty(env.num_actions, n, **f)
@@ -127,7 +151,7 @@ def run_allocator(env, method="qp", max_ep_len=None):
                             f0 * (lx[0] * s0 - ly[0] * c0) + f1 * (lx[1] * s1 - ly[1] * c1) + f2 * lx[2]])
     trust = torch.ones(n, **f)     # per-run scale of the clip: halved when the programme is infeasible (the allocator then
     for t in range(T):             # holds its state, qp_allocator.py:267-269), restored step by step when it succeeds
-        eta_s, nu_s = sensed(st)
+        eta_s, nu_s = sensed(st) if observer is None else (observer.eta_hat.contiguous(), observer.nu_hat.contiguous())
         n_pct, alpha, tau = pinv_pid(eta_s, nu_s, ref, integ, return_tau=True)
         if qp is not None:
             now = delivered(qp._prev)
@@ -144,6 +168,9 @@ def run_allocator(env, method="qp", max_ep_len=None):
         st = env.get_state()
         rec["rew"][t], rec["eta"][t + 1] = r, st["eta"]
         rec["thrust"][t + 1], rec["angles"][t + 1] = st["prev_thrust"], st["angles"][1:3]
+        if observer is not None:
+            observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
+            rec["eta_hat"][t + 1], rec["bias_hat"][t + 1] = observer.eta_hat, observer.bias_hat
     rec["ep_ret"] = rec["rew"].sum(dim=0)
     rec["metrics"] = metrics(rec["eta"], ref, rec["thrust"], rec["angles"], env.dt)
     return rec
