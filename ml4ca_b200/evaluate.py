@@ -33,8 +33,14 @@ def sensed(st):
 def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False, observer=None):
     """test_policy.py:97-186 for every env of ``env`` at once (one episode each, no early stop: finished runs keep
     being recorded, ``done_at`` tells where the reference loop would have cut).  Returns a dict of device tensors:
-    obs [T+1, obs, n], rew [T, n], eta [T+1, 3, n], thrust [T+1, 3, n], angles [T+1, 2, n], done_at [n], ep_ret [n],
-    metrics [3, n] = IAE, W*, IADC.
+    obs [T+1, obs, n], rew [T, n], eta [T+1, 3, n], thrust [T+1, 3, n], angles [T+1, 2, n], ref [T+1, 3, n], done_at [n],
+    ep_ret [n], metrics [3, n] = IAE, W*, IADC.
+
+    new_ref / ref_change_at: at step ``ref_change_at`` the env is stepped with a zero action and ``new_ref`` (test_policy.py
+    :141-146).  The env takes the new set-point after that step (customEnv.py:131), so the observation the step returns is
+    still relative to the old one: ``ref[s]`` is the set-point observation s was formed with, and a change at step k first
+    shows in sample k + 2.  The policy's state assembly (integrator / observer) uses the set-point of its sample, and the
+    IAE integrates |eta - ref| sample by sample.
 
     integrator=True: the thesis' ``RLintegral`` configuration.  The policy's three error rows come from the deployment
     node's state assembly with its body-frame integrator (ml4ca_ros_state, rl_allocator.py:252-273, one env step = h):
@@ -56,11 +62,10 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     f = dict(dtype=torch.float32, device=dev)
     rec = {"obs": torch.empty(T + 1, env.num_states, n, **f), "rew": torch.zeros(T, n, **f),
            "eta": torch.empty(T + 1, 3, n, **f), "thrust": torch.zeros(T + 1, 3, n, **f),
-           "angles": torch.zeros(T + 1, 2, n, **f)}
+           "angles": torch.zeros(T + 1, 2, n, **f), "ref": torch.empty(T + 1, 3, n, **f)}
     done_at = torch.full((n,), T, dtype=torch.int32, device=dev)
     st = env.get_state()
-    rec["obs"][0], rec["eta"][0], rec["angles"][0] = o, st["eta"], st["angles"][1:3]
-    ref = env._ref.clone()
+    rec["obs"][0], rec["eta"][0], rec["angles"][0], rec["ref"][0] = o, st["eta"], st["angles"][1:3], env._ref
     integ = t_inside = None
     if integrator:
         integ, t_inside = torch.zeros(3, n, **f), torch.zeros(n, **f)
@@ -71,7 +76,7 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
         observer.reset(sensed(st)[0])
         rec["eta_hat"][0], rec["bias_hat"][0] = observer.eta_hat, observer.bias_hat
 
-    def policy_input(o, st):
+    def policy_input(o, st, ref):
         if not integrator and observer is None:
             return o
         eta_s, nu_s = sensed(st) if observer is None else (observer.eta_hat.contiguous(), observer.nu_hat.contiguous())
@@ -85,7 +90,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
             x[3:6] = nu_s
         return x
     for t in range(T):
-        a = ac.get_action(policy_input(o, st))                               # deterministic action = mu (:90-93)
+        a = ac.get_action(policy_input(o, st, rec["ref"][t]))                # deterministic action = mu (:90-93)
+        rec["ref"][t + 1] = env._ref                                         # the set-point the step's observation is formed with
         if ref_change_at is not None and t == ref_change_at and new_ref is not None:
             o, r, d, _ = env.step(torch.zeros_like(a), new_ref=new_ref)      # :141-146
         else:
@@ -101,7 +107,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     rec["done_at"] = done_at
     steps = torch.arange(T, device=dev)[:, None]
     rec["ep_ret"] = (rec["rew"] * (steps < done_at[None, :])).sum(dim=0)
-    rec["metrics"] = metrics(rec["eta"], ref, rec["thrust"], rec["angles"], env.dt)
+    # IAE depends on eta - ref only: the per-sample error against a zero set-point is the metric of a varying set-point
+    rec["metrics"] = metrics(rec["eta"] - rec["ref"], torch.zeros(3, n, **f), rec["thrust"], rec["angles"], env.dt)
     if integrator:
         rec["integrator"] = integ
     return rec

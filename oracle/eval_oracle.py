@@ -15,11 +15,12 @@ RHO = 1025.0
 
 
 def iae(eta, ref, dt):
-    """eta [T, 3] (N, E, yaw rad), ref [3] -> final cumulative IAE with eta, ref / [5, 5, 25 deg]."""
+    """eta [T, 3] (N, E, yaw rad), ref [3] or, for a set-point that changes during the run, [T, 3] (the set-point of each
+    sample, as common.py takes it) -> final cumulative IAE with eta, ref / [5, 5, 25 deg]."""
     sc = np.array([5.0, 5.0, 25.0])
     e = np.array(eta, dtype=np.float64).copy()
-    r = np.array(ref, dtype=np.float64).copy()
-    e[:, 2], r[2] = np.rad2deg(e[:, 2]), np.rad2deg(r[2])
+    r = np.broadcast_to(np.asarray(ref, dtype=np.float64), e.shape).copy()
+    e[:, 2], r[:, 2] = np.rad2deg(e[:, 2]), np.rad2deg(r[:, 2])
     err = np.sqrt((((e - r) / sc) ** 2).sum(axis=1))
     return float(((err[1:] + err[:-1]) / 2 * dt).sum())
 

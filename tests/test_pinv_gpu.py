@@ -10,17 +10,38 @@ from oracle import constants as C
 pytestmark = pytest.mark.gpu
 
 
+def setpoint_batch(n, seed):
+    """Per-env set-points N, E ~ U(+-4 m), psi ~ U(+-0.6 rad), and the pose of synth_batch with every fourth env turned
+    round: its heading and its set-point heading on either side of +-pi (|psi - psi_ref| ~ 2 pi - 0.6 .. 2 pi), so that
+    the PID's wrap_rad(psi - psi_ref) has to wrap.  float32 values."""
+    eta, nu, _, _ = PO.synth_batch(n, seed=seed)
+    rng = np.random.default_rng(seed + 100)
+    ref = rng.uniform(-1, 1, (3, n)) * np.array([[4.0], [4.0], [0.6]])
+    far = np.arange(n) % 4 == 1
+    side = np.where(rng.random(n) < 0.5, 1.0, -1.0)
+    eta[2, far] = -side[far] * (np.pi - rng.uniform(0, 0.3, far.sum()))
+    ref[2, far] = side[far] * (np.pi - rng.uniform(0, 0.3, far.sum()))
+    return eta.astype(np.float32), nu.astype(np.float32), ref.astype(np.float32)
+
+
 @pytest.mark.parametrize("n", [1, 5, 4096, 1 << 20])
 def test_pinv_pid_matches_oracle(cuda_device, n):
+    """At the origin (the set-point of synth_batch) and at per-env set-points with headings either side of +-pi; n even
+    runs the two-envs-per-thread kernel, n odd the scalar one."""
     import ml4ca_b200 as M
-    eta, nu, ref, integ = PO.synth_batch(n, seed=1)
-    eta, nu = eta.astype(np.float32), nu.astype(np.float32)
+    origin = tuple(x.astype(np.float32) for x in PO.synth_batch(n, seed=1)[0:3])
+    for eta, nu, ref in (origin, setpoint_batch(n, 2)):
+        check_pinv_pid(M, cuda_device, n, eta, nu, ref)
+
+
+def check_pinv_pid(M, cuda_device, n, eta, nu, ref):
     integ_t = torch.zeros(3, n, device=cuda_device)
     want_integ = np.zeros((3, n))
     for it in range(2):
         n_pct, alpha, tau = M.pinv_pid(torch.as_tensor(eta, device=cuda_device), torch.as_tensor(nu, device=cuda_device),
-                                       torch.zeros(3, n, device=cuda_device), integ_t, return_tau=True)
-        wn, wa, wtau, want_integ = PO.pinv_pid(eta.astype(np.float64), nu.astype(np.float64), ref, want_integ)
+                                       torch.as_tensor(ref, device=cuda_device), integ_t, return_tau=True)
+        wn, wa, wtau, want_integ = PO.pinv_pid(eta.astype(np.float64), nu.astype(np.float64), ref.astype(np.float64),
+                                               want_integ)
         np.testing.assert_allclose(integ_t.cpu().numpy(), want_integ, rtol=1e-6, atol=1e-6)
         np.testing.assert_allclose(tau.cpu().numpy(), wtau, rtol=2e-6, atol=2e-4)
         # allocation parity is checked from the kernel's own (saturated, fp32) wrench
