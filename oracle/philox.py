@@ -94,3 +94,25 @@ def reset_thrust_normals(seed, env_id, episode):
     a0 = 2.0 * np.pi * (q[1] >> np.uint32(8)).astype(np.float64) * 2.0 ** -24
     a1 = 2.0 * np.pi * (q[3] >> np.uint32(8)).astype(np.float64) * 2.0 ** -24
     return np.stack([r0 * np.cos(a0), r0 * np.sin(a0), r1 * np.cos(a1)])
+
+
+def policy_normals(seed, env_id, step):
+    """The eight exploration normals of one (env, step) of the policy forward (csrc/policy.cu, policy_kernel): key
+    (seed_lo, seed_hi ^ 0xAC710A), TWO Philox blocks with counters (id_lo, id_hi, step, 0) and (id_lo, id_hi, step, 1);
+    Box-Muller on (x, y) and on (z, w) of each block -> eps[0..3] from the first block, eps[4..7] from the second, with
+    r = sqrt(-2 ln unit_open(a)), angle = 2 pi (b >> 8) 2^-24, (r cos, r sin) per pair.  Evaluated in float64 (the kernel's
+    __logf / __sincosf are fp32 approximations).  Returns float64 [8, n]; action a uses row a."""
+    env_id = np.asarray(env_id, dtype=np.uint64)
+    k0 = int(seed) & 0xFFFFFFFF
+    k1 = ((int(seed) >> 32) & 0xFFFFFFFF) ^ 0xAC710A
+    lo = env_id & _MASK
+    hi = env_id >> np.uint64(32)
+    st = np.full_like(lo, int(step) & 0xFFFFFFFF)
+    out = []
+    for block in (0, 1):
+        q = philox4x32(lo, hi, st, np.full_like(lo, block), k0, k1)
+        for a, b in ((q[0], q[1]), (q[2], q[3])):
+            r = np.sqrt(-2.0 * np.log(unit_open(a).astype(np.float64)))
+            ang = 2.0 * np.pi * (b >> np.uint32(8)).astype(np.float64) * 2.0 ** -24
+            out += [r * np.cos(ang), r * np.sin(ang)]
+    return np.stack(out)

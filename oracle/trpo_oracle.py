@@ -21,15 +21,20 @@ import torch
 EPS = 1e-8
 
 
+def _pi_sizes(dims):
+    """Layer widths of the pi net: [obs] + [H] * n_hidden + [act] (the pi block of mlp_oracle.unflatten)."""
+    return [dims["obs_dim"]] + [dims["hidden"]] * dims["n_hidden"] + [dims["act_dim"]]
+
+
 def n_pi(dims):
-    O, A, H = dims["obs_dim"], dims["act_dim"], dims["hidden"]
-    assert dims["n_hidden"] == 2
-    return O * H + H + H * H + H + H * A + A + A
+    """Size of the pi block: every (W [in, out], b [out]) of the pi net, then log_std [act]."""
+    s = _pi_sizes(dims)
+    return sum(s[i] * s[i + 1] + s[i + 1] for i in range(len(s) - 1)) + dims["act_dim"]
 
 
 def _pi_net(theta, dims, obs, activation):
     """theta: torch float64 [n_pi]; obs [N, obs_dim] -> mu [N, act], log_std [act]."""
-    O, A, H = dims["obs_dim"], dims["act_dim"], dims["hidden"]
+    sizes = _pi_sizes(dims)
     pos = [0]
 
     def take(*shape):
@@ -38,11 +43,14 @@ def _pi_net(theta, dims, obs, activation):
         pos[0] += k
         return t
 
-    W1, b1, W2, b2, Wo, bo, ls = take(O, H), take(H), take(H, H), take(H), take(H, A), take(A), take(A)
+    layers = [(take(sizes[i], sizes[i + 1]), take(sizes[i + 1])) for i in range(len(sizes) - 1)]
+    ls = take(dims["act_dim"])
     f = (lambda z: torch.where(z > 0, z, 0.2 * z)) if activation in ("leaky_relu", 1) else torch.tanh
-    h = f(obs @ W1 + b1)
-    h = f(h @ W2 + b2)
-    return h @ Wo + bo, ls
+    h = obs
+    for W, b in layers[:-1]:
+        h = f(h @ W + b)
+    W, b = layers[-1]
+    return h @ W + b, ls
 
 
 def gaussian_likelihood(x, mu, log_std):
@@ -120,11 +128,23 @@ def cg(Ax, b, cg_iters=10):
     return x
 
 
+def fd_hvp(prob, theta, x, radius, damping=0.0):
+    """The Hessian-vector product as ml4ca_b200.trpo.TRPOUpdater.hvp builds it: a central difference of the KL gradient over
+    +-radius along x (exact for quadratics; leaky-ReLU units that change branch inside the bracket perturb it)."""
+    x = np.asarray(x, dtype=np.float64)
+    e = radius / np.linalg.norm(x)
+    return (prob.kl_gradient(theta + e * x)[0] - prob.kl_gradient(theta - e * x)[0]) / (2 * e) + damping * x
+
+
 def update(prob, theta_old, target_kl=0.01, damping_coeff=0.1, cg_iters=10, backtrack_iters=10, backtrack_coeff=0.8,
-           algo="trpo"):
-    """trpo.py:283-321 (policy part).  -> dict(theta, x, alpha, g, pi_l_old, pi_l_new, kl, backtrack_iters)."""
+           algo="trpo", fd_radius=None):
+    """trpo.py:283-321 (policy part).  -> dict(theta, x, alpha, g, pi_l_old, pi_l_new, kl, backtrack_iters).
+    fd_radius: the Hessian-vector products by fd_hvp instead of the exact double back-propagation of the reference."""
     theta_old = np.asarray(theta_old, dtype=np.float64)
-    Hx = lambda v: prob.hvp(theta_old, v, damping_coeff)
+    if fd_radius is None:
+        Hx = lambda v: prob.hvp(theta_old, v, damping_coeff)
+    else:
+        Hx = lambda v: fd_hvp(prob, theta_old, v, fd_radius, damping_coeff)
     g, pi_l_old = prob.gradient(theta_old)
     x = cg(Hx, g, cg_iters)
     alpha = np.sqrt(2 * target_kl / (np.dot(x, Hx(x)) + EPS))

@@ -17,7 +17,15 @@ CASES = [("glorot 64x64 leaky", dict(obs_dim=9, act_dim=7, hidden=64, n_hidden=2
          ("glorot 64x64 tanh", dict(obs_dim=9, act_dim=7, hidden=64, n_hidden=2), "tanh", None),
          ("glorot 64x64 obs6 act5", dict(obs_dim=6, act_dim=5, hidden=64, n_hidden=2), "leaky_relu", None),
          ("shipped final 80x3", None, "leaky_relu", "policy_final_80x3.npz"),
-         ("shipped limited 64x3", None, "leaky_relu", "policy_limited_64x3.npz")]
+         ("shipped limited 64x3", None, "leaky_relu", "policy_limited_64x3.npz"),
+         # observation rows 12.. are loaded in place, not prefetched a tile ahead; with 15 inputs the constant-1 bias column is
+         # the last K column of the first-layer operand
+         ("glorot 64x3 obs13 act7", dict(obs_dim=13, act_dim=7, hidden=64, n_hidden=3), "leaky_relu", None),
+         ("glorot 64x64 obs15 act1", dict(obs_dim=15, act_dim=1, hidden=64, n_hidden=2), "leaky_relu", None),
+         ("glorot 80x3 tanh", dict(obs_dim=9, act_dim=7, hidden=80, n_hidden=3), "tanh", None)]
+
+# Observation scales of the 9-state RevoltFinal input, then unit scales for wider inputs.
+OBS_SCALE = [8, 8, .8, 1.4, .3, .5, 1, 1, 1.] + [1.] * 6
 
 
 def load(dims, fixture):
@@ -28,14 +36,18 @@ def load(dims, fixture):
 
 
 @pytest.mark.parametrize("name,dims,act,fixture", CASES)
-@pytest.mark.parametrize("n", [1, 127, 128 * 3 + 5, 70001])
+# The persistent kernel works through the tiles in rounds of grid x G x 128 observations (148 SMs: 75 776 for the 64-wide nets,
+# G = 4; 37 888 for the 80-wide ones, G = 2).  From the second round on, observation rows come from the one-tile-ahead prefetch
+# and the mbarrier phase carries over.  75 777: 64-wide 2 rounds (the last with one live row), 80-wide 3 rounds; 228 328:
+# 64-wide 4 rounds (the last tile holds 104 rows), 80-wide 7 rounds.
+@pytest.mark.parametrize("n", [1, 127, 128 * 3 + 5, 70001, 75777, 228328])
 def test_forward_matches_oracle(cuda_device, name, dims, act, fixture, n):
     import ml4ca_b200 as M
     flat, dims = load(dims, fixture)
     ac = M.ActorCritic(dims['obs_dim'], dims['act_dim'], (dims['hidden'],) * dims['n_hidden'], act, params=flat,
                        device=cuda_device, seed=11)
     g = torch.Generator(device=cuda_device); g.manual_seed(n)
-    scale = torch.tensor([8, 8, .8, 1.4, .3, .5, 1, 1, 1.], device=cuda_device)[:dims['obs_dim'], None]
+    scale = torch.tensor(OBS_SCALE, device=cuda_device)[:dims['obs_dim'], None]
     obs = (torch.rand(dims['obs_dim'], n, device=cuda_device, generator=g) * 2 - 1) * scale
     pi, v, logp, mu = ac.step(obs, deterministic=True, return_mu=True)
     ref = MO.forward(flat, dims, obs.cpu().numpy().astype(np.float64), act)
@@ -75,6 +87,56 @@ def test_sampling_and_loglikelihood(cuda_device):
     # a shard starting at global id 1000 draws the same noise as envs 1000.. of the full batch
     pis, _, _ = ac.step(obs[:, 1000:3000].contiguous(), step=3, env_id_offset=1000)
     assert torch.equal(pis, pi[:, 1000:3000])
+
+
+@pytest.mark.parametrize("act_dim", [7, 3])
+def test_exploration_noise_matches_philox_oracle(cuda_device, act_dim):
+    """eps = (pi - mu) / exp(log_std) draw for draw against oracle/philox.py::policy_normals: key (seed_lo, seed_hi ^ 0xAC710A)
+    with a non-zero upper seed word, two Philox blocks per (env, step) (eps[4..7] from the second), global env ids that cross
+    into the id's high word (shard offset 2^32 - 1000).
+
+    Error model, per draw.  Box-Muller in the kernel: r = sqrtf(-2 __logf(u)), (c, s) = __sincosf(2 pi f).  __logf carries
+    an absolute error <= 2^-21.41 for u in [0.5, 1] and <= 3 ulp below, so r^2 is off by dr2 = 2 max(2^-21.41, 3 2^-23 |ln u|)
+    and r by min(sqrt(dr2), dr2 / r): loose where u -> 1 and r -> 0.  The angle: 2 pi rounded to fp32 and the fp32 product
+    (<= 2^-21 together) plus the absolute error of sin.approx / cos.approx over [0, 2 pi) (2^-20.5) give r 2^-19.8.
+    Recovering eps from the fp32 outputs adds half an ulp of pi over exp(log_std), and expf (2 ulp), sqrtf and the product
+    r c in fp32 add |eps| 2^-21.  Measured on a B200: largest error 3.4e-5 (act_dim 7) and 4.1e-6 (act_dim 3), both at
+    r < 0.01 (1.0e-4 over 2^20 envs); nowhere more than 0.36 of the bound."""
+    import ml4ca_b200 as M
+    from oracle import philox as PH
+    dims = dict(obs_dim=9, act_dim=act_dim, hidden=64, n_hidden=2)
+    flat = MO.glorot_params(dims, seed=3)
+    seed = 0xC0FFEE1234ABCDEF
+    ac = M.ActorCritic(9, act_dim, (64, 64), "leaky_relu", params=flat, device=cuda_device, seed=seed)
+    n, off, step = 1 << 16, (1 << 32) - 1000, 0x80000011
+    obs = torch.rand(9, n, device=cuda_device, generator=torch.Generator(device=cuda_device).manual_seed(2)) * 2 - 1
+    pi, _, _, mu = ac.step(obs, step=step, env_id_offset=off, return_mu=True)
+    pi, mu = pi.cpu().numpy().astype(np.float64), mu.cpu().numpy().astype(np.float64)
+    sd = np.exp(MO.unflatten(flat, dims)[1])[:, None]
+    eps = (pi - mu) / sd
+    ids = np.arange(n, dtype=np.uint64) + np.uint64(off)
+    want = PH.policy_normals(seed, ids, step)[:act_dim]
+    # the uniforms of each Box-Muller pair, for the error model
+    k1 = ((seed >> 32) ^ 0xAC710A) & 0xFFFFFFFF
+    u = []
+    for block in (0, 1):
+        q = PH.philox4x32(ids & np.uint64(0xFFFFFFFF), ids >> np.uint64(32), np.full(n, step, np.uint64),
+                          np.full(n, block, np.uint64), seed & 0xFFFFFFFF, k1)
+        u += [PH.unit_open(q[0]).astype(np.float64)] * 2 + [PH.unit_open(q[2]).astype(np.float64)] * 2
+    u = np.stack(u)[:act_dim]
+    r = np.sqrt(-2.0 * np.log(u))
+    dr2 = 2.0 * np.maximum(2.0 ** -21.41, 3 * 2.0 ** -23 * np.abs(np.log(u)))
+    tol = (np.minimum(np.sqrt(dr2), dr2 / np.maximum(r, 1e-30)) + r * 2.0 ** -19.8
+           + 0.5 * np.spacing(np.abs(pi).astype(np.float32)).astype(np.float64) / sd + np.abs(want) * 2.0 ** -21)
+    assert np.isfinite(eps).all()
+    err = np.abs(eps - want)
+    assert (err <= tol).all(), (err.max(), (err / tol).max(), np.unravel_index(np.argmax(err / tol), err.shape))
+    # two blocks, not one: eps[4..7] are not a copy of eps[0..3]
+    if act_dim == 7:
+        assert np.abs(eps[4:7] - eps[0:3]).max() > 1.0
+    # the noise follows the global id: the same rows at offset 0 draw other noise
+    pi0, _, _ = ac.step(obs, step=step, env_id_offset=0)
+    assert not torch.equal(pi0.cpu(), torch.as_tensor(pi.astype(np.float32)))
 
 
 def test_parameter_update_roundtrip(cuda_device):
