@@ -212,6 +212,20 @@ ML4CA_API int ml4ca_observer_reset(int64_t n, const float* y, const uint8_t* mas
 ML4CA_API int ml4ca_observer_step(const ml4ca_observer_cfg* cfg, int64_t n, const float* y, const float* thrust,
                                   const float* angles, const float* omega_o, const uint8_t* restart, float* state,
                                   void* stream);
+/* DP observer in the loop: attach (cfg != NULL) or detach (cfg = NULL) an observer that every env step runs inside the
+ * step kernel.  state [15, n] and omega_o [n] are caller-owned, laid out as for ml4ca_observer_step, and must outlive the
+ * attachment.  cfg->step_dt must equal the env's step_dt; the hull model may differ from the env's (a model-mismatch
+ * experiment).  Attaching re-initialises every env's column from its current measured pose on `stream`.
+ * While attached, each step advances the column once with y = the measured pose after the step (LF pose plus waves) and
+ * the thrust and azimuths the step applied, and the observation rows 0-5 are error_frame(eta^, ref) and nu^.  Rows 6-8,
+ * the reward, the flags and the env state are unchanged: the observer changes only what the agent sees.  cut_obs holds the
+ * estimate-based observation of the cut step (after the update, before the restart).  An in-kernel restart, a reset or
+ * reset_to re-initialises the env's column from the new measured pose (eta^ = y, the rest 0; the returned nu^ is 0), and
+ * ml4ca_env_observe returns rows 0-5 from the current eta^ and nu^.  Cost: 124 B more per env-step (read 60 + 4, write
+ * 60), e.g. 229 -> 353 B for RevoltFinal (extended, continuous angles) in waves.  Launch parameter: CUDA graphs
+ * captured earlier keep theirs.  Bad configurations, NULL state or omega_o, a step_dt mismatch: ML4CA_ERR_INVALID. */
+ML4CA_API int ml4ca_env_set_observer(ml4ca_env* env, const ml4ca_observer_cfg* cfg, float* state, const float* omega_o,
+                                     void* stream);
 
 /* QPTA.solve_QP (src/qp/ROS/qp_allocator/src/qp_allocator.py:108-234): tau [3, n] desired wrench, prev [5, n]
  * previous thruster state [f_port, f_star, f_bow, a_port, a_star] -> x [8, n] = [f(3), a(2), s(3)] after the

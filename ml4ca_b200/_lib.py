@@ -87,6 +87,7 @@ _SIGNATURES = {
     "ml4ca_env_set_waves": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(WaveCfg), c_stream]),
     "ml4ca_env_set_wave_state": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_stream]),
     "ml4ca_env_get_waves": (ctypes.c_int, [ctypes.c_void_p, c_f32p, c_f32p, c_f32p, c_stream]),
+    "ml4ca_env_set_observer": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(ObserverCfg), c_f32p, c_f32p, c_stream]),
     "ml4ca_error_frame": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_stream]),
     "ml4ca_scale_and_clip": (ctypes.c_int, [ctypes.POINTER(EnvCfg), ctypes.c_int64, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),
     "ml4ca_pinv_pid": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_stream]),

@@ -19,6 +19,7 @@
 
 #include "common.h"
 #include "env_math.cuh"
+#include "observer_math.cuh"
 
 #ifndef ML4CA_ENV_MIN_BLOCKS
 #define ML4CA_ENV_MIN_BLOCKS 6  // scalar-row kernel: 40 registers, 48 resident warps/SM (measured best on B200)
@@ -39,6 +40,10 @@
 
 #ifndef ML4CA_ENV_MIN_BLOCKS_WAVE_DIST
 #define ML4CA_ENV_MIN_BLOCKS_WAVE_DIST 3  // wave motion and disturbance together: 4 CTAs (64 registers) would spill 12-16 B
+#endif
+
+#ifndef ML4CA_ENV_MIN_BLOCKS_OBSV
+#define ML4CA_ENV_MIN_BLOCKS_OBSV 2  // step with the observer in the loop (any LAG / DIST / WAVE): at most 128 registers
 #endif
 
 namespace ml4ca {
@@ -88,6 +93,14 @@ struct DistParams {
   DistConsts k;
 };
 
+// DP observer in the loop (ml4ca_env_set_observer): the step kernel's last argument, after WaveParams, for the reason given
+// at DistParams.  Both pointers belong to the caller; state is NULL while no observer is attached.
+struct ObserverParams {
+  float* state;        // [15, n] rows xi1^, xi2^, eta^, nu^, b^ (observer_math.cuh)
+  const float* omega;  // [n] w_o (rad/s), clamped by the kernel
+  ObsConsts k;
+};
+
 }  // namespace ml4ca
 
 namespace ml4ca {
@@ -116,6 +129,7 @@ struct ml4ca_env {
   ml4ca::EnvParams p;
   ml4ca::DistParams dist = {};
   ml4ca::WaveParams wave = {};
+  ml4ca::ObserverParams obsv = {};
 };
 
 namespace ml4ca {
@@ -198,15 +212,22 @@ __device__ __forceinline__ void st_flags(uint8_t* __restrict__ row, int64_t i, c
 // state takes one exact step (advance_waves), and the observation, reward and termination are computed from the measured
 // pose and velocity (add_wave_motion) instead of the LF state, which is stored unchanged.  28 B more read (x, x', w0)
 // and 24 B more written (x, x') per env-step: 229 B, 261 B together with the disturbance.
-template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false, bool WAVE = false>
-__global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_DIST : ML4CA_ENV_MIN_BLOCKS_WAVE) : (DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1)))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
+// OBSV = true (one env per thread only): the DP observer of ml4ca_env_set_observer runs in the loop.  Its column takes one
+// step (observer_advance) on the measured pose after this step and the thrust and azimuths this step applied, and
+// observation rows 0-5 become error_frame(eta^, ref) and nu^; rows 6-8, the reward, the flags and the env state are
+// those of the kernel without it.  cut_obs is the estimate-based observation before the restart; a restart re-initialises
+// the column from the new episode's measured pose (nu^ = 0 in the returned observation).  124 B more per env-step
+// (read 60 + 4, write 60): 301 B for RevoltFinal (extended, continuous angles), 353 B in waves.
+template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false, bool WAVE = false, bool OBSV = false>
+__global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_DIST : ML4CA_ENV_MIN_BLOCKS_WAVE) : (DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1))))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
                                                        float* __restrict__ obs, float* __restrict__ rew,
                                                        uint8_t* __restrict__ done, const DistParams d,
-                                                       const WaveParams wv) {
+                                                       const WaveParams wv, const ObserverParams ob) {
   using T = EnvTraits<KIND, CONT>;
   static_assert(!LAG || VEC == 1, "the lagged integrator is scalar");
   static_assert(!DIST || VEC == 1, "the disturbed step is scalar");
   static_assert(!WAVE || VEC == 1, "the step with wave motion is scalar");
+  static_assert(!OBSV || VEC == 1, "the step with the observer in the loop is scalar");
   const int64_t n = p.n, ios = p.io_stride;
   const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
   if (i0 >= p.count) return;
@@ -252,6 +273,12 @@ __global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_
 #pragma unroll
     for (int c = 0; c < 3; ++c) wm[c] = wv.motion[(int64_t)c * n + i0], wr[c] = wv.rate[(int64_t)c * n + i0];
     w0 = wv.omega[i0];
+  }
+  float ox[15], wo = 0.f;                                              // VEC == 1 when OBSV
+  if constexpr (OBSV) {
+#pragma unroll
+    for (int r = 0; r < 15; ++r) ox[r] = ob.state[(int64_t)r * n + i0];
+    wo = clamp_omega(ob.omega[i0]);
   }
 
   float o[9][VEC], rw[VEC];
@@ -358,6 +385,17 @@ __global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_
     ep[j] += 1;                                                        // low half: steps in this episode
     const bool trunc = (int32_t)((uint32_t)ep[j] & kEpLenMask) >= p.max_ep_len;   // ppo.py:304
     flags[j] = (term ? ML4CA_DONE_TERMINAL : 0u) | (trunc ? ML4CA_DONE_TRUNCATED : 0u);
+    if constexpr (OBSV) {         // y = the measured pose; tau from the thrust and azimuths this step applied
+      const float y[3] = {mN, mE, mP};
+      float sb, cb, sp, cp, ss, cs, tx, ty, tn;
+      sincosf(ang[0][j], &sb, &cb);
+      sincosf(ang[1][j], &sp, &cp);
+      sincosf(ang[2][j], &ss, &cs);
+      thruster_wrench_sc(thr[0][j], thr[1][j], thr[2][j], sb, cb, sp, cp, ss, cs, tx, ty, tn);
+      observer_advance(ox, y, tx, ty, tn, wo, ob.k);
+      error_frame(ox[6], ox[7], ox[8], ref[0][j], ref[1][j], ref[2][j], o[0][j], o[1][j], o[2][j]);
+      o[3][j] = ox[9], o[4][j] = ox[10], o[5][j] = ox[11];
+    }
 #pragma unroll
     for (int c = 0; c < 3; ++c) pth[c][j] = thrust[c];
     any_reset |= (flags[j] != 0u);
@@ -401,6 +439,11 @@ __global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_
       error_frame(mN, mE, mP, ref[0][j], ref[1][j], ref[2][j], o[0][j], o[1][j], o[2][j]);
       o[3][j] = mu, o[4][j] = mv, o[5][j] = mr;
       if constexpr (EXT) o[6][j] = div100(t0[0]), o[7][j] = div100(t0[1]), o[8][j] = div100(t0[2]);
+      if constexpr (OBSV) {                                            // eta^ = y of the new episode, the rest 0
+        const float y[3] = {mN, mE, mP};
+        observer_reset_column(ox, y);
+        o[3][j] = o[4][j] = o[5][j] = 0.f;
+      }
     }
   }
 
@@ -426,6 +469,10 @@ __global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_
 #pragma unroll
     for (int c = 0; c < 3; ++c) wv.motion[(int64_t)c * n + i0] = wm[c], wv.rate[(int64_t)c * n + i0] = wr[c];
   }
+  if constexpr (OBSV) {
+#pragma unroll
+    for (int r = 0; r < 15; ++r) ob.state[(int64_t)r * n + i0] = ox[r];
+  }
 #pragma unroll
   for (int c = 0; c < (EXT ? 9 : 6); ++c) st_row<VEC>(obs + (int64_t)c * ios, i0, o[c]);
   st_row<VEC>(rew, i0, rw);
@@ -433,13 +480,14 @@ __global__ void __launch_bounds__(256, WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_
 }
 
 // ---- reset ----------------------------------------------------------------------------------------------------------
-// mask nullable; explicit eta/nu (reset_to) or Philox sampling.  Writes obs for the reset envs only.
+// mask nullable; explicit eta/nu (reset_to) or Philox sampling.  Writes obs for the reset envs only.  With an observer
+// attached, the reset columns of its state start from the measured pose (eta^ = y, the rest 0) and obs rows 3-5 are nu^ = 0.
 template <int KIND, bool CONT, bool EXT>
 __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const uint8_t* __restrict__ mask,
                                                         const float* __restrict__ eta_in,
                                                         const float* __restrict__ nu_in,
                                                         float* __restrict__ obs, const DistParams d,
-                                                        const WaveParams wv) {
+                                                        const WaveParams wv, const ObserverParams ob) {
   using T = EnvTraits<KIND, CONT>;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= p.n) return;
@@ -475,6 +523,14 @@ __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const
     for (int c = 0; c < 3; ++c) wv.motion[c * n + i] = x[c], wv.rate[c * n + i] = xd[c];
     wv.omega[i] = w0;
     add_wave_motion(N, E, psi, u, v, r, x, xd);                                        // the observation is measured
+  }
+  if (ob.state != nullptr) {                                                           // observer attached
+    float x[15];
+    const float y[3] = {N, E, psi};
+    observer_reset_column(x, y);
+#pragma unroll
+    for (int c = 0; c < 15; ++c) ob.state[c * n + i] = x[c];
+    u = v = r = 0.f;                                                                   // nu^ of the observation
   }
   p.ep_len[i] = next_episode_word(epi);
   if (obs != nullptr) {

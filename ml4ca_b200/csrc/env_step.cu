@@ -19,9 +19,9 @@ __global__ void __launch_bounds__(256) error_frame_kernel(int64_t n, const float
 }
 
 // Revolt.state() / state_extended() (customEnv.py:196-205) from the state in HBM; with waves enabled, of the measured
-// pose and velocity.
+// pose and velocity; with an observer attached, rows 0-5 of its estimates eta^ and nu^.
 __global__ void __launch_bounds__(256) observe_kernel(const EnvParams p, int ext, float* __restrict__ obs,
-                                                      const WaveParams w) {
+                                                      const WaveParams w, const ObserverParams ob) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
   if (i >= n) return;
   float N = p.eta[i], E = p.eta[n + i], psi = p.eta[2 * n + i], u = p.nu[i], v = p.nu[n + i], r = p.nu[2 * n + i];
@@ -29,6 +29,10 @@ __global__ void __launch_bounds__(256) observe_kernel(const EnvParams p, int ext
     const float x[3] = {w.motion[i], w.motion[n + i], w.motion[2 * n + i]};
     const float xd[3] = {w.rate[i], w.rate[n + i], w.rate[2 * n + i]};
     add_wave_motion(N, E, psi, u, v, r, x, xd);
+  }
+  if (ob.state != nullptr) {
+    N = ob.state[6 * n + i], E = ob.state[7 * n + i], psi = ob.state[8 * n + i];
+    u = ob.state[9 * n + i], v = ob.state[10 * n + i], r = ob.state[11 * n + i];
   }
   float xb, yb, pb;
   error_frame(N, E, psi, p.ref[i], p.ref[n + i], p.ref[2 * n + i], xb, yb, pb);
@@ -160,6 +164,23 @@ __global__ void __launch_bounds__(256) draw_waves_kernel(const EnvParams p, cons
   w.omega[i] = w0;
 }
 
+// ml4ca_env_set_observer: every env's observer column starts from its current measured pose (eta^ = y, the rest 0).
+__global__ void __launch_bounds__(256) attach_observer_kernel(const EnvParams p, const WaveParams w, const ObserverParams ob) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
+  if (i >= n) return;
+  float N = p.eta[i], E = p.eta[n + i], psi = p.eta[2 * n + i], u = 0.f, v = 0.f, r = 0.f;
+  if (w.motion != nullptr) {
+    const float x[3] = {w.motion[i], w.motion[n + i], w.motion[2 * n + i]};
+    const float xd[3] = {0.f, 0.f, 0.f};
+    add_wave_motion(N, E, psi, u, v, r, x, xd);
+  }
+  float s[15];
+  const float y[3] = {N, E, psi};
+  observer_reset_column(s, y);
+#pragma unroll
+  for (int c = 0; c < 15; ++c) ob.state[c * n + i] = s[c];
+}
+
 static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&scale)[6]) {
   // fp32, one rounding per product, same order as oracle/env_oracle.py::sample_reset
   const float vfr = (float)ML4CA_VEL_FRACTION * fraction;
@@ -168,8 +189,8 @@ static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&sca
 }
 
 #define ML4CA_DECL_UNIT(name)                                                                                   \
-  int launch_step_##name(const ml4ca_env*, const EnvParams&, const DistParams&, const WaveParams&, const float*, float*, \
-                         float*, uint8_t*, cudaStream_t);                                                          \
+  int launch_step_##name(const ml4ca_env*, const EnvParams&, const DistParams&, const WaveParams&,              \
+                         const ObserverParams&, const float*, float*, float*, uint8_t*, cudaStream_t);          \
   int launch_reset_##name(const ml4ca_env*, const EnvParams&, const uint8_t*, const float*, const float*, float*, \
                           cudaStream_t);
 ML4CA_DECL_UNIT(full)
@@ -191,16 +212,18 @@ static int launch_step(const ml4ca_env* e, int64_t first, int64_t count, int64_t
   if (d.current != nullptr) d.current += first, d.bias += first;
   WaveParams w = e->wave;
   if (w.motion != nullptr) w.motion += first, w.rate += first, w.omega += first;
+  ObserverParams ob = e->obsv;
+  if (ob.state != nullptr) ob.state += first, ob.omega += first;
   p.env_off += first;
   p.count = count;
   p.io_stride = io_stride;
   switch (e->cfg.kind) {
-    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, w, action, obs, rew, done, st);
-    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, w, action, obs, rew, done, st);
-    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, w, action, obs, rew, done, st);
+    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, w, ob, action, obs, rew, done, st);
+    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, w, ob, action, obs, rew, done, st);
+    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, w, ob, action, obs, rew, done, st);
     default:
-      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, w, action, obs, rew, done, st)
-                             : launch_step_final_wrap(e, p, d, w, action, obs, rew, done, st);
+      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, w, ob, action, obs, rew, done, st)
+                             : launch_step_final_wrap(e, p, d, w, ob, action, obs, rew, done, st);
   }
 }
 
@@ -471,6 +494,28 @@ int ml4ca_env_get_waves(ml4ca_env* env, float* motion, float* rate, float* omega
   return ML4CA_OK;
 }
 
+int ml4ca_env_set_observer(ml4ca_env* env, const ml4ca_observer_cfg* cfg, float* state, const float* omega_o, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  if (cfg == nullptr) {
+    env->obsv.state = nullptr;
+    env->obsv.omega = nullptr;
+    return ML4CA_OK;
+  }
+  const int stv = validate_observer_cfg(cfg);
+  if (stv != ML4CA_OK) return stv;
+  ML4CA_REQUIRE(state != nullptr && omega_o != nullptr, "state [15, n] and omega_o [n] are required");
+  ML4CA_REQUIRE(cfg->step_dt == env->cfg.step_dt, "the observer's step_dt must equal the env's step_dt");
+  DeviceGuard guard(env->device);
+  ObserverParams ob;
+  ob.state = state;
+  ob.omega = omega_o;
+  ob.k = observer_consts(*cfg);
+  attach_observer_kernel<<<(unsigned)((env->n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(env->p, env->wave, ob);
+  const int rc = check_launch("attach_observer_kernel");
+  if (rc == ML4CA_OK) env->obsv = ob;
+  return rc;
+}
+
 int ml4ca_env_set_ref(ml4ca_env* env, const float* ref, void* stream) {
   ML4CA_REQUIRE(env != nullptr && ref != nullptr, "env and ref are required");
   DeviceGuard guard(env->device);
@@ -566,7 +611,7 @@ int ml4ca_env_observe(ml4ca_env* env, float* obs, void* stream) {
                 "ml4ca_env_step the observation lives in the caller's obs buffer");
   DeviceGuard guard(env->device);
   observe_kernel<<<(unsigned)((env->n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      env->p, env->cfg.extended_state, obs, env->wave);
+      env->p, env->cfg.extended_state, obs, env->wave, env->obsv);
   return check_launch("observe_kernel");
 }
 

@@ -212,6 +212,7 @@ class Revolt(object):
         self._has_reset = False          # self._obs holds nothing until the first reset()
         self._disturbance = None         # the arguments of the last set_disturbance(), None = calm water
         self._waves = None               # the arguments of the last set_waves(), None = no wave motion
+        self._observer = None            # the DPObserver of set_observer(), None = the agent sees the measurement
         self.EF = _EnvErrorFrame(self)
 
     # -- per-class tables (customEnv.py:58-65); subclasses override --------------------------------
@@ -423,8 +424,44 @@ class Revolt(object):
             _lib.check(_lib.lib().ml4ca_env_set_wave_state(self._handle, _lib.ptr(x), _lib.ptr(xd), _lib.ptr(w), self._stream()),
                        "ml4ca_env_set_wave_state")
 
+    def set_observer(self, observer):
+        """Run a ``DPObserver`` in the loop (DESIGN.md section 4, "DP observer in the loop"); ``set_observer(None)`` detaches.
+
+        While attached, every step advances the observer inside the step kernel, on the measured pose after the step and
+        the thrust and azimuths the step applied, and the observation rows 0-5 become the body-frame error of the estimated
+        pose eta^ and the estimated velocity nu^: what the controller of a DP vessel sees.  Rows 6-8, the reward, the
+        termination and the vessel itself are unchanged.  Every reset and in-kernel restart re-initialises the observer
+        of that env on its new measured pose.  Attaching re-initialises every env's observer on its current measured pose.
+        ``observer`` must have this env's num_envs, device and step; its hull model may differ.  The env keeps a reference:
+        the observer's ``state`` and ``omega_o`` tensors are read and written by every step.  Like the waves, the setting
+        is a launch parameter: ``rollout()`` keys its captured graphs on it."""
+        with torch.cuda.device(self.device):
+            if observer is None:
+                _lib.check(_lib.lib().ml4ca_env_set_observer(self._handle, None, None, None, self._stream()),
+                           "ml4ca_env_set_observer")
+            else:
+                assert observer.num_envs == self.num_envs, "the observer has %d envs, the env %d" % (observer.num_envs,
+                                                                                                   self.num_envs)
+                assert observer.state.device == self.device and observer.omega_o.device == self.device, \
+                    "the observer lives on %s, the env on %s" % (observer.state.device, self.device)
+                _lib.check(_lib.lib().ml4ca_env_set_observer(self._handle, ctypes.byref(observer.cfg), _lib.ptr(observer.state),
+                                                             _lib.ptr(observer.omega_o), self._stream()),
+                           "ml4ca_env_set_observer")
+        self._observer = observer
+        if self._has_reset:             # rows 0-5 of the last observation now come from the estimates (or the measurement)
+            if observer is not None:
+                eta, nu = observer.eta_hat.contiguous(), observer.nu_hat.contiguous()
+            else:
+                st = self.get_state()
+                eta, nu = (st["eta_measured"], st["nu_measured"]) if "eta_measured" in st else (st["eta"], st["nu"])
+            obs = self._obs.clone()
+            obs[0:3] = ErrorFrame(eta, self._ref, device=self.device).get_pose()
+            obs[3:6] = nu
+            self._obs = obs
+
     def observe(self):
-        """state() / state_extended() (customEnv.py:196-205) of the current device-side state (measured, with waves on)."""
+        """state() / state_extended() (customEnv.py:196-205) of the current device-side state (measured, with waves on;
+        rows 0-5 from the estimates while an observer is attached)."""
         obs = torch.empty_like(self._obs)
         with torch.cuda.device(self.device):
             _lib.check(_lib.lib().ml4ca_env_observe(self._handle, _lib.ptr(obs), self._stream()), "ml4ca_env_observe")

@@ -30,6 +30,18 @@ def sensed(st):
     return st["eta"], st["nu"]
 
 
+def in_loop_observer(env, observer):
+    """The observer a controller acts on: the one attached to ``env`` (``Revolt.set_observer``), which the env steps and
+    resets itself, else ``observer``.  -> (observer, attached).  A second observer next to an attached one is an error."""
+    attached = getattr(env, "_observer", None)
+    if attached is None:
+        return observer, False
+    if observer is not None and observer is not attached:
+        raise ValueError("the env has an observer attached (set_observer); the controllers act on it, so a second "
+                         "observer= cannot be passed")
+    return attached, True
+
+
 def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False, observer=None):
     """test_policy.py:97-186 for every env of ``env`` at once (one episode each, no early stop: finished runs keep
     being recorded, ``done_at`` tells where the reference loop would have cut).  Returns a dict of device tensors:
@@ -52,7 +64,11 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     and stepped after every env step with the measured pose and the thrust and azimuths the step applied; the policy's
     rows 0-2 are then the deployment node's state assembly (ml4ca_ros_state, with or without the integrator) on the
     estimated pose eta^, rows 3-5 the estimated velocity nu^, rows 6-8 stay the env's.  ``eta_hat`` and ``bias_hat``
-    [T+1, 3, n] are recorded; ``eta`` and the metrics keep the LF pose and the applied thrust."""
+    [T+1, 3, n] are recorded; ``eta`` and the metrics keep the LF pose and the applied thrust.  On an env with an attached
+    observer (``Revolt.set_observer``) that observer is used: the env resets and steps it, and the policy input without
+    the integrator is the env's observation, which is already formed from the estimates.  Passing another observer then
+    raises ValueError."""
+    observer, attached = in_loop_observer(env, observer)
     n, dev = env.num_envs, env.device
     T = int(max_ep_len if max_ep_len is not None else env.max_ep_len)
     eta0 = fixed_test_poses(n)
@@ -73,11 +89,12 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
         prev_u, ros = torch.zeros(6, n, **f), torch.empty(9, n, **f)       # ROS-order previous thrust: rows 6-8 unused here
     if observer is not None:
         rec["eta_hat"], rec["bias_hat"] = torch.empty(T + 1, 3, n, **f), torch.empty(T + 1, 3, n, **f)
-        observer.reset(sensed(st)[0])
+        if not attached:
+            observer.reset(sensed(st)[0])
         rec["eta_hat"][0], rec["bias_hat"][0] = observer.eta_hat, observer.bias_hat
 
     def policy_input(o, st, ref):
-        if not integrator and observer is None:
+        if not integrator and (observer is None or attached):
             return o
         eta_s, nu_s = sensed(st) if observer is None else (observer.eta_hat.contiguous(), observer.nu_hat.contiguous())
         with torch.cuda.device(dev):
@@ -100,7 +117,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
         rec["obs"][t + 1], rec["rew"][t], rec["eta"][t + 1] = o, r, st["eta"]
         rec["thrust"][t + 1], rec["angles"][t + 1] = st["prev_thrust"], st["angles"][1:3]
         if observer is not None:
-            observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
+            if not attached:
+                observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
             rec["eta_hat"][t + 1], rec["bias_hat"][t + 1] = observer.eta_hat, observer.bias_hat
         first = d & (done_at == T)
         done_at = torch.where(first, torch.full_like(done_at, t + 1), done_at)
@@ -122,7 +140,9 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
     measured pose and velocity (``sensed``); ``eta`` and the metrics keep the LF pose.
 
     observer: a ``DPObserver`` between the sensors and the PID, as in run_RL_policy: the PID acts on (eta^, nu^); the
-    records gain ``eta_hat`` and ``bias_hat`` [T+1, 3, n]."""
+    records gain ``eta_hat`` and ``bias_hat`` [T+1, 3, n].  On an env with an attached observer that observer is used, as
+    in run_RL_policy."""
+    observer, attached = in_loop_observer(env, observer)
     from .pinv import pinv_pid
     from .qp_allocator import QPTA
     n, dev = env.num_envs, env.device
@@ -138,7 +158,8 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
     rec["eta"][0], rec["angles"][0] = st["eta"], st["angles"][1:3]
     if observer is not None:
         rec["eta_hat"], rec["bias_hat"] = torch.empty(T + 1, 3, n, **f), torch.empty(T + 1, 3, n, **f)
-        observer.reset(sensed(st)[0])
+        if not attached:
+            observer.reset(sensed(st)[0])
         rec["eta_hat"][0], rec["bias_hat"][0] = observer.eta_hat, observer.bias_hat
     integ = torch.zeros(3, n, **f)
     qp = QPTA(num_envs=n, device=dev) if method == "qp" else None
@@ -176,7 +197,8 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
         rec["rew"][t], rec["eta"][t + 1] = r, st["eta"]
         rec["thrust"][t + 1], rec["angles"][t + 1] = st["prev_thrust"], st["angles"][1:3]
         if observer is not None:
-            observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
+            if not attached:
+                observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
             rec["eta_hat"][t + 1], rec["bias_hat"][t + 1] = observer.eta_hat, observer.bias_hat
     rec["ep_ret"] = rec["rew"].sum(dim=0)
     rec["metrics"] = metrics(rec["eta"], ref, rec["thrust"], rec["angles"], env.dt)

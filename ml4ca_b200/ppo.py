@@ -131,10 +131,13 @@ def rollout(env, ac, buf, seed=0, start_step=0, deterministic=False, graph=False
         _rollout_launches(env, ac, buf, seed, start_step, deterministic)
     else:
         cache = buf.__dict__.setdefault("_rollout_graphs", {})
-        # launch parameters are baked into a captured graph: the restart fraction (curriculum), the disturbance and the
-        # wave setting are part of the key
+        # launch parameters are baked into a captured graph: the restart fraction (curriculum), the disturbance, the
+        # wave setting and the attached observer are part of the key
+        obsv = getattr(env, "_observer", None)
+        obsv_key = None if obsv is None else (id(obsv), obsv.state.data_ptr(), obsv.omega_o.data_ptr(),
+                                              bytes(obsv.cfg))
         key = (id(env), id(ac), int(seed), bool(deterministic), float(env._cfg.reset_fraction),
-               getattr(env, "_disturbance", None), getattr(env, "_waves", None))
+               getattr(env, "_disturbance", None), getattr(env, "_waves", None), obsv_key)
         entry = cache.get(key)
         if entry is None:                  # first call: eager, and remember that the next one may capture
             cache[key] = {"graph": None, "counter": torch.zeros(1, dtype=torch.int32, device=buf.device)}
