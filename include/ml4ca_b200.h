@@ -227,6 +227,37 @@ ML4CA_API int ml4ca_observer_step(const ml4ca_observer_cfg* cfg, int64_t n, cons
 ML4CA_API int ml4ca_env_set_observer(ml4ca_env* env, const ml4ca_observer_cfg* cfg, float* state, const float* omega_o,
                                      void* stream);
 
+/* DP reference model (guidance; Fossen 2011 section 12.1): per env and per DOF (N, E, psi; NED) a third-order filter with
+ * saturating elements that turns a set-point r [3, n] into a smooth desired pose eta_d, velocity v_d (NED rates) and
+ * acceleration a_d for the controller.  Declared model, DESIGN.md section 4 "DP reference model":
+ *   eta_d / r = w^3 / ((s + w)(s^2 + 2 zeta w s + w^2)),  jerk = w^3 e - (2 zeta + 1) w a_d - (2 zeta + 1) w^2 v_d,
+ *   e = r - eta_d (heading: e wrapped to [-pi, pi), eta_d,psi itself is not wrapped).
+ * r is held over the env step; n_sub = max(1, round(step_dt / 0.01)) semi-implicit Euler sub-steps of h = step_dt / n_sub:
+ *   a_d <- clamp(a_d + h jerk, +-a_max),  v_d <- clamp(v_d + h a_d, +-v_max),  eta_d <- eta_d + h v_d.
+ * state [9, n] (caller-owned) rows: eta_d[3], v_d[3], a_d[3].
+ * Validation: every value finite and > 0, and per DOF the linear sub-step map stable: with q = h omega, c = 2 zeta + 1 its
+ * characteristic polynomial z^3 + a2 z^2 + a1 z + a0 (a2 = q^3 + c q^2 + c q - 3, a1 = 3 - 2 c q - c q^2, a0 = c q - 1)
+ * must meet the Jury conditions p(1) > 0, p(-1) < 0, |a0| < 1, |a0^2 - 1| > |a0 a2 - a1|.  Otherwise ML4CA_ERR_INVALID. */
+typedef struct ml4ca_refmodel_cfg {
+  float step_dt;  /* s, > 0 */
+  float zeta[3];  /* relative damping of the mass-spring-damper part, per DOF */
+  float omega[3]; /* rad/s, natural frequency (and low-pass corner) per DOF */
+  float v_max[3]; /* m/s, m/s, rad/s */
+  float a_max[3]; /* m/s^2, m/s^2, rad/s^2 */
+} ml4ca_refmodel_cfg;
+/* The declared defaults (ml4ca_constants.h ML4CA_REF_*) at step_dt = 0.2 s.  Host-only. */
+ML4CA_API int ml4ca_refmodel_cfg_default(ml4ca_refmodel_cfg* cfg);
+/* eta_d = eta0 [3, n], v_d = a_d = 0.  n = 0: no launch. */
+ML4CA_API int ml4ca_refmodel_reset(int64_t n, const float* eta0, float* state, void* stream);
+/* One env step of every env's filter toward its set-point [3, n].  Bad configurations or arguments: ML4CA_ERR_INVALID.
+ * n = 0: no launch. */
+ML4CA_API int ml4ca_refmodel_step(const ml4ca_refmodel_cfg* cfg, int64_t n, const float* setpoint, float* state,
+                                  void* stream);
+/* ml4ca_pinv_pid with velocity feed-forward: v_d [3, n] (NED rates, e.g. rows 3-5 of a reference model's state) turns the
+ * D-term into Kd (nu - R(psi)^T v_d), psi = eta[2].  Other arguments as ml4ca_pinv_pid; v_d is required. */
+ML4CA_API int ml4ca_pinv_pid_ff(int64_t n, const float* eta, const float* nu, const float* ref, const float* v_d,
+                                float* integ, float* tau, float* n_pct, float* alpha, void* stream);
+
 /* QPTA.solve_QP (src/qp/ROS/qp_allocator/src/qp_allocator.py:108-234): tau [3, n] desired wrench, prev [5, n]
  * previous thruster state [f_port, f_star, f_bow, a_port, a_star] -> x [8, n] = [f(3), a(2), s(3)] after the
  * |x| < 0.01 clean-up (:232), status [n]: bit 0 = success (the reference's second return value; on failure the

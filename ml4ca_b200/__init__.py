@@ -9,6 +9,7 @@ C ABI of libml4ca_b200.so (include/ml4ca_b200.h):
   ppo.ppo / PPOUpdater / TrajectoryBuffer, trpo.trpo / TRPOUpdater       (spinup/algos/tf1/ppo/ppo.py, trpo/trpo.py)
   pinv.pinv_pid, pinv.pinv_allocate                                      (dp_controller, absent from the reference)
   observer.DPObserver                                                    (dp_controller's state observer, absent too)
+  refmodel.ReferenceModel                                                (dp_controller's reference model, absent too)
 
 The package never imports ``oracle`` and has no CPU fallback.
 """
@@ -16,6 +17,7 @@ from . import _lib  # noqa: F401
 from .env import ErrorFrame, Revolt, RevoltFinal, RevoltLimited, RevoltSimple  # noqa: F401
 from .pinv import pinv_allocate, pinv_pid  # noqa: F401
 from .observer import DPObserver  # noqa: F401
+from .refmodel import ReferenceModel  # noqa: F401
 from .qp_allocator import QPTA  # noqa: F401
 from .rl_allocator import RLTA  # noqa: F401
 from .core import ActorCritic, mlp_actor_critic  # noqa: F401

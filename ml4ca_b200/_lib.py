@@ -49,6 +49,12 @@ class ObserverCfg(ctypes.Structure):
                 ("k3", ctypes.c_float * 3), ("k4", ctypes.c_float * 3)]
 
 
+class RefModelCfg(ctypes.Structure):
+    """struct ml4ca_refmodel_cfg"""
+    _fields_ = [("step_dt", ctypes.c_float), ("zeta", ctypes.c_float * 3), ("omega", ctypes.c_float * 3),
+                ("v_max", ctypes.c_float * 3), ("a_max", ctypes.c_float * 3)]
+
+
 class PolicyCfg(ctypes.Structure):
     """struct ml4ca_policy_cfg"""
     _fields_ = [("obs_dim", ctypes.c_int32), ("act_dim", ctypes.c_int32), ("hidden", ctypes.c_int32),
@@ -96,6 +102,11 @@ _SIGNATURES = {
     "ml4ca_observer_reset": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_u8p, c_f32p, c_stream]),
     "ml4ca_observer_step": (ctypes.c_int, [ctypes.POINTER(ObserverCfg), ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_u8p,
                                            c_f32p, c_stream]),
+    "ml4ca_refmodel_cfg_default": (ctypes.c_int, [ctypes.POINTER(RefModelCfg)]),
+    "ml4ca_refmodel_reset": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_stream]),
+    "ml4ca_refmodel_step": (ctypes.c_int, [ctypes.POINTER(RefModelCfg), ctypes.c_int64, c_f32p, c_f32p, c_stream]),
+    "ml4ca_pinv_pid_ff": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p,
+                                         c_stream]),
     "ml4ca_qp_solve": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),
     "ml4ca_qp_options_default": (ctypes.c_int, [ctypes.POINTER(QpOptions)]),
     "ml4ca_qp_solve_ex": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, ctypes.POINTER(QpOptions), c_f32p, ctypes.c_void_p, c_stream]),

@@ -14,7 +14,7 @@ LIB = os.path.join(HERE, "libml4ca_b200.so")
 STAMP = os.path.join(HERE, ".libml4ca_b200.stamp")
 
 # (source, extra defines, object suffix)
-SOURCES = [("common.cu", [], ""), ("env_step.cu", [], ""), ("pinv_pid.cu", [], ""), ("qp_alloc.cu", [], ""), ("policy.cu", [], ""), ("gae.cu", [], ""), ("ppo_update.cu", [], ""), ("ppo_update_tc.cu", [], ""), ("ppo_update_generic.cu", [], ""), ("peer_comm.cu", [], ""), ("ros_adapter.cu", [], ""), ("eval_metrics.cu", [], ""), ("observer.cu", [], "")] + \
+SOURCES = [("common.cu", [], ""), ("env_step.cu", [], ""), ("pinv_pid.cu", [], ""), ("qp_alloc.cu", [], ""), ("policy.cu", [], ""), ("gae.cu", [], ""), ("ppo_update.cu", [], ""), ("ppo_update_tc.cu", [], ""), ("ppo_update_generic.cu", [], ""), ("peer_comm.cu", [], ""), ("ros_adapter.cu", [], ""), ("eval_metrics.cu", [], ""), ("observer.cu", [], ""), ("refmodel.cu", [], "")] + \
           [("env_step_inst.cu", ["-DML4CA_STEP_UNIT=%d" % u], "_%d" % u) for u in range(5)]
 
 NVCC_FLAGS = [

@@ -118,4 +118,22 @@
 #define ML4CA_OBS_OMEGA_MAX (10.0)
 #define ML4CA_OBS_STATE_ROWS 15         // xi1[3], xi2[3], eta[3], nu[3], b[3]
 
+// ---- DP reference model (Fossen 2011 section 12.1; DECLARED defaults of ml4ca_refmodel_cfg_default) --------------
+// Per DOF (N, E, psi): eta_d / r = w^3 / ((s + w)(s^2 + 2 zeta w s + w^2)) with |v_d| <= V_MAX, |a_d| <= A_MAX.  Tuned
+// on the float64 closed loop of PID + feed-forward + pseudoinverse over the box test (DESIGN.md section 4).
+// Mirrored in tests/refmodel_oracle.py and checked there by tests/test_refmodel_cpu.py.
+#define ML4CA_REF_ZETA_N (1.0)
+#define ML4CA_REF_ZETA_E (1.0)
+#define ML4CA_REF_ZETA_PSI (1.0)
+#define ML4CA_REF_OMEGA_N (0.2)      // rad/s
+#define ML4CA_REF_OMEGA_E (0.2)
+#define ML4CA_REF_OMEGA_PSI (0.25)
+#define ML4CA_REF_V_MAX_N (0.15)     // m/s
+#define ML4CA_REF_V_MAX_E (0.1)      // m/s
+#define ML4CA_REF_V_MAX_PSI (0.1)    // rad/s
+#define ML4CA_REF_A_MAX_N (0.05)     // m/s^2
+#define ML4CA_REF_A_MAX_E (0.02)     // m/s^2
+#define ML4CA_REF_A_MAX_PSI (0.02)   // rad/s^2
+#define ML4CA_REF_STATE_ROWS 9       // eta_d[3], v_d[3], a_d[3]
+
 #endif  // ML4CA_CONSTANTS_H_

@@ -8,12 +8,13 @@
 //   PID   e = R(psi)^T (eta - ref)[0:2],  e_psi = wrap_rad(psi - psi_ref)
 //         I <- clamp(I + dt e, +-sat/Ki)                (anti-windup)
 //         tau = clamp(-(Kp e + Kd nu + Ki I), +-[69, 30, 80])
+//         with velocity feed-forward (ml4ca_pinv_pid_ff): Kd (nu - R(psi)^T v_d), v_d the reference model's NED rates
 //   PINV  extended thrust f = [F1x, F1y, F2x, F2y, F3y] (port, star stern pods; bow fixed at 90 deg),
 //         tau = T f with the 3x5 configuration matrix of the reference geometry (qp_allocator.py:69-70),
 //         f = T^+ tau (T^+ = T^T (T T^T)^-1, a constant 5x3 matrix), F_i = hypot, alpha_i = atan2,
 //         n_i = sign(F_i / K_i) sqrt(|F_i / K_i|) clipped to +-100 % (thrust law qp_allocator.py:284-288).
 //
-// HBM-bound: 80 algorithmic bytes per env (read eta, nu, ref, I = 48; write I, n, alpha = 32).
+// HBM-bound: 80 algorithmic bytes per env (read eta, nu, ref, I = 48; write I, n, alpha = 32); 92 with feed-forward.
 #include <math.h>
 
 #include "common.h"
@@ -77,14 +78,22 @@ __device__ __forceinline__ void pinv_allocate(const PinvMatrix& P, float tx, flo
   n_bow = thrust_percent(f[4], (float)ML4CA_K_BOW);
 }
 
-// One env of the PID + allocation step; integ[k] in: I, out: the updated I.
+// One env of the PID + allocation step; integ[k] in: I, out: the updated I.  FF: the D-term acts on vel - R(psi)^T vd.
+template <bool FF>
 __device__ __forceinline__ void pid_one(const PinvMatrix& P, const float (&eta)[3], const float (&vel)[3], const float (&ref)[3],
-                                        float (&integ)[3], float (&tau)[3], float (&npct)[3], float (&alpha)[2]) {
+                                        const float (&vd)[3], float (&integ)[3], float (&tau)[3], float (&npct)[3],
+                                        float (&alpha)[2]) {
   const float eN = eta[0] - ref[0], eE = eta[1] - ref[1];
   const float ep = wrap_rad(eta[2] - ref[2]);
   float s, c;
   sincosf(eta[2], &s, &c);
   const float e[3] = {c * eN + s * eE, c * eE - s * eN, ep};
+  float dv[3] = {vel[0], vel[1], vel[2]};
+  if constexpr (FF) {
+    dv[0] = vel[0] - (c * vd[0] + s * vd[1]);
+    dv[1] = vel[1] - (c * vd[1] - s * vd[0]);
+    dv[2] = vel[2] - vd[2];
+  }
   const float kp[3] = {(float)ML4CA_PID_KP_X, (float)ML4CA_PID_KP_Y, (float)ML4CA_PID_KP_N};
   const float kd[3] = {(float)ML4CA_PID_KD_X, (float)ML4CA_PID_KD_Y, (float)ML4CA_PID_KD_N};
   const float ki[3] = {(float)ML4CA_PID_KI_X, (float)ML4CA_PID_KI_Y, (float)ML4CA_PID_KI_N};
@@ -95,22 +104,24 @@ __device__ __forceinline__ void pid_one(const PinvMatrix& P, const float (&eta)[
     float I = integ[k] + (float)ML4CA_PID_DT * e[k];
     I = fminf(fmaxf(I, -lim), lim);
     integ[k] = I;
-    const float t = -(kp[k] * e[k] + kd[k] * vel[k] + ki[k] * I);
+    const float t = -(kp[k] * e[k] + kd[k] * dv[k] + ki[k] * I);
     tau[k] = fminf(fmaxf(t, -sat[k]), sat[k]);
   }
   pinv_allocate(P, tau[0], tau[1], tau[2], npct[0], npct[1], npct[2], alpha[0], alpha[1]);
 }
 
 // VEC consecutive envs per thread: with VEC = 2 every row access is 64 bits wide (a warp covers 256 contiguous bytes per
-// row), half the load / store instructions per env of the scalar variant (odd n or unaligned rows).
-template <int VEC>
+// row), half the load / store instructions per env of the scalar variant (odd n or unaligned rows).  FF reads v_d [3, n],
+// the trailing argument (unused without FF, so the FF = false kernels keep the parameter layout of the plain PID).
+template <int VEC, bool FF>
 __global__ void __launch_bounds__(256) pinv_pid_kernel(int64_t n, const PinvMatrix P, const float* __restrict__ eta,
                                                        const float* __restrict__ nu, const float* __restrict__ ref,
                                                        float* __restrict__ integ, float* __restrict__ tau_out,
-                                                       float* __restrict__ n_pct, float* __restrict__ alpha) {
+                                                       float* __restrict__ n_pct, float* __restrict__ alpha,
+                                                       const float* __restrict__ v_d) {
   const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
   if (i >= n) return;
-  float e_[3][VEC], v_[3][VEC], r_[3][VEC], I_[3][VEC];
+  float e_[3][VEC], v_[3][VEC], r_[3][VEC], I_[3][VEC], d_[3][VEC];
   auto ld = [&](const float* row, float (&x)[VEC]) {
     if constexpr (VEC == 2) {
       const float2 t = *reinterpret_cast<const float2*>(row + i);
@@ -132,13 +143,15 @@ __global__ void __launch_bounds__(256) pinv_pid_kernel(int64_t n, const PinvMatr
     ld(nu + (int64_t)k * n, v_[k]);
     ld(ref + (int64_t)k * n, r_[k]);
     ld(integ + (int64_t)k * n, I_[k]);
+    if constexpr (FF) ld(v_d + (int64_t)k * n, d_[k]);
   }
   float tau[3][VEC], np_[3][VEC], al_[2][VEC];
 #pragma unroll
   for (int j = 0; j < VEC; ++j) {
     const float e1[3] = {e_[0][j], e_[1][j], e_[2][j]}, v1[3] = {v_[0][j], v_[1][j], v_[2][j]}, r1[3] = {r_[0][j], r_[1][j], r_[2][j]};
-    float I1[3] = {I_[0][j], I_[1][j], I_[2][j]}, t1[3], n1[3], a1[2];
-    pid_one(P, e1, v1, r1, I1, t1, n1, a1);
+    float I1[3] = {I_[0][j], I_[1][j], I_[2][j]}, t1[3], n1[3], a1[2], d1[3] = {0.f, 0.f, 0.f};
+    if constexpr (FF) d1[0] = d_[0][j], d1[1] = d_[1][j], d1[2] = d_[2][j];
+    pid_one<FF>(P, e1, v1, r1, d1, I1, t1, n1, a1);
 #pragma unroll
     for (int k = 0; k < 3; ++k) I_[k][j] = I1[k], tau[k][j] = t1[k], np_[k][j] = n1[k];
     al_[0][j] = a1[0], al_[1][j] = a1[1];
@@ -170,19 +183,39 @@ using namespace ml4ca;
 
 extern "C" {
 
-int ml4ca_pinv_pid(int64_t n, const float* eta, const float* nu, const float* ref, float* integ, float* tau,
-                   float* n_pct, float* alpha, void* stream) {
-  ML4CA_REQUIRE(n >= 0 && eta && nu && ref && integ && n_pct && alpha, "bad arguments");
+}  // extern "C"
+
+namespace {
+
+template <bool FF>
+int launch_pinv_pid(int64_t n, const float* eta, const float* nu, const float* ref, const float* v_d, float* integ,
+                    float* tau, float* n_pct, float* alpha, void* stream) {
   if (n == 0) return ML4CA_OK;
   static const PinvMatrix P = make_pinv();
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   auto al8 = [](const void* p) { return p == nullptr || (reinterpret_cast<uintptr_t>(p) & 7u) == 0; };
-  if (n % 2 == 0 && al8(eta) && al8(nu) && al8(ref) && al8(integ) && al8(tau) && al8(n_pct) && al8(alpha)) {
-    pinv_pid_kernel<2><<<(unsigned)((n / 2 + 255) / 256), 256, 0, st>>>(n, P, eta, nu, ref, integ, tau, n_pct, alpha);
+  if (n % 2 == 0 && al8(eta) && al8(nu) && al8(ref) && al8(integ) && al8(tau) && al8(n_pct) && al8(alpha) && al8(v_d)) {
+    pinv_pid_kernel<2, FF><<<(unsigned)((n / 2 + 255) / 256), 256, 0, st>>>(n, P, eta, nu, ref, integ, tau, n_pct, alpha, v_d);
   } else {
-    pinv_pid_kernel<1><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, P, eta, nu, ref, integ, tau, n_pct, alpha);
+    pinv_pid_kernel<1, FF><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, P, eta, nu, ref, integ, tau, n_pct, alpha, v_d);
   }
   return check_launch("pinv_pid_kernel");
+}
+
+}  // namespace
+
+extern "C" {
+
+int ml4ca_pinv_pid(int64_t n, const float* eta, const float* nu, const float* ref, float* integ, float* tau,
+                   float* n_pct, float* alpha, void* stream) {
+  ML4CA_REQUIRE(n >= 0 && eta && nu && ref && integ && n_pct && alpha, "bad arguments");
+  return launch_pinv_pid<false>(n, eta, nu, ref, nullptr, integ, tau, n_pct, alpha, stream);
+}
+
+int ml4ca_pinv_pid_ff(int64_t n, const float* eta, const float* nu, const float* ref, const float* v_d, float* integ,
+                      float* tau, float* n_pct, float* alpha, void* stream) {
+  ML4CA_REQUIRE(n >= 0 && eta && nu && ref && v_d && integ && n_pct && alpha, "bad arguments");
+  return launch_pinv_pid<true>(n, eta, nu, ref, v_d, integ, tau, n_pct, alpha, stream);
 }
 
 int ml4ca_pinv_allocate(int64_t n, const float* tau, float* n_pct, float* alpha, void* stream) {

@@ -30,6 +30,76 @@ def sensed(st):
     return st["eta"], st["nu"]
 
 
+def box_test_schedule(side=5.0, yaw_deg=-45.0, hold_s=60.0, dt=0.2):
+    """The four-corner DP box test as a set-point schedule -> (steps [7] int, setpoints [7, 3] (N m, E m, yaw rad)).
+
+    On station at (0, 0, 0), then pure surge to (side, 0, 0), pure sway to (side, side, 0), pure yaw to
+    (side, side, yaw), combined surge and sway to (0, side, yaw), and all three back to (0, 0, 0); the start and every leg
+    are held ``hold_s``.  The last entry marks the end of the run (steps[-1] = 6 holds, the set-point of the final
+    sample), so ``run_allocator`` / ``run_RL_policy`` run exactly the test by default.
+
+    DECLARED, not pinned: the reference's own box-test schedule (results/all_plots/box_test/plot_pos.py) is not available
+    to this build; this is the usual four-corner DP test."""
+    k = int(round(hold_s / dt))
+    y = float(np.deg2rad(yaw_deg))
+    sp = np.array([[0.0, 0.0, 0.0], [side, 0.0, 0.0], [side, side, 0.0], [side, side, y], [0.0, side, y], [0.0, 0.0, 0.0],
+                   [0.0, 0.0, 0.0]])
+    return np.arange(len(sp), dtype=np.int64) * k, sp
+
+
+class _Guidance(object):
+    """The set-point side of an evaluation run with a schedule: s(t), the last entry with steps <= t, and the reference the
+    controllers track, r(t) = s(t), or with a reference model r(t) = eta_d(t) (with v_d(t) for the PID's feed-forward).
+    ``advance(t)`` moves the reference to r(t + 1) (the model steps once on s(t)) and hands it to the env (set_ref)."""
+
+    def __init__(self, env, schedule, reference_model, max_ep_len):
+        n, dev = env.num_envs, env.device
+        steps, sp = schedule
+        steps = np.asarray(steps).reshape(-1)
+        if steps.size == 0 or int(steps[0]) != 0 or np.any(np.diff(steps) <= 0):
+            raise ValueError("schedule steps must start at 0 and be strictly increasing")
+        sp = torch.as_tensor(sp, dtype=torch.float32, device=dev)
+        if sp.dim() == 2 and sp.shape == (steps.size, 3):
+            sp = sp[:, :, None].expand(steps.size, 3, n)
+        elif sp.shape != (steps.size, 3, n):
+            raise ValueError("schedule set-points must be [K, 3] or [K, 3, num_envs] for K = len(steps)")
+        self.sp = sp.contiguous()
+        if reference_model is not None and (reference_model.num_envs != n or
+                                            abs(reference_model.step_dt - float(env.dt)) > 1e-6 * float(env.dt)):
+            raise ValueError("the reference model's num_envs and step_dt must match the env's")
+        self.T = int(max_ep_len if max_ep_len is not None else steps[-1])
+        if self.T < 1:
+            raise ValueError("the run needs at least one step: give max_ep_len or a schedule whose last step is > 0")
+        self.idx = np.searchsorted(steps, np.arange(self.T + 1), side="right") - 1
+        self.env, self.model = env, reference_model
+
+    def s(self, t):
+        return self.sp[int(self.idx[t])]
+
+    def start(self, rec):
+        """r(0) = s(0): the env's set-point before the reset, the model reset on it.  -> the start pose [3, n] numpy."""
+        s0 = self.s(0)
+        self.env.set_ref(s0)
+        f = dict(dtype=torch.float32, device=self.env.device)
+        T, n = self.T, self.env.num_envs
+        rec["setpoint"] = torch.empty(T + 1, 3, n, **f)
+        rec["setpoint"][0] = s0
+        if self.model is not None:
+            self.model.reset(s0)
+            rec["v_d"] = torch.empty(T + 1, 3, n, **f)
+            rec["v_d"][0] = self.model.v_d
+        return s0.double().cpu().numpy()
+
+    def advance(self, t, rec):
+        if self.model is not None:
+            self.model.step(self.s(t))
+            self.env.set_ref(self.model.eta_d.clone())
+            rec["v_d"][t + 1] = self.model.v_d
+        else:
+            self.env.set_ref(self.s(t + 1))
+        rec["setpoint"][t + 1] = self.s(t + 1)
+
+
 def in_loop_observer(env, observer):
     """The observer a controller acts on: the one attached to ``env`` (``Revolt.set_observer``), which the env steps and
     resets itself, else ``observer``.  -> (observer, attached).  A second observer next to an attached one is an error."""
@@ -42,7 +112,8 @@ def in_loop_observer(env, observer):
     return attached, True
 
 
-def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False, observer=None):
+def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, integrator=False, observer=None,
+                  schedule=None, reference_model=None):
     """test_policy.py:97-186 for every env of ``env`` at once (one episode each, no early stop: finished runs keep
     being recorded, ``done_at`` tells where the reference loop would have cut).  Returns a dict of device tensors:
     obs [T+1, obs, n], rew [T, n], eta [T+1, 3, n], thrust [T+1, 3, n], angles [T+1, 2, n], ref [T+1, 3, n], done_at [n],
@@ -67,18 +138,33 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     [T+1, 3, n] are recorded; ``eta`` and the metrics keep the LF pose and the applied thrust.  On an env with an attached
     observer (``Revolt.set_observer``) that observer is used: the env resets and steps it, and the policy input without
     the integrator is the env's observation, which is already formed from the estimates.  Passing another observer then
-    raises ValueError."""
+    raises ValueError.
+
+    schedule = (steps [K], setpoints [K, 3] or [K, 3, n]): a set-point schedule such as ``box_test_schedule()``; s(t) is
+    the entry of the last step <= t, steps ascend strictly from 0, T defaults to steps[-1].  Every run then starts at
+    rest at s(0) instead of the fixed test poses.  The controller tracks r(t): s(t), or with ``reference_model`` (a
+    ``ReferenceModel`` of the env's num_envs and step_dt, reset on s(0)) its eta_d(t).  In step t the policy acts on
+    observation t, formed with r(t), then the reference advances to r(t + 1) (the model steps once on s(t)), the env
+    takes it (set_ref) and steps: a schedule change at step k first shows in sample k.  The state assembly uses r(t).
+    Records gain ``setpoint`` [T+1, 3, n] (s), ``ref`` is r, and with a model ``v_d`` [T+1, 3, n]; the IAE integrates
+    against ``setpoint``, so runs with and without a reference model are scored against the same command.  A schedule
+    together with new_ref / ref_change_at, bad steps, set-points of the wrong shape or a model that does not match the
+    env raise ValueError; so does a reference model without a schedule."""
     observer, attached = in_loop_observer(env, observer)
     n, dev = env.num_envs, env.device
-    T = int(max_ep_len if max_ep_len is not None else env.max_ep_len)
-    eta0 = fixed_test_poses(n)
+    plan = _plan(env, schedule, reference_model, max_ep_len)
+    if plan is not None and (new_ref is not None or ref_change_at is not None):
+        raise ValueError("a schedule replaces new_ref / ref_change_at: pass one or the other")
+    T = plan.T if plan is not None else int(max_ep_len if max_ep_len is not None else env.max_ep_len)
+    rec = {}
+    eta0 = plan.start(rec) if plan is not None else fixed_test_poses(n)
     o = env.reset(**{'Hull.PosNED': eta0[0:2], 'Hull.PosAttitude': np.stack([np.zeros(n), np.zeros(n), eta0[2]]),
                      'Hull.VelocityNu': np.zeros((6, n))})
     o = torch.as_tensor(o, dtype=torch.float32, device=dev).reshape(env.num_states, n)
     f = dict(dtype=torch.float32, device=dev)
-    rec = {"obs": torch.empty(T + 1, env.num_states, n, **f), "rew": torch.zeros(T, n, **f),
-           "eta": torch.empty(T + 1, 3, n, **f), "thrust": torch.zeros(T + 1, 3, n, **f),
-           "angles": torch.zeros(T + 1, 2, n, **f), "ref": torch.empty(T + 1, 3, n, **f)}
+    rec.update({"obs": torch.empty(T + 1, env.num_states, n, **f), "rew": torch.zeros(T, n, **f),
+                "eta": torch.empty(T + 1, 3, n, **f), "thrust": torch.zeros(T + 1, 3, n, **f),
+                "angles": torch.zeros(T + 1, 2, n, **f), "ref": torch.empty(T + 1, 3, n, **f)})
     done_at = torch.full((n,), T, dtype=torch.int32, device=dev)
     st = env.get_state()
     rec["obs"][0], rec["eta"][0], rec["angles"][0], rec["ref"][0] = o, st["eta"], st["angles"][1:3], env._ref
@@ -108,6 +194,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
         return x
     for t in range(T):
         a = ac.get_action(policy_input(o, st, rec["ref"][t]))                # deterministic action = mu (:90-93)
+        if plan is not None:
+            plan.advance(t, rec)
         rec["ref"][t + 1] = env._ref                                         # the set-point the step's observation is formed with
         if ref_change_at is not None and t == ref_change_at and new_ref is not None:
             o, r, d, _ = env.step(torch.zeros_like(a), new_ref=new_ref)      # :141-146
@@ -126,13 +214,22 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     steps = torch.arange(T, device=dev)[:, None]
     rec["ep_ret"] = (rec["rew"] * (steps < done_at[None, :])).sum(dim=0)
     # IAE depends on eta - ref only: the per-sample error against a zero set-point is the metric of a varying set-point
-    rec["metrics"] = metrics(rec["eta"] - rec["ref"], torch.zeros(3, n, **f), rec["thrust"], rec["angles"], env.dt)
+    cmd = rec["setpoint"] if plan is not None else rec["ref"]
+    rec["metrics"] = metrics(rec["eta"] - cmd, torch.zeros(3, n, **f), rec["thrust"], rec["angles"], env.dt)
     if integrator:
         rec["integrator"] = integ
     return rec
 
 
-def run_allocator(env, method="qp", max_ep_len=None, observer=None):
+def _plan(env, schedule, reference_model, max_ep_len):
+    if schedule is None:
+        if reference_model is not None:
+            raise ValueError("a reference model needs a schedule to filter")
+        return None
+    return _Guidance(env, schedule, reference_model, max_ep_len)
+
+
+def run_allocator(env, method="qp", max_ep_len=None, observer=None, schedule=None, reference_model=None):
     """The classical DP pipeline in the same batched env: PID on the body-frame error (ml4ca_pinv_pid) -> thrust
     allocation by the SLSQP-equivalent kernel (``method='qp'``, QPTA.tau_controller_callback_func) or the fixed-matrix
     pseudoinverse (``'pinv'``) -> env step.  Same records and metrics as run_RL_policy: with it, the thesis' comparison
@@ -141,19 +238,26 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
 
     observer: a ``DPObserver`` between the sensors and the PID, as in run_RL_policy: the PID acts on (eta^, nu^); the
     records gain ``eta_hat`` and ``bias_hat`` [T+1, 3, n].  On an env with an attached observer that observer is used, as
-    in run_RL_policy."""
+    in run_RL_policy.
+
+    schedule / reference_model: as in run_RL_policy.  The PID acts on r(t), and with a reference model it also gets
+    v_d(t) as velocity feed-forward (``pinv_pid(nu_d=)``).  Records gain ``setpoint``, ``ref`` (r) [T+1, 3, n], with a
+    model ``v_d``, and for ``method='qp'`` ``demand_clipped`` [T, n] (bool: the +-[4, 2, 2] demand clip below bound in
+    some DOF at that step)."""
     observer, attached = in_loop_observer(env, observer)
     from .pinv import pinv_pid
     from .qp_allocator import QPTA
     n, dev = env.num_envs, env.device
     assert env.name == 'revoltfinal', "the allocators command two rotating stern azimuths + the fixed bow thruster"
-    T = int(max_ep_len if max_ep_len is not None else env.max_ep_len)
-    eta0 = fixed_test_poses(n)
+    plan = _plan(env, schedule, reference_model, max_ep_len)
+    T = plan.T if plan is not None else int(max_ep_len if max_ep_len is not None else env.max_ep_len)
+    rec = {}
+    eta0 = plan.start(rec) if plan is not None else fixed_test_poses(n)
     o = env.reset(**{'Hull.PosNED': eta0[0:2], 'Hull.PosAttitude': np.stack([np.zeros(n), np.zeros(n), eta0[2]]),
                      'Hull.VelocityNu': np.zeros((6, n))})
     f = dict(dtype=torch.float32, device=dev)
-    rec = {"rew": torch.zeros(T, n, **f), "eta": torch.empty(T + 1, 3, n, **f), "thrust": torch.zeros(T + 1, 3, n, **f),
-           "angles": torch.zeros(T + 1, 2, n, **f)}
+    rec.update({"rew": torch.zeros(T, n, **f), "eta": torch.empty(T + 1, 3, n, **f),
+                "thrust": torch.zeros(T + 1, 3, n, **f), "angles": torch.zeros(T + 1, 2, n, **f)})
     st = env.get_state()
     rec["eta"][0], rec["angles"][0] = st["eta"], st["angles"][1:3]
     if observer is not None:
@@ -165,6 +269,11 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
     qp = QPTA(num_envs=n, device=dev) if method == "qp" else None
     action = torch.empty(env.num_actions, n, **f)
     ref = env._ref.clone()
+    if plan is not None:
+        rec["ref"] = torch.empty(T + 1, 3, n, **f)
+        rec["ref"][0] = ref
+        if qp is not None:
+            rec["demand_clipped"] = torch.empty(T, n, dtype=torch.bool, device=dev)
     # The SLSQP programme only admits demands its rate limits can follow (|df| <= 5, 5, 2 N per call): on the vessel the
     # reference filter feeds it smooth demands.  Stand-in: the demand is the wrench the thrusters deliver now plus the
     # PID's request clipped to +-[4, 2, 2] -- the neighbourhood law of BASELINE config 1 (99.7 % success with the
@@ -180,10 +289,16 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
     trust = torch.ones(n, **f)     # per-run scale of the clip: halved when the programme is infeasible (the allocator then
     for t in range(T):             # holds its state, qp_allocator.py:267-269), restored step by step when it succeeds
         eta_s, nu_s = sensed(st) if observer is None else (observer.eta_hat.contiguous(), observer.nu_hat.contiguous())
-        n_pct, alpha, tau = pinv_pid(eta_s, nu_s, ref, integ, return_tau=True)
+        if plan is None:
+            n_pct, alpha, tau = pinv_pid(eta_s, nu_s, ref, integ, return_tau=True)
+        else:
+            nu_d = rec["v_d"][t] if "v_d" in rec else None
+            n_pct, alpha, tau = pinv_pid(eta_s, nu_s, rec["ref"][t], integ, return_tau=True, nu_d=nu_d)
         if qp is not None:
             now = delivered(qp._prev)
             lim = slew * trust[None, :]
+            if plan is not None:
+                rec["demand_clipped"][t] = ((tau - now).abs() > lim).any(dim=0)
             qp.tau_controller_callback_func(now + torch.minimum(torch.maximum(tau - now, -lim), lim))
             ok = (qp.last_status & 1).bool()
             trust = torch.where(ok, (trust * 2).clamp(max=1.0), trust * 0.5)
@@ -192,6 +307,9 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
             _lib.check(_lib.lib().ml4ca_alloc_to_action(n, int(env.cont_ang), float(env.real_action_bounds[3]), _lib.ptr(n_pct),
                                                         _lib.ptr(alpha), _lib.ptr(action), _lib.current_stream()),
                        "ml4ca_alloc_to_action")
+        if plan is not None:
+            plan.advance(t, rec)
+            rec["ref"][t + 1] = env._ref
         o, r, d, _ = env.step(action)
         st = env.get_state()
         rec["rew"][t], rec["eta"][t + 1] = r, st["eta"]
@@ -201,7 +319,10 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None):
                 observer.step(sensed(st)[0], st["prev_thrust"], st["angles"])
             rec["eta_hat"][t + 1], rec["bias_hat"][t + 1] = observer.eta_hat, observer.bias_hat
     rec["ep_ret"] = rec["rew"].sum(dim=0)
-    rec["metrics"] = metrics(rec["eta"], ref, rec["thrust"], rec["angles"], env.dt)
+    if plan is None:
+        rec["metrics"] = metrics(rec["eta"], ref, rec["thrust"], rec["angles"], env.dt)
+    else:
+        rec["metrics"] = metrics(rec["eta"] - rec["setpoint"], torch.zeros(3, n, **f), rec["thrust"], rec["angles"], env.dt)
     return rec
 
 

@@ -29,10 +29,12 @@ def pinv_allocate(tau, device=None):
     return n_pct, alpha
 
 
-def pinv_pid(eta, nu, ref, integ, device=None, return_tau=False):
+def pinv_pid(eta, nu, ref, integ, device=None, return_tau=False, nu_d=None):
     """One DP control step: PID on the body-frame error, then pseudoinverse allocation.
 
     eta, nu, ref [3, n]; integ [3, n] float32 CUDA tensor updated IN PLACE (integral state).
+    nu_d [3, n]: velocity feed-forward, the desired NED rates of a reference model (``ReferenceModel.v_d``); the D-term
+    then acts on nu - R(psi)^T nu_d (ml4ca_pinv_pid_ff).
     Returns (n_pct [3, n], alpha [2, n]) and the saturated wrench tau [3, n] if return_tau.
     """
     assert torch.is_tensor(integ) and integ.is_cuda and integ.dtype == torch.float32 and integ.is_contiguous(), \
@@ -45,7 +47,14 @@ def pinv_pid(eta, nu, ref, integ, device=None, return_tau=False):
     alpha = torch.empty(2, n, dtype=torch.float32, device=device)
     tau = torch.empty(3, n, dtype=torch.float32, device=device) if return_tau else None
     with torch.cuda.device(device):
-        _lib.check(_lib.lib().ml4ca_pinv_pid(n, _lib.ptr(eta), _lib.ptr(nu), _lib.ptr(ref), _lib.ptr(integ),
-                                             _lib.ptr(tau), _lib.ptr(n_pct), _lib.ptr(alpha),
-                                             _lib.current_stream()), "ml4ca_pinv_pid")
+        if nu_d is None:
+            _lib.check(_lib.lib().ml4ca_pinv_pid(n, _lib.ptr(eta), _lib.ptr(nu), _lib.ptr(ref), _lib.ptr(integ),
+                                                 _lib.ptr(tau), _lib.ptr(n_pct), _lib.ptr(alpha),
+                                                 _lib.current_stream()), "ml4ca_pinv_pid")
+        else:
+            nu_d = _f32(nu_d, 3, device)
+            assert nu_d.shape == (3, n)
+            _lib.check(_lib.lib().ml4ca_pinv_pid_ff(n, _lib.ptr(eta), _lib.ptr(nu), _lib.ptr(ref), _lib.ptr(nu_d),
+                                                    _lib.ptr(integ), _lib.ptr(tau), _lib.ptr(n_pct), _lib.ptr(alpha),
+                                                    _lib.current_stream()), "ml4ca_pinv_pid_ff")
     return (n_pct, alpha, tau) if return_tau else (n_pct, alpha)
