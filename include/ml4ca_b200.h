@@ -257,6 +257,21 @@ ML4CA_API int ml4ca_refmodel_step(const ml4ca_refmodel_cfg* cfg, int64_t n, cons
  * D-term into Kd (nu - R(psi)^T v_d), psi = eta[2].  Other arguments as ml4ca_pinv_pid; v_d is required. */
 ML4CA_API int ml4ca_pinv_pid_ff(int64_t n, const float* eta, const float* nu, const float* ref, const float* v_d,
                                 float* integ, float* tau, float* n_pct, float* alpha, void* stream);
+/* DP reference model in the loop: attach (cfg != NULL) or detach (cfg = NULL) a reference model that every env step runs
+ * inside the step kernel.  state [9, n] is caller-owned, laid out as for ml4ca_refmodel_step, and must outlive the
+ * attachment.  cfg is validated as by ml4ca_refmodel_step (Jury test included) and cfg->step_dt must equal the env's
+ * step_dt.  Attaching re-initialises every env's column from its current LF pose (eta_d = eta, v_d = a_d = 0) on `stream`.
+ * While attached, the env's set-point rows (ml4ca_env_set_ref) hold the operator's command s.  Each step first advances
+ * the env's column once on s (eta_d(t) -> eta_d(t+1), the arithmetic of ml4ca_refmodel_step), and then forms everything
+ * it forms against the set-point against eta_d(t+1) instead: observation rows 0-2 (and an attached observer's error
+ * frame), the reward and the termination.  Rows 3-8 are unchanged; the reward's velocity penalty still acts on nu.  So a
+ * step equals, bit for bit, ml4ca_refmodel_step on s, ml4ca_env_set_ref(eta_d) and a step without the model.  cut_obs is
+ * formed after this step's advance and before the restart.  An in-kernel restart, a reset or reset_to starts the env's
+ * column again at the new episode's LF pose (not the measured one), and ml4ca_env_observe forms rows 0-2 against the
+ * current eta_d.  Cost: 72 B more per env-step (read 36, write 36), e.g. 177 -> 249 B for RevoltFinal (extended,
+ * continuous angles).  Launch parameter: CUDA graphs captured earlier keep theirs.  Bad configurations, a NULL state, a
+ * step_dt mismatch: ML4CA_ERR_INVALID. */
+ML4CA_API int ml4ca_env_set_refmodel(ml4ca_env* env, const ml4ca_refmodel_cfg* cfg, float* state, void* stream);
 
 /* QPTA.solve_QP (src/qp/ROS/qp_allocator/src/qp_allocator.py:108-234): tau [3, n] desired wrench, prev [5, n]
  * previous thruster state [f_port, f_star, f_bow, a_port, a_star] -> x [8, n] = [f(3), a(2), s(3)] after the

@@ -105,6 +105,7 @@ _SIGNATURES = {
     "ml4ca_refmodel_cfg_default": (ctypes.c_int, [ctypes.POINTER(RefModelCfg)]),
     "ml4ca_refmodel_reset": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_stream]),
     "ml4ca_refmodel_step": (ctypes.c_int, [ctypes.POINTER(RefModelCfg), ctypes.c_int64, c_f32p, c_f32p, c_stream]),
+    "ml4ca_env_set_refmodel": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(RefModelCfg), c_f32p, c_stream]),
     "ml4ca_pinv_pid_ff": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p,
                                          c_stream]),
     "ml4ca_qp_solve": (ctypes.c_int, [ctypes.c_int64, c_f32p, c_f32p, c_f32p, ctypes.c_void_p, c_stream]),

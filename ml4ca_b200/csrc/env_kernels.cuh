@@ -20,6 +20,7 @@
 #include "common.h"
 #include "env_math.cuh"
 #include "observer_math.cuh"
+#include "refmodel_math.cuh"
 
 #ifndef ML4CA_ENV_MIN_BLOCKS
 #define ML4CA_ENV_MIN_BLOCKS 6  // scalar-row kernel: 40 registers, 48 resident warps/SM (measured best on B200)
@@ -43,7 +44,12 @@
 #endif
 
 #ifndef ML4CA_ENV_MIN_BLOCKS_OBSV
-#define ML4CA_ENV_MIN_BLOCKS_OBSV 2  // step with the observer in the loop (any LAG / DIST / WAVE): at most 128 registers
+#define ML4CA_ENV_MIN_BLOCKS_OBSV 2  // step with the observer in the loop (any LAG / DIST / WAVE / REF): at most 128 registers
+#endif                              // (94-118 with the reference model as well, no spills)
+
+#ifndef ML4CA_ENV_MIN_BLOCKS_REF
+#define ML4CA_ENV_MIN_BLOCKS_REF 3  // step with the reference model in the loop, no observer (any LAG / DIST / WAVE): 63-79
+                                    // registers, no spills; 4 CTAs (64 registers) spill 4-28 B in the WAVE variants
 #endif
 
 namespace ml4ca {
@@ -101,6 +107,13 @@ struct ObserverParams {
   ObsConsts k;
 };
 
+// DP reference model in the loop (ml4ca_env_set_refmodel): the step kernel's last argument, after ObserverParams, for the
+// reason given at DistParams.  state belongs to the caller and is NULL while no model is attached.
+struct RefParams {
+  float* state;        // [9, n] rows eta_d, v_d, a_d (refmodel_math.cuh)
+  RefConsts k;
+};
+
 }  // namespace ml4ca
 
 namespace ml4ca {
@@ -130,6 +143,7 @@ struct ml4ca_env {
   ml4ca::DistParams dist = {};
   ml4ca::WaveParams wave = {};
   ml4ca::ObserverParams obsv = {};
+  ml4ca::RefParams refm = {};
 };
 
 namespace ml4ca {
@@ -218,16 +232,25 @@ __device__ __forceinline__ void st_flags(uint8_t* __restrict__ row, int64_t i, c
 // those of the kernel without it.  cut_obs is the estimate-based observation before the restart; a restart re-initialises
 // the column from the new episode's measured pose (nu^ = 0 in the returned observation).  124 B more per env-step
 // (read 60 + 4, write 60): 301 B for RevoltFinal (extended, continuous angles), 353 B in waves.
-template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false, bool WAVE = false, bool OBSV = false>
-__global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_DIST : ML4CA_ENV_MIN_BLOCKS_WAVE) : (DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1))))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
+// REF = true (one env per thread only): the DP reference model of ml4ca_env_set_refmodel runs in the loop.  Its column
+// first takes one step (refmodel_advance) on the set-point rows s, and everything the step forms against the set-point
+// then uses eta_d(t+1) instead: observation rows 0-2 (and the observer's error frame), the reward and the termination.
+// cut_obs is formed after the advance and before the restart; a restart starts the column again at the new episode's LF
+// pose (eta_d = eta, v_d = a_d = 0).  72 B more per env-step (read 36, write 36; s is read anyway): 249 B for RevoltFinal
+// (extended, continuous angles), 373 B with the observer.
+template <int KIND, bool CONT, bool EXT, int VEC, bool LAG = false, bool DIST = false, bool WAVE = false, bool OBSV = false,
+          bool REF = false>
+__global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (REF ? ML4CA_ENV_MIN_BLOCKS_REF : (WAVE ? (DIST ? ML4CA_ENV_MIN_BLOCKS_WAVE_DIST : ML4CA_ENV_MIN_BLOCKS_WAVE) : (DIST ? ML4CA_ENV_MIN_BLOCKS_DIST : (VEC == 1 ? ML4CA_ENV_MIN_BLOCKS : (VEC == 2 ? ML4CA_ENV_MIN_BLOCKS2 : 1)))))) env_step_kernel(const EnvParams p, const float* __restrict__ action,
                                                        float* __restrict__ obs, float* __restrict__ rew,
                                                        uint8_t* __restrict__ done, const DistParams d,
-                                                       const WaveParams wv, const ObserverParams ob) {
+                                                       const WaveParams wv, const ObserverParams ob,
+                                                       const RefParams rf) {
   using T = EnvTraits<KIND, CONT>;
   static_assert(!LAG || VEC == 1, "the lagged integrator is scalar");
   static_assert(!DIST || VEC == 1, "the disturbed step is scalar");
   static_assert(!WAVE || VEC == 1, "the step with wave motion is scalar");
   static_assert(!OBSV || VEC == 1, "the step with the observer in the loop is scalar");
+  static_assert(!REF || VEC == 1, "the step with the reference model in the loop is scalar");
   const int64_t n = p.n, ios = p.io_stride;
   const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * VEC;
   if (i0 >= p.count) return;
@@ -279,6 +302,11 @@ __global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE 
 #pragma unroll
     for (int r = 0; r < 15; ++r) ox[r] = ob.state[(int64_t)r * n + i0];
     wo = clamp_omega(ob.omega[i0]);
+  }
+  float rx[9];                                                         // VEC == 1 when REF
+  if constexpr (REF) {
+#pragma unroll
+    for (int q = 0; q < 9; ++q) rx[q] = rf.state[(int64_t)q * n + i0];
   }
 
   float o[9][VEC], rw[VEC];
@@ -362,6 +390,11 @@ __global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE 
   }
   // ---- phase C: observation, reward, termination --------------------------------------------------------------------
   if constexpr (WAVE) advance_waves(p.seed, p.env_off + i0, ep[0] + 1, wv.k, w0, wm, wr);   // word after this step
+  if constexpr (REF) {                 // eta_d(t) -> eta_d(t+1) on s; from here on the step forms everything against eta_d
+    const float s[3] = {ref[0][0], ref[1][0], ref[2][0]};
+    refmodel_advance(rx, s, rf.k);
+    ref[0][0] = rx[0], ref[1][0] = rx[1], ref[2][0] = rx[2];
+  }
 #pragma unroll
   for (int j = 0; j < VEC; ++j) {
     float mN = eta[0][j], mE = eta[1][j], mP = eta[2][j], mu = nu[0][j], mv = nu[1][j], mr = nu[2][j];
@@ -432,6 +465,11 @@ __global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE 
         for (int c = 0; c < 3; ++c) wm[c] = xj[c], wr[c] = xdj[c];
         add_wave_motion(mN, mE, mP, mu, mv, mr, wm, wr);
       }
+      if constexpr (REF) {                                             // eta_d = the new LF pose, v_d = a_d = 0
+#pragma unroll
+        for (int q = 0; q < 9; ++q) rx[q] = q < 3 ? eta[q][j] : 0.f;
+        ref[0][j] = rx[0], ref[1][j] = rx[1], ref[2][j] = rx[2];
+      }
       float t0[3] = {0.f, 0.f, 0.f};                                   // customEnv.py:190
       if (p.reset_acts) sample_reset_thrust(p.seed, p.env_off + i0 + j, ep[j], t0);   // :179-188 (old episode word)
       ep[j] = next_episode_word(ep[j]);
@@ -473,6 +511,10 @@ __global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE 
 #pragma unroll
     for (int r = 0; r < 15; ++r) ob.state[(int64_t)r * n + i0] = ox[r];
   }
+  if constexpr (REF) {
+#pragma unroll
+    for (int q = 0; q < 9; ++q) rf.state[(int64_t)q * n + i0] = rx[q];
+  }
 #pragma unroll
   for (int c = 0; c < (EXT ? 9 : 6); ++c) st_row<VEC>(obs + (int64_t)c * ios, i0, o[c]);
   st_row<VEC>(rew, i0, rw);
@@ -482,12 +524,15 @@ __global__ void __launch_bounds__(256, OBSV ? ML4CA_ENV_MIN_BLOCKS_OBSV : (WAVE 
 // ---- reset ----------------------------------------------------------------------------------------------------------
 // mask nullable; explicit eta/nu (reset_to) or Philox sampling.  Writes obs for the reset envs only.  With an observer
 // attached, the reset columns of its state start from the measured pose (eta^ = y, the rest 0) and obs rows 3-5 are nu^ = 0.
+// With a reference model attached, the reset columns of its state start from the LF pose (eta_d = eta, v_d = a_d = 0) and
+// obs rows 0-2 are formed against that eta_d.
 template <int KIND, bool CONT, bool EXT>
 __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const uint8_t* __restrict__ mask,
                                                         const float* __restrict__ eta_in,
                                                         const float* __restrict__ nu_in,
                                                         float* __restrict__ obs, const DistParams d,
-                                                        const WaveParams wv, const ObserverParams ob) {
+                                                        const WaveParams wv, const ObserverParams ob,
+                                                        const RefParams rf) {
   using T = EnvTraits<KIND, CONT>;
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= p.n) return;
@@ -503,6 +548,15 @@ __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const
   }
   p.eta[i] = N, p.eta[n + i] = E, p.eta[2 * n + i] = psi;
   p.nu[i] = u, p.nu[n + i] = v, p.nu[2 * n + i] = r;
+  float rN, rE, rP;                                                                    // what obs rows 0-2 are formed against
+  if (rf.state != nullptr) {                                                           // reference model attached
+    rN = N, rE = E, rP = psi;
+    rf.state[i] = N, rf.state[n + i] = E, rf.state[2 * n + i] = psi;
+#pragma unroll
+    for (int q = 3; q < 9; ++q) rf.state[q * n + i] = 0.f;
+  } else {
+    rN = p.ref[i], rE = p.ref[n + i], rP = p.ref[2 * n + i];
+  }
   float t0[3] = {0.f, 0.f, 0.f};                                                       // customEnv.py:190
   if (p.reset_acts) sample_reset_thrust(p.seed, p.env_off + i, epi, t0);               // :179-188
   p.prev_thrust[i] = t0[0], p.prev_thrust[n + i] = t0[1], p.prev_thrust[2 * n + i] = t0[2];
@@ -535,7 +589,7 @@ __global__ void __launch_bounds__(256) env_reset_kernel(const EnvParams p, const
   p.ep_len[i] = next_episode_word(epi);
   if (obs != nullptr) {
     float xb, yb, pb;
-    error_frame(N, E, psi, p.ref[i], p.ref[n + i], p.ref[2 * n + i], xb, yb, pb);
+    error_frame(N, E, psi, rN, rE, rP, xb, yb, pb);
     obs[i] = xb, obs[n + i] = yb, obs[2 * n + i] = pb;
     obs[3 * n + i] = u, obs[4 * n + i] = v, obs[5 * n + i] = r;
     if constexpr (EXT) obs[6 * n + i] = div100(t0[0]), obs[7 * n + i] = div100(t0[1]), obs[8 * n + i] = div100(t0[2]);

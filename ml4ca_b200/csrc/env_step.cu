@@ -19,9 +19,10 @@ __global__ void __launch_bounds__(256) error_frame_kernel(int64_t n, const float
 }
 
 // Revolt.state() / state_extended() (customEnv.py:196-205) from the state in HBM; with waves enabled, of the measured
-// pose and velocity; with an observer attached, rows 0-5 of its estimates eta^ and nu^.
+// pose and velocity; with an observer attached, rows 0-5 of its estimates eta^ and nu^; with a reference model attached,
+// rows 0-2 against its eta_d.
 __global__ void __launch_bounds__(256) observe_kernel(const EnvParams p, int ext, float* __restrict__ obs,
-                                                      const WaveParams w, const ObserverParams ob) {
+                                                      const WaveParams w, const ObserverParams ob, const RefParams rf) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
   if (i >= n) return;
   float N = p.eta[i], E = p.eta[n + i], psi = p.eta[2 * n + i], u = p.nu[i], v = p.nu[n + i], r = p.nu[2 * n + i];
@@ -34,8 +35,9 @@ __global__ void __launch_bounds__(256) observe_kernel(const EnvParams p, int ext
     N = ob.state[6 * n + i], E = ob.state[7 * n + i], psi = ob.state[8 * n + i];
     u = ob.state[9 * n + i], v = ob.state[10 * n + i], r = ob.state[11 * n + i];
   }
+  const float* ref = rf.state != nullptr ? rf.state : p.ref;                        // eta_d: rows 0-2 of the model's state
   float xb, yb, pb;
-  error_frame(N, E, psi, p.ref[i], p.ref[n + i], p.ref[2 * n + i], xb, yb, pb);
+  error_frame(N, E, psi, ref[i], ref[n + i], ref[2 * n + i], xb, yb, pb);
   obs[i] = xb, obs[n + i] = yb, obs[2 * n + i] = pb;
   obs[3 * n + i] = u, obs[4 * n + i] = v, obs[5 * n + i] = r;
   if (ext) obs[6 * n + i] = p.obs_tail[i], obs[7 * n + i] = p.obs_tail[n + i], obs[8 * n + i] = p.obs_tail[2 * n + i];
@@ -181,6 +183,16 @@ __global__ void __launch_bounds__(256) attach_observer_kernel(const EnvParams p,
   for (int c = 0; c < 15; ++c) ob.state[c * n + i] = s[c];
 }
 
+// ml4ca_env_set_refmodel: every env's reference-model column starts from its current LF pose (eta_d = eta, v_d = a_d = 0).
+__global__ void __launch_bounds__(256) attach_refmodel_kernel(const EnvParams p, const RefParams rf) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = p.n;
+  if (i >= n) return;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) rf.state[c * n + i] = p.eta[c * n + i];
+#pragma unroll
+  for (int q = 3; q < 9; ++q) rf.state[q * n + i] = 0.f;
+}
+
 static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&scale)[6]) {
   // fp32, one rounding per product, same order as oracle/env_oracle.py::sample_reset
   const float vfr = (float)ML4CA_VEL_FRACTION * fraction;
@@ -190,7 +202,8 @@ static void make_reset_scale(const ml4ca_env_cfg& c, float fraction, float (&sca
 
 #define ML4CA_DECL_UNIT(name)                                                                                   \
   int launch_step_##name(const ml4ca_env*, const EnvParams&, const DistParams&, const WaveParams&,              \
-                         const ObserverParams&, const float*, float*, float*, uint8_t*, cudaStream_t);          \
+                         const ObserverParams&, const RefParams&, const float*, float*, float*, uint8_t*,       \
+                         cudaStream_t);                                                                         \
   int launch_reset_##name(const ml4ca_env*, const EnvParams&, const uint8_t*, const float*, const float*, float*, \
                           cudaStream_t);
 ML4CA_DECL_UNIT(full)
@@ -214,16 +227,18 @@ static int launch_step(const ml4ca_env* e, int64_t first, int64_t count, int64_t
   if (w.motion != nullptr) w.motion += first, w.rate += first, w.omega += first;
   ObserverParams ob = e->obsv;
   if (ob.state != nullptr) ob.state += first, ob.omega += first;
+  RefParams rf = e->refm;
+  if (rf.state != nullptr) rf.state += first;
   p.env_off += first;
   p.count = count;
   p.io_stride = io_stride;
   switch (e->cfg.kind) {
-    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, w, ob, action, obs, rew, done, st);
-    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, w, ob, action, obs, rew, done, st);
-    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, w, ob, action, obs, rew, done, st);
+    case ML4CA_ENV_FULL: return launch_step_full(e, p, d, w, ob, rf, action, obs, rew, done, st);
+    case ML4CA_ENV_SIMPLE: return launch_step_simple(e, p, d, w, ob, rf, action, obs, rew, done, st);
+    case ML4CA_ENV_LIMITED: return launch_step_limited(e, p, d, w, ob, rf, action, obs, rew, done, st);
     default:
-      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, w, ob, action, obs, rew, done, st)
-                             : launch_step_final_wrap(e, p, d, w, ob, action, obs, rew, done, st);
+      return e->cfg.cont_ang ? launch_step_final_cont(e, p, d, w, ob, rf, action, obs, rew, done, st)
+                             : launch_step_final_wrap(e, p, d, w, ob, rf, action, obs, rew, done, st);
   }
 }
 
@@ -516,6 +531,25 @@ int ml4ca_env_set_observer(ml4ca_env* env, const ml4ca_observer_cfg* cfg, float*
   return rc;
 }
 
+int ml4ca_env_set_refmodel(ml4ca_env* env, const ml4ca_refmodel_cfg* cfg, float* state, void* stream) {
+  ML4CA_REQUIRE(env != nullptr, "env is NULL");
+  if (cfg == nullptr) {
+    env->refm.state = nullptr;
+    return ML4CA_OK;
+  }
+  RefParams rf;
+  const int stv = refmodel_consts(cfg, rf.k);
+  if (stv != ML4CA_OK) return stv;
+  ML4CA_REQUIRE(state != nullptr, "state [9, n] is required");
+  ML4CA_REQUIRE(cfg->step_dt == env->cfg.step_dt, "the reference model's step_dt must equal the env's step_dt");
+  DeviceGuard guard(env->device);
+  rf.state = state;
+  attach_refmodel_kernel<<<(unsigned)((env->n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(env->p, rf);
+  const int rc = check_launch("attach_refmodel_kernel");
+  if (rc == ML4CA_OK) env->refm = rf;
+  return rc;
+}
+
 int ml4ca_env_set_ref(ml4ca_env* env, const float* ref, void* stream) {
   ML4CA_REQUIRE(env != nullptr && ref != nullptr, "env and ref are required");
   DeviceGuard guard(env->device);
@@ -611,7 +645,7 @@ int ml4ca_env_observe(ml4ca_env* env, float* obs, void* stream) {
                 "ml4ca_env_step the observation lives in the caller's obs buffer");
   DeviceGuard guard(env->device);
   observe_kernel<<<(unsigned)((env->n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      env->p, env->cfg.extended_state, obs, env->wave, env->obsv);
+      env->p, env->cfg.extended_state, obs, env->wave, env->obsv, env->refm);
   return check_launch("observe_kernel");
 }
 

@@ -213,6 +213,7 @@ class Revolt(object):
         self._disturbance = None         # the arguments of the last set_disturbance(), None = calm water
         self._waves = None               # the arguments of the last set_waves(), None = no wave motion
         self._observer = None            # the DPObserver of set_observer(), None = the agent sees the measurement
+        self._refmodel = None            # the ReferenceModel of set_reference_model(), None = the set-point is the reference
         self.EF = _EnvErrorFrame(self)
 
     # -- per-class tables (customEnv.py:58-65); subclasses override --------------------------------
@@ -455,13 +456,53 @@ class Revolt(object):
                 st = self.get_state()
                 eta, nu = (st["eta_measured"], st["nu_measured"]) if "eta_measured" in st else (st["eta"], st["nu"])
             obs = self._obs.clone()
-            obs[0:3] = ErrorFrame(eta, self._ref, device=self.device).get_pose()
+            obs[0:3] = ErrorFrame(eta, self._obs_ref(), device=self.device).get_pose()
             obs[3:6] = nu
+            self._obs = obs
+
+    def _obs_ref(self):
+        """What observation rows 0-2 are formed against: eta_d of an attached reference model, else the set-point."""
+        return self._ref if self._refmodel is None else self._refmodel.eta_d.contiguous()
+
+    def set_reference_model(self, model):
+        """Run a ``ReferenceModel`` in the loop (DESIGN.md section 4, "DP reference model in the loop");
+        ``set_reference_model(None)`` detaches.
+
+        While attached, the set-point (``set_ref``, ``step(new_ref=)``) is the operator's command s, and every step first
+        advances the model once on s inside the step kernel; the observation rows 0-2, the reward and the termination are
+        then formed against the model's eta_d instead of s, so the agent is trained and evaluated on tracking a smooth
+        reference.  Rows 3-8 are unchanged (the reward's velocity penalty still acts on nu, not nu - v_d).  Every reset and
+        in-kernel restart starts that env's model again at its new LF pose (eta_d = eta, v_d = a_d = 0); attaching starts
+        every env's model at its current LF pose.  ``model`` must have this env's num_envs, device and step.  The env keeps
+        a reference: the model's ``state`` is read and written by every step, so ``eta_d`` / ``v_d`` / ``a_d`` show the
+        in-loop values.  Like the observer, the setting is a launch parameter: ``rollout()`` keys its captured graphs on
+        it."""
+        with torch.cuda.device(self.device):
+            if model is None:
+                _lib.check(_lib.lib().ml4ca_env_set_refmodel(self._handle, None, None, self._stream()),
+                           "ml4ca_env_set_refmodel")
+            else:
+                assert model.num_envs == self.num_envs, "the reference model has %d envs, the env %d" % (model.num_envs,
+                                                                                                         self.num_envs)
+                assert model.state.device == self.device, \
+                    "the reference model lives on %s, the env on %s" % (model.state.device, self.device)
+                _lib.check(_lib.lib().ml4ca_env_set_refmodel(self._handle, ctypes.byref(model.cfg), _lib.ptr(model.state),
+                                                             self._stream()), "ml4ca_env_set_refmodel")
+        self._refmodel = model
+        if self._has_reset:             # rows 0-2 of the last observation are now formed against eta_d (or the set-point)
+            if self._observer is not None:
+                eta = self._observer.eta_hat.contiguous()
+            else:
+                st = self.get_state()
+                eta = st.get("eta_measured", st["eta"])
+            obs = self._obs.clone()
+            obs[0:3] = ErrorFrame(eta, self._obs_ref(), device=self.device).get_pose()
             self._obs = obs
 
     def observe(self):
         """state() / state_extended() (customEnv.py:196-205) of the current device-side state (measured, with waves on;
-        rows 0-5 from the estimates while an observer is attached)."""
+        rows 0-5 from the estimates while an observer is attached; rows 0-2 against eta_d while a reference model is
+        attached)."""
         obs = torch.empty_like(self._obs)
         with torch.cuda.device(self.device):
             _lib.check(_lib.lib().ml4ca_env_observe(self._handle, _lib.ptr(obs), self._stream()), "ml4ca_env_observe")

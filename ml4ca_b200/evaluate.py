@@ -50,10 +50,18 @@ def box_test_schedule(side=5.0, yaw_deg=-45.0, hold_s=60.0, dt=0.2):
 class _Guidance(object):
     """The set-point side of an evaluation run with a schedule: s(t), the last entry with steps <= t, and the reference the
     controllers track, r(t) = s(t), or with a reference model r(t) = eta_d(t) (with v_d(t) for the PID's feed-forward).
-    ``advance(t)`` moves the reference to r(t + 1) (the model steps once on s(t)) and hands it to the env (set_ref)."""
+    ``advance(t)`` moves the reference to r(t + 1) (the model steps once on s(t)) and hands it to the env (set_ref).
 
-    def __init__(self, env, schedule, reference_model, max_ep_len):
+    With the model attached to the env (``attached``), the env steps and resets it: ``advance(t)`` only hands s(t) to the
+    env, and ``stepped(t)`` reads r(t + 1) and v_d(t + 1) from the model after the env step.  Without a schedule an attached
+    model guides the fixed-test-pose runs to the env's set-point: s(t) is that set-point throughout."""
+
+    def __init__(self, env, schedule, reference_model, max_ep_len, attached=False):
         n, dev = env.num_envs, env.device
+        self.fixed = schedule is None
+        if self.fixed:
+            schedule = (np.zeros(1, dtype=np.int64), env._ref.clone()[None])
+            max_ep_len = max_ep_len if max_ep_len is not None else env.max_ep_len
         steps, sp = schedule
         steps = np.asarray(steps).reshape(-1)
         if steps.size == 0 or int(steps[0]) != 0 or np.any(np.diff(steps) <= 0):
@@ -71,13 +79,18 @@ class _Guidance(object):
         if self.T < 1:
             raise ValueError("the run needs at least one step: give max_ep_len or a schedule whose last step is > 0")
         self.idx = np.searchsorted(steps, np.arange(self.T + 1), side="right") - 1
-        self.env, self.model = env, reference_model
+        self.env, self.model, self.attached = env, reference_model, attached
 
     def s(self, t):
         return self.sp[int(self.idx[t])]
 
+    def r(self):
+        """The reference the env's observation is formed with now."""
+        return self.model.eta_d.clone() if self.attached else self.env._ref.clone()
+
     def start(self, rec):
-        """r(0) = s(0): the env's set-point before the reset, the model reset on it.  -> the start pose [3, n] numpy."""
+        """r(0) = s(0): the env's set-point before the reset, the model reset on it (an attached model is reset by the
+        env's reset_to).  -> the start pose [3, n] numpy: s(0), or the fixed test poses without a schedule."""
         s0 = self.s(0)
         self.env.set_ref(s0)
         f = dict(dtype=torch.float32, device=self.env.device)
@@ -85,19 +98,32 @@ class _Guidance(object):
         rec["setpoint"] = torch.empty(T + 1, 3, n, **f)
         rec["setpoint"][0] = s0
         if self.model is not None:
-            self.model.reset(s0)
+            if not self.attached:
+                self.model.reset(s0)
             rec["v_d"] = torch.empty(T + 1, 3, n, **f)
+        return fixed_test_poses(n) if self.fixed else s0.double().cpu().numpy()
+
+    def started(self, rec):
+        """After the env reset: v_d(0)."""
+        if self.model is not None:
             rec["v_d"][0] = self.model.v_d
-        return s0.double().cpu().numpy()
 
     def advance(self, t, rec):
-        if self.model is not None:
+        if self.attached:
+            self.env.set_ref(self.s(t))
+        elif self.model is not None:
             self.model.step(self.s(t))
             self.env.set_ref(self.model.eta_d.clone())
             rec["v_d"][t + 1] = self.model.v_d
         else:
             self.env.set_ref(self.s(t + 1))
         rec["setpoint"][t + 1] = self.s(t + 1)
+
+    def stepped(self, t, rec):
+        """After the env step of step t: r(t + 1) and v_d(t + 1) of an attached model."""
+        if self.attached:
+            rec["ref"][t + 1] = self.model.eta_d
+            rec["v_d"][t + 1] = self.model.v_d
 
 
 def in_loop_observer(env, observer):
@@ -109,6 +135,19 @@ def in_loop_observer(env, observer):
     if observer is not None and observer is not attached:
         raise ValueError("the env has an observer attached (set_observer); the controllers act on it, so a second "
                          "observer= cannot be passed")
+    return attached, True
+
+
+def in_loop_reference_model(env, reference_model):
+    """The reference model a run follows: the one attached to ``env`` (``Revolt.set_reference_model``), which the env steps
+    and resets itself, else ``reference_model``.  -> (model, attached).  A second model next to an attached one is an
+    error."""
+    attached = getattr(env, "_refmodel", None)
+    if attached is None:
+        return reference_model, False
+    if reference_model is not None and reference_model is not attached:
+        raise ValueError("the env has a reference model attached (set_reference_model); the run follows it, so a second "
+                         "reference_model= cannot be passed")
     return attached, True
 
 
@@ -149,12 +188,18 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
     Records gain ``setpoint`` [T+1, 3, n] (s), ``ref`` is r, and with a model ``v_d`` [T+1, 3, n]; the IAE integrates
     against ``setpoint``, so runs with and without a reference model are scored against the same command.  A schedule
     together with new_ref / ref_change_at, bad steps, set-points of the wrong shape or a model that does not match the
-    env raise ValueError; so does a reference model without a schedule."""
+    env raise ValueError; so does a reference model without a schedule.
+
+    On an env with an attached reference model (``Revolt.set_reference_model``) that model is used: the env resets and
+    steps it, and ``ref`` / ``v_d`` are read from it after each step; the records and metrics are those of the same run
+    with ``reference_model=`` on a plain env.  Passing another model then raises ValueError.  Without a schedule the
+    attached model guides the fixed-test-pose runs to the env's set-point: the records gain ``setpoint`` and the IAE is
+    scored against it; new_ref / ref_change_at then raise ValueError."""
     observer, attached = in_loop_observer(env, observer)
     n, dev = env.num_envs, env.device
     plan = _plan(env, schedule, reference_model, max_ep_len)
     if plan is not None and (new_ref is not None or ref_change_at is not None):
-        raise ValueError("a schedule replaces new_ref / ref_change_at: pass one or the other")
+        raise ValueError("a schedule (or an attached reference model) replaces new_ref / ref_change_at: pass one or the other")
     T = plan.T if plan is not None else int(max_ep_len if max_ep_len is not None else env.max_ep_len)
     rec = {}
     eta0 = plan.start(rec) if plan is not None else fixed_test_poses(n)
@@ -167,7 +212,10 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
                 "angles": torch.zeros(T + 1, 2, n, **f), "ref": torch.empty(T + 1, 3, n, **f)})
     done_at = torch.full((n,), T, dtype=torch.int32, device=dev)
     st = env.get_state()
-    rec["obs"][0], rec["eta"][0], rec["angles"][0], rec["ref"][0] = o, st["eta"], st["angles"][1:3], env._ref
+    rec["obs"][0], rec["eta"][0], rec["angles"][0] = o, st["eta"], st["angles"][1:3]
+    rec["ref"][0] = plan.r() if plan is not None else env._ref
+    if plan is not None:
+        plan.started(rec)
     integ = t_inside = None
     if integrator:
         integ, t_inside = torch.zeros(3, n, **f), torch.zeros(n, **f)
@@ -201,6 +249,8 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
             o, r, d, _ = env.step(torch.zeros_like(a), new_ref=new_ref)      # :141-146
         else:
             o, r, d, _ = env.step(a)
+        if plan is not None:
+            plan.stepped(t, rec)
         st = env.get_state()
         rec["obs"][t + 1], rec["rew"][t], rec["eta"][t + 1] = o, r, st["eta"]
         rec["thrust"][t + 1], rec["angles"][t + 1] = st["prev_thrust"], st["angles"][1:3]
@@ -222,11 +272,12 @@ def run_RL_policy(env, ac, max_ep_len=None, new_ref=None, ref_change_at=None, in
 
 
 def _plan(env, schedule, reference_model, max_ep_len):
-    if schedule is None:
+    reference_model, attached = in_loop_reference_model(env, reference_model)
+    if schedule is None and not attached:
         if reference_model is not None:
             raise ValueError("a reference model needs a schedule to filter")
         return None
-    return _Guidance(env, schedule, reference_model, max_ep_len)
+    return _Guidance(env, schedule, reference_model, max_ep_len, attached)
 
 
 def run_allocator(env, method="qp", max_ep_len=None, observer=None, schedule=None, reference_model=None):
@@ -243,7 +294,8 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None, schedule=Non
     schedule / reference_model: as in run_RL_policy.  The PID acts on r(t), and with a reference model it also gets
     v_d(t) as velocity feed-forward (``pinv_pid(nu_d=)``).  Records gain ``setpoint``, ``ref`` (r) [T+1, 3, n], with a
     model ``v_d``, and for ``method='qp'`` ``demand_clipped`` [T, n] (bool: the +-[4, 2, 2] demand clip below bound in
-    some DOF at that step)."""
+    some DOF at that step).  An attached reference model is used as in run_RL_policy; the PID's feed-forward then reads
+    v_d from it."""
     observer, attached = in_loop_observer(env, observer)
     from .pinv import pinv_pid
     from .qp_allocator import QPTA
@@ -271,7 +323,8 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None, schedule=Non
     ref = env._ref.clone()
     if plan is not None:
         rec["ref"] = torch.empty(T + 1, 3, n, **f)
-        rec["ref"][0] = ref
+        rec["ref"][0] = plan.r()
+        plan.started(rec)
         if qp is not None:
             rec["demand_clipped"] = torch.empty(T, n, dtype=torch.bool, device=dev)
     # The SLSQP programme only admits demands its rate limits can follow (|df| <= 5, 5, 2 N per call): on the vessel the
@@ -311,6 +364,8 @@ def run_allocator(env, method="qp", max_ep_len=None, observer=None, schedule=Non
             plan.advance(t, rec)
             rec["ref"][t + 1] = env._ref
         o, r, d, _ = env.step(action)
+        if plan is not None:
+            plan.stepped(t, rec)
         st = env.get_state()
         rec["rew"][t], rec["eta"][t + 1] = r, st["eta"]
         rec["thrust"][t + 1], rec["angles"][t + 1] = st["prev_thrust"], st["angles"][1:3]

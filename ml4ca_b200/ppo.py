@@ -132,12 +132,14 @@ def rollout(env, ac, buf, seed=0, start_step=0, deterministic=False, graph=False
     else:
         cache = buf.__dict__.setdefault("_rollout_graphs", {})
         # launch parameters are baked into a captured graph: the restart fraction (curriculum), the disturbance, the
-        # wave setting and the attached observer are part of the key
+        # wave setting, the attached observer and the attached reference model are part of the key
         obsv = getattr(env, "_observer", None)
         obsv_key = None if obsv is None else (id(obsv), obsv.state.data_ptr(), obsv.omega_o.data_ptr(),
                                               bytes(obsv.cfg))
+        refm = getattr(env, "_refmodel", None)
+        ref_key = None if refm is None else (id(refm), refm.state.data_ptr(), bytes(refm.cfg))
         key = (id(env), id(ac), int(seed), bool(deterministic), float(env._cfg.reset_fraction),
-               getattr(env, "_disturbance", None), getattr(env, "_waves", None), obsv_key)
+               getattr(env, "_disturbance", None), getattr(env, "_waves", None), obsv_key, ref_key)
         entry = cache.get(key)
         if entry is None:                  # first call: eager, and remember that the next one may capture
             cache[key] = {"graph": None, "counter": torch.zeros(1, dtype=torch.int32, device=buf.device)}
